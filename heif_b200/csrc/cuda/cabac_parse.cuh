@@ -146,6 +146,7 @@ struct Engine {
   HEIC_HD bool offset_is_illegal() const { return (val >> 22) >= 510u; }
   HEIC_HD void expect_terminate(int) {}  // hook for the test-only encoder engine (tests/synth); nothing to do when decoding
   HEIC_HD void hint_ctx(int) {}          // likewise: tells that engine which context the next decision uses
+  HEIC_HD void hint_level_remaining(int, int) {}  // likewise: a coeff_abs_level_remaining (cRiceParam, baseLevel) follows
   HEIC_HD void refill() {
     if (nbits < 7) {
       val |= look0 << (6 - nbits);
@@ -282,6 +283,15 @@ struct Engine {
     return ((uint32_t)prefix << rice) + ((hi << 1) | (uint32_t)bypass());
   }
 };
+
+// Engine::hint_level_remaining is optional for the engines the parser is instantiated with: one without it compiles and
+// behaves as before (overload resolution prefers the first form when the call is well formed).
+template <class Eng>
+HEIC_HD auto hint_level_remaining(Eng& e, int rice, int base_level, int) -> decltype(e.hint_level_remaining(rice, base_level)) {
+  return e.hint_level_remaining(rice, base_level);
+}
+template <class Eng>
+HEIC_HD void hint_level_remaining(Eng&, int, int, long) {}
 
 #if defined(__CUDA_ARCH__) && !defined(HEIC_CABAC_INLINE_ENGINE)
 // Out-of-line engine entry points for the device parser.  The engine lives in registers and travels by value (the
@@ -525,7 +535,7 @@ struct Parser {
     if (r.bad) fail(-3);
     return r.v;
   }
-  HEIC_HD uint32_t coeff_abs_level_remaining(int rice) {
+  HEIC_HD uint32_t coeff_abs_level_remaining(int rice, int) {
     const EngRet r = eng_calr(e, rice);
     e = r.e;
     if (r.bad) fail(-3);
@@ -552,7 +562,8 @@ struct Parser {
     uint32_t suffix = e.fl_bypass(ones + k);
     return (((1u << ones) - 1u) << k) + suffix;
   }
-  HEIC_HD uint32_t coeff_abs_level_remaining(int rice) {  // decoder.rs:224-261
+  HEIC_HD uint32_t coeff_abs_level_remaining(int rice, int base_level) {  // decoder.rs:224-261
+    hint_level_remaining(e, rice, base_level, 0);
     uint32_t prefix = 0;
     while (prefix < 4 && e.bypass()) prefix++;
     if (prefix < 4) return (prefix << rice) + e.fl_bypass(rice);
@@ -827,7 +838,7 @@ HEIC_NO_UNROLL
       m &= ~(1u << k);
       int abs_level = 1 + (int)((g1 >> k) & 1u) + (int)((g2x >> k) & 1u);
       if ((need_rem >> k) & 1u) {
-        uint32_t rem = coeff_abs_level_remaining(rice);
+        uint32_t rem = coeff_abs_level_remaining(rice, abs_level);
         if (rem > 32768u) {
           fail(-3);
           return;

@@ -40,3 +40,34 @@ CONFIGS = [
                         cb_qp_offset=-2, cr_qp_offset=5, init_qp_minus26=-3, lps_gain=1.3)),
 ]
 SEEDS = (0, 1)
+
+# Value-range extremes, kept apart from CONFIGS (whose streams are pinned to FFmpeg hashes): escape-coded levels up to
+# 32767 (big_level_prob), explicit scaling lists over the whole legal range 1..255, QP 0 and 51, cu_qp_delta wrapping
+# around 0/51, chroma QP offsets of +-12 and deblocking offsets of +-6.  Scaled coefficients saturate at both int16 ends,
+# the 64-bit scaling branch of the transform kernels runs, residuals reach ~23 K and reconstructed samples pin to 0 / 255.
+_BIG = dict(big_level_prob=0.3, max_transform_hierarchy_depth_intra=1)
+_FULL_LISTS = dict(scaling_list_min=1, scaling_list_max=255)
+EXTREME_CONFIGS = [
+    ("big_qp51_flat", dict(_BIG, init_qp_minus26=25)),
+    ("big_qp51_sps_lists", dict(_BIG, **_FULL_LISTS, init_qp_minus26=25, scaling_list_mode=2)),
+    ("big_qp51_pps_lists_tskip", dict(_BIG, **_FULL_LISTS, init_qp_minus26=25, scaling_list_mode=3, transform_skip=1)),
+    ("big_qp0", dict(_BIG, init_qp_minus26=-26, transform_skip=1)),
+    # lists of ones at QP 30 with few, large 16x16 / 32x32 blocks: the kernels' 32-bit product test (which assumes entries
+    # up to 255) fails on blocks whose scaled coefficients stay in range, so the 64-bit branch yields unsaturated values
+    ("big_qp30_unit_lists", dict(big_level_prob=0.05, init_qp_minus26=4, scaling_list_mode=2, scaling_list_min=1, scaling_list_max=1,
+                                 split_cu_prob=0.2, width=256, height=256)),
+    ("big_qp51_ctb64", dict(_BIG, init_qp_minus26=25, log2_ctb=6, width=192, height=128, scaling_list_mode=1)),
+    ("big_qp51_ctb16", dict(_BIG, init_qp_minus26=25, log2_ctb=4, log2_max_tb=4, width=96, height=80)),
+    ("cu_qp_delta_low_qp", dict(_BIG, cu_qp_delta=1, diff_cu_qp_delta_depth=2, init_qp_minus26=-25)),
+    ("cu_qp_delta_high_qp", dict(_BIG, cu_qp_delta=1, diff_cu_qp_delta_depth=2, init_qp_minus26=24)),
+    ("chroma_offsets_pps12_slice_m12", dict(_BIG, init_qp_minus26=10, cb_qp_offset=12, cr_qp_offset=12, slice_cb_qp_offset=-12,
+                                            slice_cr_qp_offset=-12, cu_qp_delta=1, diff_cu_qp_delta_depth=1)),
+    ("chroma_offsets_pps_m12_slice12", dict(_BIG, init_qp_minus26=10, cb_qp_offset=-12, cr_qp_offset=-12, slice_cb_qp_offset=12,
+                                            slice_cr_qp_offset=12, cu_qp_delta=1, diff_cu_qp_delta_depth=1)),
+    ("deblock_plus6_qp51", dict(_BIG, init_qp_minus26=25, beta_offset_div2=6, tc_offset_div2=6)),
+    ("deblock_plus6_qp30", dict(_BIG, init_qp_minus26=4, beta_offset_div2=6, tc_offset_div2=6)),
+    ("deblock_minus6_qp51", dict(_BIG, init_qp_minus26=25, beta_offset_div2=-6, tc_offset_div2=-6)),
+    ("deblock_minus6_qp30", dict(_BIG, init_qp_minus26=4, beta_offset_div2=-6, tc_offset_div2=-6)),
+    ("big_monochrome", dict(_BIG, init_qp_minus26=25, chroma_format_idc=0)),
+]
+EXTREME_SEEDS = (0, 1)

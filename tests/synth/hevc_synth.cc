@@ -8,9 +8,10 @@
 // EncodeBypass, EncodeTerminate, EncodeFlush, PutBit with outstanding bits) and returned, so the walker's control
 // flow guarantees a syntactically valid slice that exercises whatever the parameter sets enable (CTB 16/32/64,
 // transform hierarchy, transform skip, sign data hiding, cu_qp_delta, SAO, WPP on/off, scaling lists, 4:0:0, picture
-// sizes that are not CTB multiples).  VPS/SPS/PPS/slice-header writers (7.3.1-7.3.6) and emulation prevention
+// sizes that are not CTB multiples, escape-coded levels up to 32767 on request).  VPS/SPS/PPS/slice-header writers (7.3.1-7.3.6) and emulation prevention
 // make it a complete Annex-B-able stream, so FFmpeg — not just this repo's oracle — can decode it.
 // Never linked into libheic_b200.so.
+#include <cmath>
 #include <cstdint>
 #include <cstring>
 #include <vector>
@@ -60,6 +61,52 @@ struct BitWriter {
   bool aligned() const { return nbits == 0; }
 };
 
+// 9.3.3.11 binarization of coeff_abs_level_remaining: TR prefix (cMax 4 << cRiceParam) and, past it, an EG(k) escape with
+// k = cRiceParam + 1 (unary prefix of ones, a zero, prefix + k suffix bits).  Appends the bins to `out`.
+void level_remaining_bins(int rice, uint32_t v, std::vector<uint8_t>& out) {
+  if (v < (4u << rice)) {
+    for (uint32_t i = 0; i < (v >> rice); i++) out.push_back(1);
+    out.push_back(0);
+    for (int b = rice - 1; b >= 0; b--) out.push_back((uint8_t)((v >> b) & 1u));
+    return;
+  }
+  for (int i = 0; i < 4; i++) out.push_back(1);
+  uint32_t u = v - (4u << rice);
+  int k = rice + 1, ones = 0;
+  while (u >= (1u << k)) {
+    u -= 1u << k;
+    k++;
+    ones++;
+  }
+  for (int i = 0; i < ones; i++) out.push_back(1);
+  out.push_back(0);
+  for (int b = k - 1; b >= 0; b--) out.push_back((uint8_t)((u >> b) & 1u));
+}
+
+// A coeff_abs_level_remaining value in [0, max_value]: the maximum, a value next to a change of the escape's prefix length
+// (first value of a prefix length, +-1), or log-uniform over the range.
+uint32_t large_level_target(Rng& rng, int rice, int max_value) {
+  if (max_value <= 0) return 0;
+  const uint32_t pick = (uint32_t)(rng.next() % 8);
+  if (pick == 0) return (uint32_t)max_value;
+  if (pick == 1) {
+    uint32_t edges[24];
+    int n = 0;
+    for (int ones = 0; ones < 24; ones++) {
+      const uint64_t first = (4ull << rice) + ((((1ull << ones) - 1ull)) << (rice + 1));
+      if (first > (uint64_t)max_value) break;
+      edges[n++] = (uint32_t)first;
+    }
+    if (n) {
+      const int64_t v = (int64_t)edges[rng.next() % (uint64_t)n] + (int64_t)(rng.next() % 3) - 1;
+      return (uint32_t)(v < 0 ? 0 : (v > max_value ? max_value : v));
+    }
+  }
+  const double x = std::exp(rng.uniform() * std::log((double)max_value + 1.0)) - 1.0;
+  const uint32_t v = (uint32_t)x;
+  return v > (uint32_t)max_value ? (uint32_t)max_value : v;
+}
+
 // Encoder twin of dev::Engine (same member functions the Parser calls).
 struct EncEngine {
   const uint8_t* data = nullptr;  // unused
@@ -71,7 +118,12 @@ struct EncEngine {
   // (< 0: off, the context's own probability is used): real streams switch SAO on for a few per cent of the CTBs and
   // smooth pictures rarely split their coding units.
   double sao_on_prob = -1.0, split_cu_prob = -1.0;
+  // With this probability a coeff_abs_level_remaining takes a chosen value (large_level_target) instead of the random walk:
+  // its bins are queued and served to the next bypass() calls without the ones cap.
+  double big_level_prob = 0.0;
   int ctx_hint = -1;
+  std::vector<uint8_t> queued;  // bypass bins still to serve, in order
+  size_t queued_pos = 0;
   // arithmetic encoder state (9.3.4.x)
   uint32_t low = 0, range = 510;
   int first_bit = 1, outstanding = 0, ones_run = 0, next_term = 0;
@@ -148,6 +200,11 @@ struct EncEngine {
   bool offset_is_illegal() const { return false; }
   void expect_terminate(int v) { next_term = v; }
   void hint_ctx(int idx) { ctx_hint = idx; }
+  void hint_level_remaining(int rice, int base_level) {
+    if (big_level_prob <= 0.0 || rng->uniform() >= big_level_prob) return;  // no draw at all when off: streams stay as before
+    level_remaining_bins(rice, large_level_target(*rng, rice, 32767 - base_level), queued);
+    queued_pos = 0;
+  }
   int decision(const CabacTabs* T, uint32_t& s) {
     double forced = -1.0;
     if (ctx_hint == CTX_SAO_TYPE) forced = sao_on_prob;
@@ -174,6 +231,17 @@ struct EncEngine {
     return bin;
   }
   int bypass() {
+    if (queued_pos < queued.size()) {
+      const int bin = queued[queued_pos++];
+      if (queued_pos == queued.size()) {
+        queued.clear();
+        queued_pos = 0;
+      }
+      ones_run = 0;
+      encode_bypass(bin);
+      bins++;
+      return bin;
+    }
     int bin = (int)(rng->next() >> 63);
     if (bin && ones_run >= max_bypass_ones) bin = 0;
     ones_run = bin ? ones_run + 1 : 0;
@@ -296,6 +364,8 @@ struct synth_config {
   double lps_gain;                     // 1.0 = draw bins from the contexts' own probabilities
   uint32_t max_bypass_ones;
   double sao_on_prob, split_cu_prob;   // < 0: unbiased (see EncEngine)
+  double big_level_prob;               // 0: every coeff_abs_level_remaining from the random walk (see EncEngine)
+  uint32_t scaling_list_min, scaling_list_max;  // range of the explicit scaling-list entries (0, 0: 8..63)
 };
 
 // Writes the four NAL units (2-byte header + escaped payload) of one IDR_N_LP picture.  Each out_* buffer has `cap`
@@ -344,11 +414,13 @@ int synth_encode_picture(const synth_config* cfg, uint64_t seed, uint8_t* out_vp
     pps.pps_scaling_list_data_present_flag = cfg->scaling_list_mode == 3;
     heic_scaling_list lists;
     default_scaling_list(lists);
-    if (cfg->scaling_list_mode >= 2) {  // seeded explicit lists in [8, 64)
+    if (cfg->scaling_list_mode >= 2) {  // seeded explicit lists in [scaling_list_min, scaling_list_max]
+      const uint32_t lo = cfg->scaling_list_min ? cfg->scaling_list_min : 8, hi = cfg->scaling_list_max ? cfg->scaling_list_max : 63;
+      if (lo < 1 || hi > 255 || lo > hi) return -2;
       for (int s = 0; s < 4; s++)
         for (int m = 0; m < 6; m++) {
-          for (int i = 0; i < 64; i++) lists.list[s][m][i] = (uint8_t)(8 + rng.next() % 56);
-          if (s >= 2) lists.dc[s - 2][m] = (uint8_t)(8 + rng.next() % 56);
+          for (int i = 0; i < 64; i++) lists.list[s][m][i] = (uint8_t)(lo + rng.next() % (hi - lo + 1));
+          if (s >= 2) lists.dc[s - 2][m] = (uint8_t)(lo + rng.next() % (hi - lo + 1));
         }
       // sizeId 3 only codes matrixId 0 and 3; a decoder copies nothing else, so keep the chroma slots consistent with
       // what 7.3.4 infers for ChromaArrayType != 3 (not used for 4:2:0 intra 32x32, but keep the struct well defined)
@@ -395,6 +467,7 @@ int synth_encode_picture(const synth_config* cfg, uint64_t seed, uint8_t* out_vp
     P.e.max_bypass_ones = cfg->max_bypass_ones ? (int)cfg->max_bypass_ones : 6;
     P.e.sao_on_prob = cfg->sao_on_prob;
     P.e.split_cu_prob = cfg->split_cu_prob;
+    P.e.big_level_prob = cfg->big_level_prob;
     P.T = &tabs;
     P.ctx = ctx.data();
     P.pp = &pp;
@@ -577,6 +650,72 @@ int synth_encode_picture(const synth_config* cfg, uint64_t seed, uint8_t* out_vp
   } catch (const Error&) {
     return -2;
   }
+}
+
+// Round trip of one coeff_abs_level_remaining through the arithmetic coder: `value` is encoded as bypass bins (the bins the
+// generator queues) behind a seeded run of context-coded bins, which sets ivlCurrRange and the bit position, and the stream
+// is placed at an even or odd byte offset (the engine's 16-bit refill phase).  The bins are then decoded twice: with
+// dev::Engine::coeff_abs_level_remaining (the device routine: 7-bin division steps) and with the parser's bin-by-bin loop.
+// out[0..4]: value and bins of the device routine, value and bins of the loop, bins the encoder wrote.  Returns 0; the
+// `bad` flags of the two decodes (1: device routine, 2: loop) when one of them rejected the bins; -1 when the leading
+// context-coded bins did not decode back.
+int synth_level_remaining_roundtrip(int rice, uint32_t value, uint64_t seed, uint32_t* out) {
+  static const CabacTabs tabs = [] {
+    CabacTabs t;
+    build_cabac_tabs(t);
+    return t;
+  }();
+  Rng rng{seed * 0x9e3779b97f4a7c15ull + 0x51ed27ull};
+  const int n_lead = (int)(rng.next() % 48), n_tail = 40;
+  const int odd = (int)(rng.next() & 1u);
+  std::vector<uint32_t> states;  // context state of each leading bin, drawn afresh per bin (both sides start from it)
+  std::vector<uint8_t> lead;
+  for (int i = 0; i < n_lead; i++) {
+    states.push_back((uint32_t)(rng.next() % 126));
+    lead.push_back((uint8_t)(rng.next() >> 63));
+  }
+  std::vector<uint8_t> bins;
+  level_remaining_bins(rice, value, bins);
+  EncEngine E;
+  E.rng = &rng;
+  E.init(nullptr, 0, 0);
+  for (int i = 0; i < n_lead; i++) {
+    uint32_t s = states[i];
+    E.encode_decision(&tabs, s, lead[i]);
+  }
+  for (uint8_t b : bins) E.encode_bypass(b);
+  for (int i = 0; i < n_tail; i++) E.encode_bypass((int)(rng.next() >> 63));
+  E.range -= 2;  // end_of_slice_segment_flag = 1
+  E.low += E.range;
+  E.flush();
+  std::vector<uint8_t> buf((size_t)odd, 0xa5);
+  buf.insert(buf.end(), E.cur->bytes.begin(), E.cur->bytes.end());
+  buf.resize(buf.size() + 8, 0);
+
+  int flags = 0;
+  uint32_t vals[2], used[2];
+  for (int pass = 0; pass < 2; pass++) {
+    Parser<1> P;
+    P.err = 0;
+    P.e.init(buf.data(), (uint32_t)odd, (uint32_t)buf.size());
+    P.e.bins = 0;
+    for (int i = 0; i < n_lead; i++) {
+      uint32_t s = states[i];
+      if (P.e.decision(&tabs, s) != lead[i]) return -1;  // the leading bins must come back unchanged
+    }
+    const uint32_t b0 = P.e.bins;
+    int bad = 0;
+    if (pass == 0) vals[0] = P.e.coeff_abs_level_remaining(rice, bad);
+    else vals[1] = P.coeff_abs_level_remaining(rice, 0), bad = P.err != 0;
+    used[pass] = P.e.bins - b0;
+    if (bad) flags |= 1 << pass;
+  }
+  out[0] = vals[0];
+  out[1] = used[0];
+  out[2] = vals[1];
+  out[3] = used[1];
+  out[4] = (uint32_t)bins.size();
+  return flags;
 }
 
 }  // extern "C"

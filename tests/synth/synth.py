@@ -23,7 +23,8 @@ class Config(C.Structure):
         ("deblocking_disabled", C.c_uint32), ("beta_offset_div2", C.c_int32), ("tc_offset_div2", C.c_int32),
         ("slice_sao_luma", C.c_uint32), ("slice_sao_chroma", C.c_uint32), ("full_range", C.c_uint32),
         ("matrix_coeffs", C.c_uint32), ("lps_gain", C.c_double), ("max_bypass_ones", C.c_uint32),
-        ("sao_on_prob", C.c_double), ("split_cu_prob", C.c_double),
+        ("sao_on_prob", C.c_double), ("split_cu_prob", C.c_double), ("big_level_prob", C.c_double),
+        ("scaling_list_min", C.c_uint32), ("scaling_list_max", C.c_uint32),
     ]
 
 
@@ -32,7 +33,7 @@ DEFAULTS = dict(width=128, height=128, chroma_format_idc=1, log2_min_cb=3, log2_
                 transform_skip=0, cu_qp_delta=0, diff_cu_qp_delta_depth=0, init_qp_minus26=0, slice_qp_delta=0, cb_qp_offset=0,
                 cr_qp_offset=0, slice_cb_qp_offset=0, slice_cr_qp_offset=0, wpp=1, deblocking_disabled=0, beta_offset_div2=0,
                 tc_offset_div2=0, slice_sao_luma=1, slice_sao_chroma=1, full_range=1, matrix_coeffs=6, lps_gain=1.0,
-                max_bypass_ones=0, sao_on_prob=-1.0, split_cu_prob=-1.0)
+                max_bypass_ones=0, sao_on_prob=-1.0, split_cu_prob=-1.0, big_level_prob=0.0, scaling_list_min=8, scaling_list_max=63)
 
 _lib = None
 
@@ -43,7 +44,16 @@ def _load():
         subprocess.check_call(["make", "-s", "-C", HERE])
         _lib = C.CDLL(os.path.join(HERE, "_build", "libhevc_synth.so"))
         _lib.synth_encode_picture.argtypes = [C.POINTER(Config), C.c_uint64] + [C.c_void_p] * 4 + [C.c_size_t, C.POINTER(C.c_size_t)]
+        _lib.synth_level_remaining_roundtrip.argtypes = [C.c_int, C.c_uint32, C.c_uint64, C.POINTER(C.c_uint32)]
     return _lib
+
+
+def level_remaining_roundtrip(rice: int, value: int, seed: int):
+    """coeff_abs_level_remaining `value` encoded as bypass bins and decoded by the device routine and by the bin-by-bin
+    loop (see hevc_synth.cc).  Returns (flags, (device value, device bins), (loop value, loop bins), encoded bins)."""
+    out = (C.c_uint32 * 5)()
+    rc = _load().synth_level_remaining_roundtrip(rice, value, seed, out)
+    return rc, (out[0], out[1]), (out[2], out[3]), out[4]
 
 
 class Picture:

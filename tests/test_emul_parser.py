@@ -71,10 +71,18 @@ def _synth_cases():
     return [(name, cfg, SEEDS[0]) for name, cfg in CONFIGS]
 
 
-@pytest.mark.parametrize("name,cfg,seed", _synth_cases(), ids=[c[0] for c in _synth_cases()])
+def _extreme_cases():
+    from tests.synth.configs import EXTREME_CONFIGS, EXTREME_SEEDS
+
+    return [(name, cfg, seed) for name, cfg in EXTREME_CONFIGS for seed in EXTREME_SEEDS]
+
+
+@pytest.mark.parametrize("name,cfg,seed", _synth_cases() + _extreme_cases(),
+                         ids=[c[0] for c in _synth_cases()] + [f"{c[0]}/{c[2]}" for c in _extreme_cases()])
 def test_device_parser_matches_oracle_on_synthetic_streams(emul, name, cfg, seed):
     """Every feature configuration of the synthetic generator (CTB 16/64, no WPP, transform skip, sign data hiding,
-    cu_qp_delta, transform hierarchy, 4:0:0, ragged sizes, ...) through the host build of the device parser."""
+    cu_qp_delta, transform hierarchy, 4:0:0, ragged sizes, ...) through the host build of the device parser; and the
+    value-range extremes (escape-coded levels up to 32767, QP 0 / 51, cu_qp_delta wrap-around)."""
     from tests.synth import synth
 
     pic = synth.encode(seed, **cfg)

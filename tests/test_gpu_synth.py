@@ -19,7 +19,12 @@ GOLDEN = json.load(open(os.path.join(HERE, "golden", "synth_hashes.json")))["str
 
 @pytest.mark.parametrize("name,cfg", CONFIGS, ids=[n for n, _ in CONFIGS])
 def test_stages_match_oracle(decoder, name, cfg):
-    pic = synth.encode(SEEDS[0], **cfg)
+    check_stages(decoder, synth.encode(SEEDS[0], **cfg))
+
+
+def check_stages(decoder, pic):
+    """One picture stage by stage against the oracle: status and bins, levels, residual, recon, deblocked, SAO, RGB.
+    Returns the GPU's residual arrays."""
     t = pic.tile
     ref = O.decode_picture(pic.sps, pic.pps, t.header, (t.rbsp, t.rbsp_len))
     n_comp = 3 if pic.sps.chroma_format_idc else 1
@@ -35,8 +40,9 @@ def test_stages_match_oracle(decoder, name, cfg):
         assert np.array_equal(d["qp_map"], ref["qp_map"]) and np.array_equal(d["sao"], ref["sao"])
         b.run(H.STAGE_TRANSFORM)
         d = b.dump_tile(0)
+        resid = [np.array(d["coeff"][c]) for c in range(n_comp)]
         for c in range(n_comp):
-            assert np.array_equal(d["coeff"][c], ref["resid"][c]), f"residual {c}"
+            assert np.array_equal(resid[c], ref["resid"][c]), f"residual {c}"
         for stage, key in ((H.STAGE_INTRA, "recon"), (H.STAGE_DEBLOCK, "deblocked"), (H.STAGE_SAO, "plane")):
             b.run(stage)
             d = b.dump_tile(0)
@@ -49,6 +55,7 @@ def test_stages_match_oracle(decoder, name, cfg):
         planes = np.concatenate([p.ravel() for p in ref["plane"]])
         exp = O.color_stitch(planes, 1, 1, w, h, w, h, pic.sps.video_full_range_flag, pic.sps.matrix_coeffs)
         assert np.array_equal(rgb, exp)
+    return resid
 
 
 def test_heterogeneous_batch_matches_ffmpeg_golden(decoder):

@@ -1,6 +1,7 @@
 """The opt-out paths selected by environment variables (read once per process, hence the subprocess): the register
-butterflies for 8x8 .. 32x32 transforms (HEIC_B200_TRANSFORM_MMA=0, the A/B partner of the tensor-core kernels) and the
-unordered chunk pipeline (HEIC_B200_PIPE_ORDER=0) must stay bit-exact too."""
+butterflies for 8x8 .. 32x32 transforms (HEIC_B200_TRANSFORM_MMA=0, the A/B partner of the tensor-core kernels; on the
+ordinary synthetic streams and at the value-range extremes) and the unordered chunk pipeline (HEIC_B200_PIPE_ORDER=0) must
+stay bit-exact too."""
 import os
 import subprocess
 import sys
@@ -15,9 +16,10 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
     "env,target",
     [
         ({"HEIC_B200_TRANSFORM_MMA": "0"}, "tests/test_gpu_synth.py::test_stages_match_oracle"),
+        ({"HEIC_B200_TRANSFORM_MMA": "0"}, "tests/test_gpu_extremes.py"),
         ({"HEIC_B200_PIPE_ORDER": "0"}, "tests/test_gpu_pipeline.py"),
     ],
-    ids=["transform_butterflies", "pipeline_unordered"],
+    ids=["transform_butterflies", "transform_butterflies_extremes", "pipeline_unordered"],
 )
 def test_opt_out_path_is_bit_exact(built, env, target):
     e = dict(os.environ)
