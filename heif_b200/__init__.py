@@ -134,6 +134,12 @@ class HeicFile:
         K.check(self._lib.heic_b200_file_info(self._h, C.byref(out)))
         return out
 
+    def transform(self, image: int = -1) -> K.ImageTransform:
+        """The image item's clap / irot / imir properties in normal form (image = -1: primary, >= 0: auxiliary)."""
+        out = K.ImageTransform()
+        K.check(self._lib.heic_b200_file_image_transform(self._h, image, C.byref(out)))
+        return out
+
     def parameter_set_nal(self, nal_unit_type: int, image: int = -1) -> bytes:
         p, n = C.POINTER(K.u8)(), C.c_size_t()
         K.check(self._lib.heic_b200_file_parameter_set_nal(self._h, image, nal_unit_type, C.byref(p), C.byref(n)))
@@ -155,12 +161,43 @@ class HeifReader:
         return HeicFile(self._data)
 
 
-def _canvas(img: K.ImageDesc, apply_transforms: bool):
-    w = img.output_width or img.grid_cols * img.sps.pic_width_in_luma_samples
-    h = img.output_height or img.grid_rows * img.sps.pic_height_in_luma_samples
-    if apply_transforms and (img.rotation_ccw_quarter_turns & 1):
-        w, h = h, w
+def tile_size(img: K.ImageDesc):
+    """(width, height) at which the grid stitches a tile: the SPS conformance window of its decoded picture."""
+    sps = img.sps
+    w, h = sps.pic_width_in_luma_samples, sps.pic_height_in_luma_samples
+    if sps.conformance_window_flag:
+        sub = 2 if sps.chroma_format_idc == 1 else 1
+        w -= sub * (sps.conf_win_left_offset + sps.conf_win_right_offset)
+        h -= sub * (sps.conf_win_top_offset + sps.conf_win_bottom_offset)
     return w, h
+
+
+def canvas_transform(img: K.ImageDesc, apply_transforms: bool = False) -> K.ImageTransform:
+    """What the calls without transforms apply: the whole canvas, turned by irot when apply_transforms is set."""
+    tw, th = tile_size(img)
+    w = img.output_width or img.grid_cols * tw
+    h = img.output_height or img.grid_rows * th
+    return K.ImageTransform(0, 0, w, h, (img.rotation_ccw_quarter_turns & 3) if apply_transforms else 0)
+
+
+def _transform(t) -> K.ImageTransform:
+    return t if isinstance(t, K.ImageTransform) else K.ImageTransform(*t)
+
+
+def _canvas(img: K.ImageDesc, apply_transforms: bool = False, transform=None):
+    """(width, height) of an image's output: the transform's crop, turned for odd quarter turns."""
+    t = _transform(transform) if transform is not None else canvas_transform(img, apply_transforms)
+    return (t.crop_h, t.crop_w) if t.orientation & 1 else (t.crop_w, t.crop_h)
+
+
+def _transform_array(transforms, n: int):
+    transforms = [_transform(t) for t in transforms]
+    if len(transforms) != n:
+        raise ValueError("one transform per image")
+    arr = (K.ImageTransform * n)()
+    for i, t in enumerate(transforms):
+        arr[i] = t
+    return arr
 
 
 def _desc_array(images):
@@ -173,14 +210,22 @@ def _desc_array(images):
 class Batch:
     """A resident batch: bitstreams, descriptors and every intermediate live in HBM (heic_b200_batch_*)."""
 
-    def __init__(self, dec: "HeicDecoder", images, apply_transforms: bool = False):
+    def __init__(self, dec: "HeicDecoder", images, apply_transforms: bool = False, transforms=None):
+        """transforms: one heic_image_transform (K.ImageTransform or (x, y, w, h, orientation)) per image; when None,
+        apply_transforms selects the irot turn of every image or none."""
         self._lib = dec._lib
         self._dec = dec
         self.images = list(images)
         self.apply_transforms = bool(apply_transforms)
         self._arr = _desc_array(self.images)
         self._h = C.c_void_p()
-        K.check(self._lib.heic_b200_batch_create_ex(dec._h, self._arr, len(self.images), int(self.apply_transforms), C.byref(self._h)))
+        if transforms is None:
+            self.transforms = [canvas_transform(im, self.apply_transforms) for im in self.images]
+            K.check(self._lib.heic_b200_batch_create_ex(dec._h, self._arr, len(self.images), int(self.apply_transforms), C.byref(self._h)))
+        else:
+            self._xf = _transform_array(transforms, len(self.images))
+            self.transforms = list(self._xf)
+            K.check(self._lib.heic_b200_batch_create_transformed(dec._h, self._arr, self._xf, len(self.images), C.byref(self._h)))
 
     def close(self):
         if self._h:
@@ -230,7 +275,7 @@ class Batch:
         return int(p.value or 0), pitch.value, stride.value
 
     def download_rgb(self, out: np.ndarray | None = None) -> np.ndarray:
-        w, h = _canvas(self.images[0], self.apply_transforms)
+        w, h = _canvas(self.images[0], transform=self.transforms[0])
         if out is None:
             out = np.empty((len(self.images), h, w, 3), np.uint8)
         K.check(self._lib.heic_b200_batch_download_rgb(self._h, out.ctypes.data, out.strides[1], out.strides[0]))
@@ -238,7 +283,7 @@ class Batch:
 
     def download_image(self, index: int) -> np.ndarray:
         """RGB of one image of the batch (H, W, 3)."""
-        w, h = _canvas(self.images[index], self.apply_transforms)
+        w, h = _canvas(self.images[index], transform=self.transforms[index])
         out = np.empty((h, w, 3), np.uint8)
         K.check(self._lib.heic_b200_batch_download_image(self._h, index, out.ctypes.data, out.strides[0]))
         return out
@@ -312,37 +357,52 @@ class HeicDecoder:
         return int(self._lib.heic_b200_launch_count(self._h))
 
     def decode(self, data, apply_transforms: bool = False) -> np.ndarray:
-        """bytes | HeicFile -> (H, W, 3) uint8 RGB of the primary item."""
+        """bytes | HeicFile -> (H, W, 3) uint8 RGB of the primary item; apply_transforms: with the file's clap / irot / imir."""
         f = data if isinstance(data, HeicFile) else HeicFile(data)
-        return self.decode_grids([f.primary], apply_transforms=apply_transforms)[0]
+        if apply_transforms:
+            return self.decode_grids([f.primary], transforms=[f.transform()])[0]
+        return self.decode_grids([f.primary])[0]
 
-    def decode_grids(self, images, out: np.ndarray | None = None, apply_transforms: bool = False, return_status: bool = False):
-        """Batch of image descriptors (host) -> (n, H, W, 3) uint8 RGB (host).  All images must share one canvas size."""
+    def decode_grids(self, images, out: np.ndarray | None = None, apply_transforms: bool = False, return_status: bool = False,
+                     transforms=None):
+        """Batch of image descriptors (host) -> (n, H, W, 3) uint8 RGB (host).  All outputs must share one size.
+        transforms: one heic_image_transform per image (see Batch); when None, apply_transforms selects irot or nothing."""
         images = list(images)
         arr = _desc_array(images)
-        w, h = _canvas(images[0], apply_transforms)
-        if any(_canvas(im, apply_transforms) != (w, h) for im in images[1:]):
-            raise ValueError("decode_grids packs the images into one (n, H, W, 3) array: all canvases (after rotation) must be equal")
+        xf = [None] * len(images) if transforms is None else list(transforms)
+        sizes = [_canvas(im, apply_transforms, t) for im, t in zip(images, xf)]
+        w, h = sizes[0]
+        if any(s != (w, h) for s in sizes[1:]):
+            raise ValueError("decode_grids packs the images into one (n, H, W, 3) array: all outputs (after the transform) must be equal")
         if out is None:
             out = np.empty((len(images), h, w, 3), np.uint8)
         n_tiles = sum(im.n_tiles for im in images)
         st = (K.TileStatus * n_tiles)()
-        rc = self._lib.heic_b200_decode_grids(self._h, arr, len(images), out.ctypes.data, out.strides[1], out.strides[0],
-                                              1 if apply_transforms else 0, st)
+        if transforms is None:
+            rc = self._lib.heic_b200_decode_grids(self._h, arr, len(images), out.ctypes.data, out.strides[1], out.strides[0],
+                                                  1 if apply_transforms else 0, st)
+        else:
+            rc = self._lib.heic_b200_decode_grids_transformed(self._h, arr, _transform_array(xf, len(images)), len(images),
+                                                              out.ctypes.data, out.strides[1], out.strides[0], st)
         if return_status:
             return out, rc, st
         K.check(rc)
         return out
 
-    def submit_grids(self, images, out: np.ndarray, apply_transforms: bool = False):
+    def submit_grids(self, images, out: np.ndarray, apply_transforms: bool = False, transforms=None):
         """Asynchronous decode_grids: returns a job; call ``wait_job(job)`` before reading ``out``."""
         images = list(images)
         arr = _desc_array(images)
         n_tiles = sum(im.n_tiles for im in images)
         st = (K.TileStatus * n_tiles)()
         job = C.c_void_p()
-        K.check(self._lib.heic_b200_decode_grids_submit(self._h, arr, len(images), out.ctypes.data, out.strides[1], out.strides[0],
-                                                        1 if apply_transforms else 0, st, C.byref(job)))
+        if transforms is None:
+            K.check(self._lib.heic_b200_decode_grids_submit(self._h, arr, len(images), out.ctypes.data, out.strides[1], out.strides[0],
+                                                            1 if apply_transforms else 0, st, C.byref(job)))
+        else:
+            K.check(self._lib.heic_b200_decode_grids_submit_transformed(self._h, arr, _transform_array(transforms, len(images)),
+                                                                        len(images), out.ctypes.data, out.strides[1],
+                                                                        out.strides[0], st, C.byref(job)))
         return (job, st, out)
 
     def unescape(self, nal_payload: bytes, data_offset: int = 0, substream_offsets=()):
@@ -378,8 +438,8 @@ class HeicDecoder:
             co += cw * ch
         return res
 
-    def batch(self, images, apply_transforms: bool = False) -> Batch:
-        return Batch(self, images, apply_transforms)
+    def batch(self, images, apply_transforms: bool = False, transforms=None) -> Batch:
+        return Batch(self, images, apply_transforms, transforms)
 
     def color_stitch(self, dev_planes: int, n_images, grid_rows, grid_cols, tile_w, tile_h, out_w, out_h, dev_rgb: int,
                      pitch: int, image_stride: int, full_range: int = 1, matrix_coeffs: int = 6):

@@ -108,6 +108,12 @@ class ImageDesc(C.Structure):
     ]
 
 
+class ImageTransform(C.Structure):
+    """heic_image_transform: out = canvas[crop_y:crop_y+crop_h, crop_x:crop_x+crop_w], rotated by orientation & 3 ccw quarter
+    turns, then mirrored left<->right when orientation & 4."""
+    _fields_ = _u32_fields("crop_x,crop_y,crop_w,crop_h,orientation")
+
+
 class TileStatus(C.Structure):
     _fields_ = [("code", i32), ("bins_decoded", u32), ("ctus_decoded", u32), ("reserved", u32)]
 
@@ -160,6 +166,7 @@ SYMBOLS = [
     ("heic_b200_file_parameter_set_nal", i32, [_vp, i32, u32, C.POINTER(C.POINTER(u8)), C.POINTER(_sz)]),
     ("heic_b200_file_tile_nal", i32, [_vp, i32, u32, C.POINTER(C.POINTER(u8)), C.POINTER(_sz)]),
     ("heic_b200_file_info", i32, [_vp, C.POINTER(FileInfo)]),
+    ("heic_b200_file_image_transform", i32, [_vp, i32, C.POINTER(ImageTransform)]),
     ("heic_b200_unescape", i32,
      [_vp, C.c_char_p, _sz, u32, C.POINTER(u32), u32, C.POINTER(u8), C.POINTER(_sz), C.POINTER(u32), C.POINTER(u32)]),
     ("heic_b200_decode_grids", i32,
@@ -167,11 +174,16 @@ SYMBOLS = [
     ("heic_b200_decode_grids_submit", i32,
      [_vp, C.POINTER(ImageDesc), u32, _vp, _sz, _sz, i32, C.POINTER(TileStatus), C.POINTER(_vp)]),
     ("heic_b200_job_wait", i32, [_vp]),
+    ("heic_b200_decode_grids_transformed", i32,
+     [_vp, C.POINTER(ImageDesc), C.POINTER(ImageTransform), u32, _vp, _sz, _sz, C.POINTER(TileStatus)]),
+    ("heic_b200_decode_grids_submit_transformed", i32,
+     [_vp, C.POINTER(ImageDesc), C.POINTER(ImageTransform), u32, _vp, _sz, _sz, C.POINTER(TileStatus), C.POINTER(_vp)]),
     ("heic_b200_decode_grids_yuv", i32,
      [_vp, C.POINTER(ImageDesc), u32, _vp, _vp, _vp, C.POINTER(TileStatus)]),
     ("heic_b200_decode_file", i32, [_vp, C.c_char_p, _sz, _vp, _sz, i32]),
     ("heic_b200_batch_create", i32, [_vp, C.POINTER(ImageDesc), u32, C.POINTER(_vp)]),
     ("heic_b200_batch_create_ex", i32, [_vp, C.POINTER(ImageDesc), u32, i32, C.POINTER(_vp)]),
+    ("heic_b200_batch_create_transformed", i32, [_vp, C.POINTER(ImageDesc), C.POINTER(ImageTransform), u32, C.POINTER(_vp)]),
     ("heic_b200_batch_destroy", None, [_vp]),
     ("heic_b200_batch_decode", i32, [_vp]),
     ("heic_b200_batch_run_stages", i32, [_vp, u32]),

@@ -1,6 +1,7 @@
-// Stage 6: YCbCr 4:2:0 -> RGB8 fused with HEIF grid stitching, conformance/canvas crop and (optionally)
-// the irot rotation — one bandwidth-bound pass: 1.5 B read + 3 B written per output pixel.  Unrotated rows leave through
-// shared memory as bulk copies (TMA, cp.async.bulk: UBLKCP in SASS); rotated output is transposed in shared memory.
+// Stage 6: YCbCr 4:2:0 -> RGB8 fused with HEIF grid stitching, conformance windows, the canvas crop and the output geometry
+// (clap crop, irot turns, imir mirrors) — one bandwidth-bound pass: 1.5 B read + 3 B written per output pixel.  Unturned,
+// uncropped rows leave through shared memory as bulk copies (TMA, cp.async.bulk: UBLKCP in SASS); every other geometry is
+// laid down in output orientation in shared memory.
 //
 // The reference's src/color is an ICC-header stub, not a converter (SURVEY 0.3), so the conversion is the
 // frozen integer definition of SURVEY row C1 (libheif-style nearest-neighbour chroma, 8.8 fixed point):
@@ -192,40 +193,96 @@ __global__ void __launch_bounds__(kColorThreads) color_stitch_kernel(ColorJob J,
   }
 }
 
-// irot (ISO/IEC 23008-12 6.5.10: anti-clockwise quarter turns) applied on the way out.  A CTA converts a 64 x 64 tile of the
-// canvas and lays it down ROTATED in shared memory, so that the rows of the rotated picture leave as contiguous runs of
-// 16-byte stores (a per-pixel scatter to HBM wrote 3 bytes per store).  canvas (sx, sy) -> rotated (dx, dy):
+// The 16 x 2 block of convert_block for any geometry, pixel by pixel: any source alignment, blocks that straddle tiles, tiles
+// stitched from inside their conformance window (win_x, win_y).  (x, y): canvas position; nx (1..16) pixels of ny (1..2)
+// rows are converted, the other bytes are zero.  A pixel's chroma is the sample of its 2x2 quad in the tile's decoded
+// picture.  The arithmetic is convert_block's general form (with y_mul = 256, y_sub = 0 it equals the FULL form).
+template <bool FUSED>
+__device__ __forceinline__ void gather_block(const ColorJob& J, const ColorWindow& G, const Coeffs& K, uint32_t image, uint32_t x,
+                                             uint32_t y, uint32_t nx, uint32_t ny, uint32_t (&w)[2][12]) {
+#pragma unroll
+  for (int r = 0; r < 2; r++) {
+#pragma unroll
+    for (int q = 0; q < 12; q++) w[r][q] = 0u;
+    if ((uint32_t)r >= ny) continue;
+    const uint32_t tr = (y + r) / J.tile_h, ly = y + r - tr * J.tile_h + G.win_y;
+    uint32_t tc = x / J.tile_w, lx = x - tc * J.tile_w;  // column inside the tile's window
+#pragma unroll
+    for (int i = 0; i < 16; i++) {
+      if ((uint32_t)i < nx) {
+        const uint32_t ti = image * J.grid_cols * J.grid_rows + tr * J.grid_cols + tc, sx = lx + G.win_x;
+        const uint8_t* t = J.planes + (size_t)ti * J.tile_stride;
+        const uint8_t *ty = t, *tcb = t, *tcr = t;
+        if (FUSED) {  // as in convert_block; the CTB is found in decoded-picture coordinates
+          const uint4 sp = *reinterpret_cast<const uint4*>(J.sao + (size_t)ti * J.sao_stride +
+                                                           (size_t)((ly >> J.log2_ctb) * J.wctb + (sx >> J.log2_ctb)) * 4);
+          const uint8_t* t2 = J.planes_sao + (size_t)ti * J.tile_stride;
+          if (sp.x & 3u) ty = t2;
+          if (sp.y & 3u) tcb = t2;
+          if (sp.z & 3u) tcr = t2;
+        }
+        int c = 0, d = 0;
+        if (J.chroma) {
+          const size_t co = (size_t)(ly >> 1) * J.pitch_c + (sx >> 1);
+          c = (int)tcb[J.cb_off + co] - 128;
+          d = (int)tcr[J.cr_off + co] - 128;
+        }
+        const int yy = K.y_mul * ((int)ty[(size_t)ly * J.pitch_y + sx] - K.y_sub);
+        const uint32_t px[3] = {clip8((yy + K.rv * d + 128) >> 8), clip8((yy + K.gu * c + K.gv * d + 128) >> 8),
+                                clip8((yy + K.bu * c + 128) >> 8)};
+#pragma unroll
+        for (int ch = 0; ch < 3; ch++) w[r][(3 * i + ch) >> 2] |= px[ch] << (8 * ((3 * i + ch) & 3));
+        if (++lx == J.tile_w) lx = 0, tc++;
+      }
+    }
+  }
+}
+
+// Everything color_stitch_kernel does not take: a crop at any offset, any of the 8 orientations of heic_image_transform,
+// tiles stitched from inside a conformance window or at widths that are not multiples of 8.  A CTA converts a 64 x 64 block
+// of the crop rectangle and lays it down in shared memory in output orientation, so that the rows of the output leave as
+// contiguous runs of 16-byte stores (a per-pixel scatter to HBM wrote 3 bytes per store).  Crop position (sx, sy) of a
+// W x H crop -> output (dx, dy), for the quarter turns:
 //   1: (sy, W - 1 - sx)    2: (W - 1 - sx, H - 1 - sy)    3: (H - 1 - sy, sx)
+// and then dx -> (output width) - 1 - dx when the mirror bit is set.
+// aligned: no window offset, crop origin at x % 8 == 0 and y % 2 == 0, stitch seams at multiples of 8 columns and 2 rows,
+// so convert_block's 8-pixel loads apply; otherwise gather_block.
 constexpr int kRotTile = 64;
-constexpr int kRotRowBytes = kRotTile * 3 + 16;  // padded row of the rotated tile (a multiple of 16)
+constexpr int kRotRowBytes = kRotTile * 3 + 16;  // padded row of the oriented block (a multiple of 16)
 
 template <bool FULL, bool FUSED>
-__global__ void __launch_bounds__(kColorThreads) color_rotate_kernel(ColorJob J, Coeffs K, uint32_t tiles_x, uint32_t tiles_y) {
+__global__ void __launch_bounds__(kColorThreads) color_geom_kernel(ColorJob J, ColorWindow G, Coeffs K, uint32_t tiles_x, uint32_t tiles_y,
+                                                                   uint32_t aligned) {
   __shared__ __align__(16) uint8_t tile[kRotTile * kRotRowBytes];
   const uint32_t per_image = tiles_x * tiles_y;
   const uint32_t image = blockIdx.x / per_image, rem = blockIdx.x % per_image;
-  const uint32_t x0 = (rem % tiles_x) * kRotTile, y0 = (rem / tiles_x) * kRotTile;
-  const uint32_t w_v = min((uint32_t)kRotTile, J.out_w - x0), h_v = min((uint32_t)kRotTile, J.out_h - y0);  // valid part of the tile
-  // a warp takes a 16-pixel column strip of the tile, a lane two of its rows
+  const uint32_t x0 = (rem % tiles_x) * kRotTile, y0 = (rem / tiles_x) * kRotTile;  // block origin in the crop
+  const uint32_t w_v = min((uint32_t)kRotTile, G.crop_w - x0), h_v = min((uint32_t)kRotTile, G.crop_h - y0);  // valid part
+  // a warp takes a 16-pixel column strip of the block, a lane two of its rows
   const uint32_t lx = (threadIdx.x >> 5) * 16, ly = (threadIdx.x & 31) * 2;
-  const uint32_t rot = J.rotation;
+  const uint32_t rot = J.orientation & 3u;
+  const bool mir = (J.orientation & 4u) != 0;
+  const uint32_t n_cols = (rot & 1u) ? h_v : w_v, n_rows = (rot & 1u) ? w_v : h_v;  // the block in output orientation
   if (lx < w_v && ly < h_v) {
     const bool two_rows = ly + 1 < h_v;
+    const uint32_t cx = G.crop_x + x0 + lx, cy = G.crop_y + y0 + ly;
     uint32_t w[2][12];
-    convert_block<FULL, FUSED>(J, K, image, x0 + lx, y0 + ly, y0 + ly + 1 < J.out_h, w);
+    if (aligned) convert_block<FULL, FUSED>(J, K, image, cx, cy, cy + 1 < J.out_h, w);
+    else gather_block<FUSED>(J, G, K, image, cx, cy, min(16u, w_v - lx), two_rows ? 2u : 1u, w);
     // byte b (0..47) of row r's 48 bytes of RGB
 #define HEIC_RGB_BYTE(r, b) ((w[r][(b) >> 2] >> (8 * ((b) & 3))) & 0xffu)
     // two such bytes as one 16-bit value (low byte first): one PRMT
 #define HEIC_RGB_PAIR(ra, ba, rb, bb) __byte_perm(w[ra][(ba) >> 2], w[rb][(bb) >> 2], ((ba) & 3) | ((4 + ((bb) & 3)) << 4))
-    if (two_rows && lx + 16 <= w_v && rot != 2 && !(h_v & 1u)) {
-      // quarter turns: the two rows of a column are two neighbouring pixels of one rotated row -- six contiguous bytes at an
-      // even address, written as three 16-bit stores (rot 3: the lower canvas row comes first, rot 1: the upper one)
+    if ((rot & 1u) && two_rows && lx + 16 <= w_v && !(h_v & 1u)) {
+      // odd quarter turns: the two rows of a column are two neighbouring pixels of one output row -- six contiguous bytes
+      // at an even address, written as three 16-bit stores, the upper canvas row first for turn 1 and for turn 3 mirrored
+      const bool upper_first = (rot == 1u) != mir;
+      const uint32_t col = upper_first ? ly : h_v - 2 - ly;
 #pragma unroll
       for (int i = 0; i < 16; i++) {
         const uint32_t sx = lx + i;
-        uint8_t* o = rot == 1 ? tile + (w_v - 1 - sx) * kRotRowBytes + ly * 3 : tile + sx * kRotRowBytes + (h_v - 2 - ly) * 3;
-        uint16_t* o16 = reinterpret_cast<uint16_t*>(o);
-        if (rot == 1) {
+        uint16_t* o16 = reinterpret_cast<uint16_t*>(tile + (rot == 1u ? w_v - 1 - sx : sx) * kRotRowBytes + col * 3);
+        if (upper_first) {
           o16[0] = (uint16_t)HEIC_RGB_PAIR(0, 3 * i, 0, 3 * i + 1);
           o16[1] = (uint16_t)HEIC_RGB_PAIR(0, 3 * i + 2, 1, 3 * i);
           o16[2] = (uint16_t)HEIC_RGB_PAIR(1, 3 * i + 1, 1, 3 * i + 2);
@@ -234,6 +291,17 @@ __global__ void __launch_bounds__(kColorThreads) color_rotate_kernel(ColorJob J,
           o16[1] = (uint16_t)HEIC_RGB_PAIR(1, 3 * i + 2, 0, 3 * i);
           o16[2] = (uint16_t)HEIC_RGB_PAIR(0, 3 * i + 1, 0, 3 * i + 2);
         }
+      }
+    } else if (((rot == 0 && !mir) || (rot == 2 && mir)) && lx + 16 <= w_v) {
+      // unturned, or flipped top <-> bottom: the thread's 48 bytes of each row stay contiguous and in order (and 16-byte
+      // aligned: lx * 3 is a multiple of 48)
+#pragma unroll
+      for (int r = 0; r < 2; r++) {
+        if (r == 1 && !two_rows) break;
+        uint4* s = reinterpret_cast<uint4*>(tile + (rot == 0 ? ly + r : h_v - 1 - ly - r) * kRotRowBytes + lx * 3);
+        s[0] = make_uint4(w[r][0], w[r][1], w[r][2], w[r][3]);
+        s[1] = make_uint4(w[r][4], w[r][5], w[r][6], w[r][7]);
+        s[2] = make_uint4(w[r][8], w[r][9], w[r][10], w[r][11]);
       }
     } else {
 #pragma unroll
@@ -244,10 +312,12 @@ __global__ void __launch_bounds__(kColorThreads) color_rotate_kernel(ColorJob J,
         for (int i = 0; i < 16; i++) {
           const uint32_t sx = lx + i;
           if (sx < w_v) {
-            uint32_t row, col;  // position inside the rotated tile
-            if (rot == 1) row = w_v - 1 - sx, col = sy;
+            uint32_t row, col;  // position inside the oriented block
+            if (rot == 0) row = sy, col = sx;
+            else if (rot == 1) row = w_v - 1 - sx, col = sy;
             else if (rot == 2) row = h_v - 1 - sy, col = w_v - 1 - sx;
             else row = sx, col = h_v - 1 - sy;
+            if (mir) col = n_cols - 1 - col;
             uint8_t* o = tile + row * kRotRowBytes + col * 3;
             o[0] = (uint8_t)HEIC_RGB_BYTE(r, 3 * i);
             o[1] = (uint8_t)HEIC_RGB_BYTE(r, 3 * i + 1);
@@ -260,11 +330,14 @@ __global__ void __launch_bounds__(kColorThreads) color_rotate_kernel(ColorJob J,
 #undef HEIC_RGB_PAIR
   }
   __syncthreads();
-  // rotated tile -> HBM
-  uint32_t n_rows, n_cols, dx0, dy0;
-  if (rot == 1) n_rows = w_v, n_cols = h_v, dx0 = y0, dy0 = J.out_w - x0 - w_v;
-  else if (rot == 2) n_rows = h_v, n_cols = w_v, dx0 = J.out_w - x0 - w_v, dy0 = J.out_h - y0 - h_v;
-  else n_rows = w_v, n_cols = h_v, dx0 = J.out_h - y0 - h_v, dy0 = x0;
+  // oriented block -> HBM
+  const uint32_t W = G.crop_w, H = G.crop_h;
+  uint32_t dx0, dy0;
+  if (rot == 0) dx0 = x0, dy0 = y0;
+  else if (rot == 1) dx0 = y0, dy0 = W - x0 - w_v;
+  else if (rot == 2) dx0 = W - x0 - w_v, dy0 = H - y0 - h_v;
+  else dx0 = H - y0 - h_v, dy0 = x0;
+  if (mir) dx0 = ((rot & 1u) ? H : W) - dx0 - n_cols;
   uint8_t* dst = J.rgb + (size_t)image * J.image_stride + (size_t)dy0 * J.pitch + (size_t)dx0 * 3;
   const uint32_t row_bytes = n_cols * 3;
   if (((row_bytes | (uint32_t)J.pitch | (uint32_t)((uintptr_t)dst)) & 15u) == 0) {
@@ -283,8 +356,8 @@ __global__ void __launch_bounds__(kColorThreads) color_rotate_kernel(ColorJob J,
 
 }  // namespace
 
-cudaError_t launch_color(const ColorJob& job, cudaStream_t stream) {
-  if (!job.n_images || !job.out_w || !job.out_h) return cudaSuccess;
+cudaError_t launch_color(const ColorJob& job, const ColorWindow& win, cudaStream_t stream) {
+  if (!job.n_images || !job.out_w || !job.out_h || !win.crop_w || !win.crop_h) return cudaSuccess;
   Coeffs k;
   const bool bt709 = job.matrix_coeffs == 1;
   if (job.full_range) {
@@ -298,28 +371,35 @@ cudaError_t launch_color(const ColorJob& job, cudaStream_t stream) {
     if (bt709) k.rv = 459, k.gu = -55, k.gv = -136, k.bu = 541;
     else k.rv = 409, k.gu = -100, k.gv = -208, k.bu = 516;
   }
-  const uint32_t groups = (job.out_w + 15) / 16;
-  const uint32_t xblocks = (groups + kColorThreads - 1) / kColorThreads, row_pairs = (job.out_h + 1) / 2;
-  const unsigned grid = job.n_images * row_pairs * xblocks;
-  // bulk (TMA) stores need 16-byte aligned rows whose length is a multiple of 16 bytes
-  const bool bulk = job.rotation == 0 && job.out_w % 16 == 0 && job.pitch % 16 == 0 && job.image_stride % 16 == 0 &&
-                    ((uintptr_t)job.rgb & 15u) == 0;
-  if (job.rotation != 0) {
-    const uint32_t tiles_x = (job.out_w + kRotTile - 1) / kRotTile, tiles_y = (job.out_h + kRotTile - 1) / kRotTile;
+  // seams between tiles at multiples of 8 columns and of 2 rows (or none): the first and the second 8 pixels of a
+  // 16-pixel group may lie in different tiles, not within one, and the two rows of a thread lie in one tile
+  const bool seams = (job.tile_w % 8 == 0 || job.grid_cols == 1) && (job.tile_h % 2 == 0 || job.grid_rows == 1);
+  if (job.orientation != 0 || win.crop_x || win.crop_y || win.win_x || win.win_y || !seams) {
+    const uint32_t tiles_x = (win.crop_w + kRotTile - 1) / kRotTile, tiles_y = (win.crop_h + kRotTile - 1) / kRotTile;
     const unsigned rgrid = job.n_images * tiles_x * tiles_y;
+    const uint32_t aligned = !win.win_x && !win.win_y && seams && win.crop_x % 8 == 0 && win.crop_y % 2 == 0;
     if (job.fused) {
-      if (job.full_range) color_rotate_kernel<true, true><<<rgrid, kColorThreads, 0, stream>>>(job, k, tiles_x, tiles_y);
-      else color_rotate_kernel<false, true><<<rgrid, kColorThreads, 0, stream>>>(job, k, tiles_x, tiles_y);
+      if (job.full_range) color_geom_kernel<true, true><<<rgrid, kColorThreads, 0, stream>>>(job, win, k, tiles_x, tiles_y, aligned);
+      else color_geom_kernel<false, true><<<rgrid, kColorThreads, 0, stream>>>(job, win, k, tiles_x, tiles_y, aligned);
     } else {
-      if (job.full_range) color_rotate_kernel<true, false><<<rgrid, kColorThreads, 0, stream>>>(job, k, tiles_x, tiles_y);
-      else color_rotate_kernel<false, false><<<rgrid, kColorThreads, 0, stream>>>(job, k, tiles_x, tiles_y);
+      if (job.full_range) color_geom_kernel<true, false><<<rgrid, kColorThreads, 0, stream>>>(job, win, k, tiles_x, tiles_y, aligned);
+      else color_geom_kernel<false, false><<<rgrid, kColorThreads, 0, stream>>>(job, win, k, tiles_x, tiles_y, aligned);
     }
     return cudaGetLastError();
   }
+  // the crop is a top-left part of the canvas: the stitch kernel, with the crop as its canvas
+  ColorJob j = job;
+  j.out_w = win.crop_w;
+  j.out_h = win.crop_h;
+  const uint32_t groups = (j.out_w + 15) / 16;
+  const uint32_t xblocks = (groups + kColorThreads - 1) / kColorThreads, row_pairs = (j.out_h + 1) / 2;
+  const unsigned grid = j.n_images * row_pairs * xblocks;
+  // bulk (TMA) stores need 16-byte aligned rows whose length is a multiple of 16 bytes
+  const bool bulk = j.out_w % 16 == 0 && j.pitch % 16 == 0 && j.image_stride % 16 == 0 && ((uintptr_t)j.rgb & 15u) == 0;
 #define HEIC_COLOR_LAUNCH(FULL, FUSED)                                                                                  \
   do {                                                                                                                  \
-    if (bulk) color_stitch_kernel<FULL, FUSED, true><<<grid, kColorThreads, 0, stream>>>(job, k, row_pairs, xblocks);   \
-    else color_stitch_kernel<FULL, FUSED, false><<<grid, kColorThreads, 0, stream>>>(job, k, row_pairs, xblocks);       \
+    if (bulk) color_stitch_kernel<FULL, FUSED, true><<<grid, kColorThreads, 0, stream>>>(j, k, row_pairs, xblocks);     \
+    else color_stitch_kernel<FULL, FUSED, false><<<grid, kColorThreads, 0, stream>>>(j, k, row_pairs, xblocks);         \
   } while (0)
   if (job.fused) {
     if (job.full_range) HEIC_COLOR_LAUNCH(true, true);

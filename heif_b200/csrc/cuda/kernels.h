@@ -43,19 +43,19 @@ cudaError_t launch_sao(const Arenas& A, uint32_t max_pitch, uint32_t max_h, cuda
 // runs, followed by a colour kernel that picks every CTB's component from the arena holding its final samples.
 cudaError_t launch_sao_sparse(const Arenas& A, int max_hctb, cudaStream_t stream);
 
-// Stage 6 — YCbCr 4:2:0 -> RGB8 + grid stitch + crop (+ irot).
+// Stage 6 — YCbCr 4:2:0 -> RGB8 + grid stitch + crop (+ orientation).
 struct ColorJob {
   const uint8_t* planes;        // tile t: planes + t * tile_stride; Y then Cb then Cr
   uint64_t tile_stride;         // bytes between tiles
   uint64_t cb_off, cr_off;      // offsets of Cb / Cr inside a tile
   uint32_t pitch_y, pitch_c;
-  uint32_t tile_w, tile_h;      // decoded picture size of a tile
+  uint32_t tile_w, tile_h;      // size at which the grid stitches a tile (its conformance window)
   uint32_t grid_cols, grid_rows;
-  uint32_t out_w, out_h;        // canvas (before rotation)
+  uint32_t out_w, out_h;        // canvas (before the crop and the orientation)
   uint32_t n_images;            // images are consecutive groups of grid_cols*grid_rows tiles
   uint32_t chroma;              // 0: monochrome (Cb = Cr = 128)
   uint32_t full_range, matrix_coeffs;
-  uint32_t rotation;            // ccw quarter turns applied to the output
+  uint32_t orientation;         // heic_image_transform::orientation applied to the output
   uint8_t* rgb;
   uint64_t pitch, image_stride; // output layout in bytes
   // fused == 1: `planes` is the deblocked reconstruction, and a CTB component whose SAO type is non-zero is read from
@@ -66,7 +66,15 @@ struct ColorJob {
   uint32_t sao_stride;          // words between tiles
   uint32_t log2_ctb, wctb;
 };
-cudaError_t launch_color(const ColorJob& job, cudaStream_t stream);
+// The rest of the output geometry.  It travels beside ColorJob rather than inside it: the stitch kernel takes ColorJob by
+// value, and a longer ColorJob would move the kernel parameters after it.
+struct ColorWindow {
+  uint32_t crop_x, crop_y, crop_w, crop_h;  // output rectangle in canvas coordinates, before the orientation
+  uint32_t win_x, win_y;                    // origin of a tile's stitched part inside its decoded picture (luma samples)
+};
+// Identity orientation, crop and window at the origin, tiles stitched at multiples of 8 pixels: color_stitch_kernel.
+// Everything else: color_geom_kernel.
+cudaError_t launch_color(const ColorJob& job, const ColorWindow& win, cudaStream_t stream);
 
 }  // namespace dev
 }  // namespace heic

@@ -138,9 +138,60 @@ struct heic_b200_ctx {
 
 struct ImageInfo {
   uint32_t first_tile, n_tiles, pic;
-  uint32_t grid_rows, grid_cols, out_w, out_h, rot_w, rot_h, rotation;
+  uint32_t grid_rows, grid_cols, out_w, out_h, rot_w, rot_h;
+  uint32_t tile_w, tile_h, win_x, win_y;                    // conformance window of every tile (luma samples)
+  uint32_t crop_x, crop_y, crop_w, crop_h, orientation;     // heic_image_transform
   uint32_t full_range, matrix_coeffs;
 };
+
+namespace {
+
+// The part of a decoded picture that a grid stitches: its conformance window, in luma samples.
+struct TileWindow {
+  uint32_t x, y, w, h;
+};
+
+// Decoded picture, conformance window and output canvas of an image descriptor; throws for a window or a canvas that
+// the tiles do not cover.
+void image_geometry(const heic_image_desc& im, PicParams& pp, TileWindow& tw, uint32_t& out_w, uint32_t& out_h) {
+  if (!im.tiles || im.n_tiles == 0 || im.n_tiles != im.grid_rows * im.grid_cols)
+    bail(HEIC_E_INVALID_ARG, "image descriptor: n_tiles must equal grid_rows * grid_cols");
+  make_pic_params(im.sps, im.pps, pp);
+  tw = {0, 0, (uint32_t)pp.w, (uint32_t)pp.h};
+  if (im.sps.conformance_window_flag) {
+    const uint64_t sub = pp.chroma ? 2 : 1;  // SubWidthC = SubHeightC: 4:2:0 or 4:0:0 (make_pic_params rejects the rest)
+    const uint64_t l = sub * im.sps.conf_win_left_offset, r = sub * im.sps.conf_win_right_offset;
+    const uint64_t t = sub * im.sps.conf_win_top_offset, b = sub * im.sps.conf_win_bottom_offset;
+    if (l + r >= (uint64_t)pp.w || t + b >= (uint64_t)pp.h) bail(HEIC_E_BITSTREAM, "conformance window is empty");
+    tw = {(uint32_t)l, (uint32_t)t, (uint32_t)(pp.w - l - r), (uint32_t)(pp.h - t - b)};
+  }
+  const uint64_t mosaic_w = (uint64_t)im.grid_cols * tw.w, mosaic_h = (uint64_t)im.grid_rows * tw.h;
+  const uint64_t ow = im.output_width ? im.output_width : mosaic_w, oh = im.output_height ? im.output_height : mosaic_h;
+  if (ow > mosaic_w || oh > mosaic_h) bail(HEIC_E_BITSTREAM, "grid canvas is larger than the tile mosaic");
+  out_w = (uint32_t)ow;
+  out_h = (uint32_t)oh;
+}
+
+void check_transform(const heic_image_transform& x, uint32_t out_w, uint32_t out_h) {
+  if (x.orientation > 7 || !x.crop_w || !x.crop_h || (uint64_t)x.crop_x + x.crop_w > out_w || (uint64_t)x.crop_y + x.crop_h > out_h)
+    bail(HEIC_E_INVALID_ARG, "image transform: crop rectangle not inside the canvas, or orientation above 7");
+}
+
+// What the calls without transforms apply: the whole canvas, turned by irot when apply_transforms is set.
+std::vector<heic_image_transform> canvas_transforms(const heic_image_desc* imgs, uint32_t n_imgs, int32_t apply_transforms) {
+  if (!imgs) bail(HEIC_E_INVALID_ARG, "null argument");
+  std::vector<heic_image_transform> x(n_imgs);
+  for (uint32_t i = 0; i < n_imgs; i++) {
+    PicParams pp;
+    TileWindow tw;
+    uint32_t ow, oh;
+    image_geometry(imgs[i], pp, tw, ow, oh);
+    x[i] = {0, 0, ow, oh, apply_transforms ? (imgs[i].rotation_ccw_quarter_turns & 3u) : 0u};
+  }
+  return x;
+}
+
+}  // namespace
 
 struct CabacClass {  // tiles launched together: same wavefront shape
   int n_slots, hctb;
@@ -151,7 +202,6 @@ struct heic_b200_batch {
   heic_b200_ctx* ctx = nullptr;
   cudaStream_t stream = nullptr;  // ctx->stream for explicit batches, a pipeline stream for decode_grids chunks
   int tiles_per_cta = 32;         // CABAC mapping of this load: 32 (throughput) or 1 (lowest latency, small loads)
-  bool apply_transforms = false;
   std::vector<PicParams> pics;
   std::vector<ScalingSet> scaling;
   std::vector<TileParams> tiles;
@@ -198,7 +248,7 @@ struct heic_b200_batch {
     for (int k = 0; k < LIST_CLASSES; k++) a.list_off[k] = list_off[k];
     return a;
   }
-  void load(const heic_image_desc* imgs, uint32_t n_imgs, bool with_rgb);
+  void load(const heic_image_desc* imgs, const heic_image_transform* xforms, uint32_t n_imgs, bool with_rgb);
   void run(uint32_t mask);
 };
 
@@ -217,7 +267,7 @@ heic_b200_ctx::~heic_b200_ctx() {
 }
 
 // ---- batch construction --------------------------------------------------------------------------------
-void heic_b200_batch::load(const heic_image_desc* imgs, uint32_t n_imgs, bool with_rgb) {
+void heic_b200_batch::load(const heic_image_desc* imgs, const heic_image_transform* xforms, uint32_t n_imgs, bool with_rgb) {
   pics.clear();
   scaling.clear();
   tiles.clear();
@@ -235,20 +285,18 @@ void heic_b200_batch::load(const heic_image_desc* imgs, uint32_t n_imgs, bool wi
   intra_slots = 1;
   max_hctb = 1;
   stages_run = 0;
-  size_t max_rgb_bytes = 0, max_rgb_pitch = 0, n_tiles_hint = 0;
+  size_t max_rgb_rows = 0, max_rgb_pitch = 0, n_tiles_hint = 0;
   for (uint32_t i = 0; i < n_imgs; i++) n_tiles_hint += imgs[i].n_tiles;
   for (uint32_t i = 0; i < n_imgs; i++) {
     const heic_image_desc& im = imgs[i];
     if (!im.tiles || im.n_tiles == 0 || im.n_tiles != im.grid_rows * im.grid_cols)
       bail(HEIC_E_INVALID_ARG, "image descriptor: n_tiles must equal grid_rows * grid_cols");
     PicParams pp;
-    make_pic_params(im.sps, im.pps, pp);
-    // The colour/stitch stage crops from the picture origin: a conformance window is honoured when it only trims the
-    // right / bottom of a single picture (the canvas size does that); anything else would shift or mis-stitch the image.
-    if (im.sps.conformance_window_flag &&
-        (im.sps.conf_win_left_offset || im.sps.conf_win_top_offset ||
-         (im.n_tiles > 1 && (im.sps.conf_win_right_offset || im.sps.conf_win_bottom_offset))))
-      bail(HEIC_E_UNSUPPORTED, "conformance window with a left/top offset, or cropped grid tiles, is not supported");
+    TileWindow win;
+    uint32_t out_w, out_h;
+    image_geometry(im, pp, win, out_w, out_h);
+    const heic_image_transform& xf = xforms[i];
+    check_transform(xf, out_w, out_h);
     ScalingSet ss;
     build_scaling_set(im.sps, im.pps, ss);
     size_t s = 0;
@@ -265,19 +313,25 @@ void heic_b200_batch::load(const heic_image_desc* imgs, uint32_t n_imgs, bool wi
     info.pic = pic;
     info.grid_rows = im.grid_rows;
     info.grid_cols = im.grid_cols;
-    info.out_w = im.output_width ? im.output_width : im.grid_cols * (uint32_t)pp.w;
-    info.out_h = im.output_height ? im.output_height : im.grid_rows * (uint32_t)pp.h;
-    if (info.out_w > im.grid_cols * (uint32_t)pp.w || info.out_h > im.grid_rows * (uint32_t)pp.h)
-      bail(HEIC_E_BITSTREAM, "grid canvas is larger than the tile mosaic");
-    info.rotation = apply_transforms ? (im.rotation_ccw_quarter_turns & 3u) : 0u;
-    info.rot_w = (info.rotation & 1u) ? info.out_h : info.out_w;
-    info.rot_h = (info.rotation & 1u) ? info.out_w : info.out_h;
+    info.out_w = out_w;
+    info.out_h = out_h;
+    info.tile_w = win.w;
+    info.tile_h = win.h;
+    info.win_x = win.x;
+    info.win_y = win.y;
+    info.crop_x = xf.crop_x;
+    info.crop_y = xf.crop_y;
+    info.crop_w = xf.crop_w;
+    info.crop_h = xf.crop_h;
+    info.orientation = xf.orientation;
+    info.rot_w = (xf.orientation & 1u) ? xf.crop_h : xf.crop_w;
+    info.rot_h = (xf.orientation & 1u) ? xf.crop_w : xf.crop_h;
     info.full_range = im.sps.vui_parameters_present_flag ? im.sps.video_full_range_flag : 0u;
     info.matrix_coeffs = im.sps.vui_parameters_present_flag ? im.sps.matrix_coeffs : 2u;
     images.push_back(info);
     const size_t pitch = up((size_t)info.rot_w * 3, 16);
     max_rgb_pitch = std::max(max_rgb_pitch, pitch);
-    max_rgb_bytes = std::max(max_rgb_bytes, pitch * info.rot_h);
+    max_rgb_rows = std::max(max_rgb_rows, (size_t)info.rot_h);
     const int ctb4 = 1 << (pp.log2_ctb - 2);
     for (uint32_t t = 0; t < im.n_tiles; t++) {
       TileParams tp;
@@ -331,7 +385,8 @@ void heic_b200_batch::load(const heic_image_desc* imgs, uint32_t n_imgs, bool wi
     intra_slots = std::max(intra_slots, std::min(8, std::min(pp.hctb, (pp.wctb + 1) / 2 + 1)));
   }
   rgb_pitch = max_rgb_pitch;
-  rgb_image_stride = up(max_rgb_bytes, 256);
+  // every image is written at the widest pitch: the stride holds the tallest image at that pitch
+  rgb_image_stride = up(max_rgb_pitch * max_rgb_rows, 256);
   if (tiles.size() >= (1u << 24)) bail(HEIC_E_UNSUPPORTED, "more than 2^24 tiles in one batch (the transform lists keep the tile index in 24 bits)");
 
   // ---- CABAC launch classes: tiles with the same wavefront shape, heaviest first, TILES per CTA ----------
@@ -584,8 +639,9 @@ void heic_b200_batch::run(uint32_t mask) {
       size_t j = i + 1;
       auto same = [&](const ImageInfo& a, const ImageInfo& b) {
         return a.pic == b.pic && a.n_tiles == b.n_tiles && a.grid_cols == b.grid_cols && a.out_w == b.out_w &&
-               a.out_h == b.out_h && a.rotation == b.rotation && a.full_range == b.full_range &&
-               a.matrix_coeffs == b.matrix_coeffs;
+               a.out_h == b.out_h && a.tile_w == b.tile_w && a.tile_h == b.tile_h && a.win_x == b.win_x && a.win_y == b.win_y &&
+               a.crop_x == b.crop_x && a.crop_y == b.crop_y && a.crop_w == b.crop_w && a.crop_h == b.crop_h &&
+               a.orientation == b.orientation && a.full_range == b.full_range && a.matrix_coeffs == b.matrix_coeffs;
       };
       while (j < images.size() && same(images[i], images[j])) j++;
       const ImageInfo& im = images[i];
@@ -606,8 +662,8 @@ void heic_b200_batch::run(uint32_t mask) {
       job.cr_off = t0.plane_off[2] - t0.plane_off[0];
       job.pitch_y = (uint32_t)pp.pitch_y;
       job.pitch_c = (uint32_t)pp.pitch_c;
-      job.tile_w = (uint32_t)pp.w;
-      job.tile_h = (uint32_t)pp.h;
+      job.tile_w = im.tile_w;
+      job.tile_h = im.tile_h;
       job.grid_cols = im.grid_cols;
       job.grid_rows = im.grid_rows;
       job.out_w = im.out_w;
@@ -616,11 +672,12 @@ void heic_b200_batch::run(uint32_t mask) {
       job.chroma = (uint32_t)pp.chroma;
       job.full_range = im.full_range;
       job.matrix_coeffs = im.matrix_coeffs;
-      job.rotation = im.rotation;
+      job.orientation = im.orientation;
       job.rgb = (uint8_t*)d_rgb.p + i * rgb_image_stride;
       job.pitch = rgb_pitch;
       job.image_stride = rgb_image_stride;
-      CU(launch_color(job, st));
+      const ColorWindow win = {im.crop_x, im.crop_y, im.crop_w, im.crop_h, im.win_x, im.win_y};
+      CU(launch_color(job, win, st));
       ctx->launches++;
       i = j;
     }
@@ -702,21 +759,32 @@ int32_t heic_b200_batch_create(heic_b200_ctx* ctx, const heic_image_desc* imgs, 
   return heic_b200_batch_create_ex(ctx, imgs, n_imgs, 0, out);
 }
 
+static int64_t batch_create(heic_b200_ctx* ctx, const heic_image_desc* imgs, const heic_image_transform* xforms, uint32_t n_imgs,
+                            heic_b200_batch** out) {
+  if (!ctx || !imgs || !xforms || !out || !n_imgs) bail(HEIC_E_INVALID_ARG, "null argument");
+  *out = nullptr;
+  CU(cudaSetDevice(ctx->device));
+  auto b = std::make_unique<heic_b200_batch>();
+  b->ctx = ctx;
+  b->stream = ctx->stream;
+  b->load(imgs, xforms, n_imgs, true);
+  CU(cudaStreamSynchronize(ctx->stream));
+  *out = b.release();
+  return 0;
+}
+
 int32_t heic_b200_batch_create_ex(heic_b200_ctx* ctx, const heic_image_desc* imgs, uint32_t n_imgs, int32_t apply_transforms,
                                   heic_b200_batch** out) {
   return static_cast<int32_t>(guard([&]() -> int64_t {
     if (!ctx || !imgs || !out || !n_imgs) bail(HEIC_E_INVALID_ARG, "null argument");
     *out = nullptr;
-    CU(cudaSetDevice(ctx->device));
-    auto b = std::make_unique<heic_b200_batch>();
-    b->ctx = ctx;
-    b->stream = ctx->stream;
-    b->apply_transforms = apply_transforms != 0;
-    b->load(imgs, n_imgs, true);
-    CU(cudaStreamSynchronize(ctx->stream));
-    *out = b.release();
-    return 0;
+    return batch_create(ctx, imgs, canvas_transforms(imgs, n_imgs, apply_transforms).data(), n_imgs, out);
   }));
+}
+
+int32_t heic_b200_batch_create_transformed(heic_b200_ctx* ctx, const heic_image_desc* imgs, const heic_image_transform* xforms,
+                                           uint32_t n_imgs, heic_b200_batch** out) {
+  return static_cast<int32_t>(guard([&]() -> int64_t { return batch_create(ctx, imgs, xforms, n_imgs, out); }));
 }
 
 void heic_b200_batch_destroy(heic_b200_batch* b) {
@@ -887,26 +955,27 @@ static void harvest_slot(heic_b200_ctx* ctx, int slot) {
   pd.job = nullptr;
 }
 
-static heic_b200_job* submit_grids(heic_b200_ctx* ctx, const heic_image_desc* imgs, uint32_t n_imgs, uint8_t* rgb_out,
-                                   size_t pitch, size_t image_stride, int32_t apply_transforms, uint8_t* y_out,
+// xforms: one output geometry per image (RGB output; ignored for the planar output, which applies none)
+static heic_b200_job* submit_grids(heic_b200_ctx* ctx, const heic_image_desc* imgs, const heic_image_transform* xforms,
+                                   uint32_t n_imgs, uint8_t* rgb_out, size_t pitch, size_t image_stride, uint8_t* y_out,
                                    uint8_t* cb_out, uint8_t* cr_out, heic_tile_status* status) {
-  if (!ctx || !imgs || !n_imgs) bail(HEIC_E_INVALID_ARG, "null argument");
+  if (!ctx || !imgs || !xforms || !n_imgs) bail(HEIC_E_INVALID_ARG, "null argument");
   CU(cudaSetDevice(ctx->device));
   // validate every descriptor before any work is queued, so a bad image rejects the call as a whole
   std::vector<size_t> first_tile(n_imgs + 1, 0), y_off(n_imgs + 1, 0), c_off(n_imgs + 1, 0);
   for (uint32_t i = 0; i < n_imgs; i++) {
     const heic_image_desc& im = imgs[i];
-    if (!im.tiles || im.n_tiles == 0 || im.n_tiles != im.grid_rows * im.grid_cols)
-      bail(HEIC_E_INVALID_ARG, "image descriptor: n_tiles must equal grid_rows * grid_cols");
     PicParams pp;
-    make_pic_params(im.sps, im.pps, pp);
+    TileWindow win;
+    uint32_t out_w, out_h;
+    image_geometry(im, pp, win, out_w, out_h);
+    check_transform(xforms[i], out_w, out_h);
     TileParams tp;
     for (uint32_t t = 0; t < im.n_tiles; t++) make_tile_params(pp, im.pps, im.tiles[t], tp);
-    const size_t ow = im.output_width ? im.output_width : (size_t)im.grid_cols * pp.w;
-    const size_t oh = im.output_height ? im.output_height : (size_t)im.grid_rows * pp.h;
+    const size_t ow = out_w, oh = out_h;
     if (rgb_out) {  // the caller's buffer layout, checked for every image before anything is queued
-      const bool turn = apply_transforms && (im.rotation_ccw_quarter_turns & 1u);
-      const size_t rw = turn ? oh : ow, rh = turn ? ow : oh;
+      const bool turn = xforms[i].orientation & 1u;
+      const size_t rw = turn ? xforms[i].crop_h : xforms[i].crop_w, rh = turn ? xforms[i].crop_w : xforms[i].crop_h;
       if (pitch < rw * 3) bail(HEIC_E_INVALID_ARG, "output pitch smaller than a row of RGB");
       if (n_imgs > 1 && rh * pitch > image_stride) bail(HEIC_E_INVALID_ARG, "image_stride smaller than one image (rows x pitch)");
     }
@@ -962,9 +1031,8 @@ static heic_b200_job* submit_grids(heic_b200_ctx* ctx, const heic_image_desc* im
     t_wait += ms_since(t0);
     heic_b200_batch* b = ctx->pipe_batch[slot].get();
     cudaStream_t st = b->stream;
-    b->apply_transforms = apply_transforms != 0;
     t0 = clk::now();
-    b->load(imgs + i0, cnt, rgb_out != nullptr);
+    b->load(imgs + i0, xforms + i0, cnt, rgb_out != nullptr);
     t_load += ms_since(t0);
     t0 = clk::now();
     PipePending& pend = ctx->pipe_pending[slot];
@@ -1015,25 +1083,28 @@ static heic_b200_job* submit_grids(heic_b200_ctx* ctx, const heic_image_desc* im
         }
       }
     } else {
-      // planar output: tile mosaic cropped to the canvas, images back to back
+      // planar output: tile mosaic (each tile's conformance window) cropped to the canvas, images back to back
       for (size_t i = 0; i < b->images.size(); i++) {
         const ImageInfo& im = b->images[i];
         const PicParams& pp = b->pics[im.pic];
         const size_t yo = y_off[i0 + i], co = c_off[i0 + i];
         const size_t cw = (im.out_w + 1) / 2, chh = (im.out_h + 1) / 2;
+        const uint8_t* fin = (const uint8_t*)b->d_final.p;
         for (uint32_t t = 0; t < im.n_tiles; t++) {
           const TileParams& tp = b->tiles[im.first_tile + t];
-          const size_t tx = (size_t)(t % im.grid_cols) * pp.w, ty = (size_t)(t / im.grid_cols) * pp.h;
+          const size_t tx = (size_t)(t % im.grid_cols) * im.tile_w, ty = (size_t)(t / im.grid_cols) * im.tile_h;
           if (tx >= im.out_w || ty >= im.out_h) continue;
-          const size_t w = std::min<size_t>(pp.w, im.out_w - tx), h = std::min<size_t>(pp.h, im.out_h - ty);
-          CU(cudaMemcpy2DAsync(y_out + yo + ty * im.out_w + tx, im.out_w, (const uint8_t*)b->d_final.p + tp.plane_off[0],
-                               pp.pitch_y, w, h, cudaMemcpyDeviceToHost, st));
-          if (pp.chroma && cb_out && cr_out) {
-            const size_t wc = std::min<size_t>(pp.w / 2, cw - tx / 2), hc = std::min<size_t>(pp.h / 2, chh - ty / 2);
-            CU(cudaMemcpy2DAsync(cb_out + co + (ty / 2) * cw + tx / 2, cw, (const uint8_t*)b->d_final.p + tp.plane_off[1],
-                                 pp.pitch_c, wc, hc, cudaMemcpyDeviceToHost, st));
-            CU(cudaMemcpy2DAsync(cr_out + co + (ty / 2) * cw + tx / 2, cw, (const uint8_t*)b->d_final.p + tp.plane_off[2],
-                                 pp.pitch_c, wc, hc, cudaMemcpyDeviceToHost, st));
+          const size_t w = std::min<size_t>(im.tile_w, im.out_w - tx), h = std::min<size_t>(im.tile_h, im.out_h - ty);
+          CU(cudaMemcpy2DAsync(y_out + yo + ty * im.out_w + tx, im.out_w,
+                               fin + tp.plane_off[0] + (size_t)im.win_y * pp.pitch_y + im.win_x, pp.pitch_y, w, h,
+                               cudaMemcpyDeviceToHost, st));
+          if (pp.chroma && cb_out && cr_out) {  // 4:2:0: the window's offsets and sizes are even
+            const size_t wc = std::min<size_t>(im.tile_w / 2, cw - tx / 2), hc = std::min<size_t>(im.tile_h / 2, chh - ty / 2);
+            const size_t wo = (size_t)(im.win_y / 2) * pp.pitch_c + im.win_x / 2;
+            CU(cudaMemcpy2DAsync(cb_out + co + (ty / 2) * cw + tx / 2, cw, fin + tp.plane_off[1] + wo, pp.pitch_c, wc, hc,
+                                 cudaMemcpyDeviceToHost, st));
+            CU(cudaMemcpy2DAsync(cr_out + co + (ty / 2) * cw + tx / 2, cw, fin + tp.plane_off[2] + wo, pp.pitch_c, wc, hc,
+                                 cudaMemcpyDeviceToHost, st));
           }
         }
       }
@@ -1081,18 +1152,27 @@ static int64_t job_wait(heic_b200_job* job) {
   return 0;
 }
 
-static int64_t decode_grids_impl(heic_b200_ctx* ctx, const heic_image_desc* imgs, uint32_t n_imgs, uint8_t* rgb_out,
-                                 size_t pitch, size_t image_stride, int32_t apply_transforms, uint8_t* y_out,
+static int64_t decode_grids_impl(heic_b200_ctx* ctx, const heic_image_desc* imgs, const heic_image_transform* xforms,
+                                 uint32_t n_imgs, uint8_t* rgb_out, size_t pitch, size_t image_stride, uint8_t* y_out,
                                  uint8_t* cb_out, uint8_t* cr_out, heic_tile_status* status) {
-  return job_wait(submit_grids(ctx, imgs, n_imgs, rgb_out, pitch, image_stride, apply_transforms, y_out, cb_out, cr_out, status));
+  return job_wait(submit_grids(ctx, imgs, xforms, n_imgs, rgb_out, pitch, image_stride, y_out, cb_out, cr_out, status));
 }
 
 int32_t heic_b200_decode_grids(heic_b200_ctx* ctx, const heic_image_desc* imgs, uint32_t n_imgs, uint8_t* rgb_out,
                                size_t pitch, size_t image_stride, int32_t apply_transforms, heic_tile_status* status) {
   return static_cast<int32_t>(guard([&]() -> int64_t {
+    if (!ctx || !rgb_out) bail(HEIC_E_INVALID_ARG, "null argument");
+    return decode_grids_impl(ctx, imgs, canvas_transforms(imgs, n_imgs, apply_transforms).data(), n_imgs, rgb_out, pitch,
+                             image_stride, nullptr, nullptr, nullptr, status);
+  }));
+}
+
+int32_t heic_b200_decode_grids_transformed(heic_b200_ctx* ctx, const heic_image_desc* imgs, const heic_image_transform* xforms,
+                                           uint32_t n_imgs, uint8_t* rgb_out, size_t pitch, size_t image_stride,
+                                           heic_tile_status* status) {
+  return static_cast<int32_t>(guard([&]() -> int64_t {
     if (!rgb_out) bail(HEIC_E_INVALID_ARG, "null output buffer");
-    return decode_grids_impl(ctx, imgs, n_imgs, rgb_out, pitch, image_stride, apply_transforms, nullptr, nullptr, nullptr,
-                             status);
+    return decode_grids_impl(ctx, imgs, xforms, n_imgs, rgb_out, pitch, image_stride, nullptr, nullptr, nullptr, status);
   }));
 }
 
@@ -1100,8 +1180,20 @@ int32_t heic_b200_decode_grids_submit(heic_b200_ctx* ctx, const heic_image_desc*
                                       size_t pitch, size_t image_stride, int32_t apply_transforms, heic_tile_status* status,
                                       heic_b200_job** out_job) {
   return static_cast<int32_t>(guard([&]() -> int64_t {
+    if (!ctx || !rgb_out || !out_job) bail(HEIC_E_INVALID_ARG, "null argument");
+    *out_job = submit_grids(ctx, imgs, canvas_transforms(imgs, n_imgs, apply_transforms).data(), n_imgs, rgb_out, pitch,
+                            image_stride, nullptr, nullptr, nullptr, status);
+    return 0;
+  }));
+}
+
+int32_t heic_b200_decode_grids_submit_transformed(heic_b200_ctx* ctx, const heic_image_desc* imgs,
+                                                  const heic_image_transform* xforms, uint32_t n_imgs, uint8_t* rgb_out,
+                                                  size_t pitch, size_t image_stride, heic_tile_status* status,
+                                                  heic_b200_job** out_job) {
+  return static_cast<int32_t>(guard([&]() -> int64_t {
     if (!rgb_out || !out_job) bail(HEIC_E_INVALID_ARG, "null argument");
-    *out_job = submit_grids(ctx, imgs, n_imgs, rgb_out, pitch, image_stride, apply_transforms, nullptr, nullptr, nullptr, status);
+    *out_job = submit_grids(ctx, imgs, xforms, n_imgs, rgb_out, pitch, image_stride, nullptr, nullptr, nullptr, status);
     return 0;
   }));
 }
@@ -1116,8 +1208,9 @@ int32_t heic_b200_job_wait(heic_b200_job* job) {
 int32_t heic_b200_decode_grids_yuv(heic_b200_ctx* ctx, const heic_image_desc* imgs, uint32_t n_imgs, uint8_t* y_out,
                                    uint8_t* cb_out, uint8_t* cr_out, heic_tile_status* status) {
   return static_cast<int32_t>(guard([&]() -> int64_t {
-    if (!y_out) bail(HEIC_E_INVALID_ARG, "null output buffer");
-    return decode_grids_impl(ctx, imgs, n_imgs, nullptr, 0, 0, 0, y_out, cb_out, cr_out, status);
+    if (!ctx || !y_out) bail(HEIC_E_INVALID_ARG, "null argument");
+    return decode_grids_impl(ctx, imgs, canvas_transforms(imgs, n_imgs, 0).data(), n_imgs, nullptr, 0, 0, y_out, cb_out, cr_out,
+                             status);
   }));
 }
 
@@ -1126,8 +1219,8 @@ int32_t heic_b200_decode_file(heic_b200_ctx* ctx, const uint8_t* data, size_t le
   return static_cast<int32_t>(guard([&]() -> int64_t {
     if (!ctx || !data || !rgb_out) bail(HEIC_E_INVALID_ARG, "null argument");
     std::unique_ptr<HeicFile> f = HeicDecoder::open(data, len);
-    return decode_grids_impl(ctx, &f->primary.desc, 1, rgb_out, pitch, 0, apply_transforms, nullptr, nullptr, nullptr,
-                             nullptr);
+    const heic_image_transform xf = apply_transforms ? f->primary.transform : canvas_transforms(&f->primary.desc, 1, 0)[0];
+    return decode_grids_impl(ctx, &f->primary.desc, &xf, 1, rgb_out, pitch, 0, nullptr, nullptr, nullptr, nullptr);
   }));
 }
 
@@ -1214,11 +1307,11 @@ int32_t heic_b200_color_stitch(heic_b200_ctx* ctx, const void* dev_planes, uint3
     job.chroma = 1;
     job.full_range = full_range;
     job.matrix_coeffs = matrix_coeffs;
-    job.rotation = 0;
+    job.orientation = 0;
     job.rgb = (uint8_t*)dev_rgb;
     job.pitch = pitch;
     job.image_stride = image_stride;
-    CU(launch_color(job, ctx->stream));
+    CU(launch_color(job, ColorWindow{0, 0, out_w, out_h, 0, 0}, ctx->stream));
     ctx->launches++;
     CU(cudaStreamSynchronize(ctx->stream));
     return 0;

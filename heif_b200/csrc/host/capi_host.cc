@@ -157,5 +157,14 @@ int32_t heic_b200_file_info(const heic_b200_file* f, heic_file_info* out) {
   *out = f->f->info;
   return 0;
 }
+int32_t heic_b200_file_image_transform(const heic_b200_file* f, int32_t image, heic_image_transform* out) {
+  const ImageStorage* img = image_of(f, image);
+  if (!img || !out) {
+    set_last_error("invalid argument");
+    return HEIC_E_INVALID_ARG;
+  }
+  *out = img->transform;
+  return 0;
+}
 
 }  // extern "C"

@@ -104,7 +104,6 @@ void HeicDecoder::build_image(const HeifReader& reader, const Heif& heif, uint32
       out.desc.sps.colour_primaries = colr->nclx_primaries;
       out.desc.sps.transfer_characteristics = colr->nclx_transfer;
     }
-    if (heif.property_of(item_id, fourcc("imir"))) bail(HEIC_E_UNSUPPORTED, "'imir' (mirroring) is not supported");
   }
   const heic_sps& sps = out.desc.sps;
 
@@ -150,6 +149,7 @@ void HeicDecoder::build_image(const HeifReader& reader, const Heif& heif, uint32
   }
   const ItemProperty* irot = heif.property_of(item_id, fourcc("irot"));
   out.desc.rotation_ccw_quarter_turns = irot ? irot->irot_angle : 0;
+  out.transform = compose_transform(out.desc.output_width, out.desc.output_height, heif.properties_of(item_id));
   out.desc.n_tiles = static_cast<uint32_t>(tile_ids.size());
   out.desc.tiles = out.tiles.data();
   out.desc_raw = out.desc;
@@ -181,9 +181,10 @@ std::unique_ptr<HeicFile> HeicDecoder::open(const uint8_t* data, size_t len) {
   fi.ispe_width = ispe ? ispe->ispe_width : f->primary.desc.output_width;
   fi.ispe_height = ispe ? ispe->ispe_height : f->primary.desc.output_height;
   fi.rotation_ccw_quarter_turns = f->primary.desc.rotation_ccw_quarter_turns;
-  bool swap = fi.rotation_ccw_quarter_turns & 1;
-  fi.rotated_width = swap ? fi.ispe_height : fi.ispe_width;
-  fi.rotated_height = swap ? fi.ispe_width : fi.ispe_height;
+  const heic_image_transform& xf = f->primary.transform;
+  bool swap = xf.orientation & 1;
+  fi.rotated_width = swap ? xf.crop_h : xf.crop_w;
+  fi.rotated_height = swap ? xf.crop_w : xf.crop_h;
   fi.luma_bits = f->primary.desc.sps.bit_depth_luma_minus8 + 8;
   fi.chroma_bits = f->primary.desc.sps.bit_depth_chroma_minus8 + 8;
   fi.thumbnail_count = static_cast<uint32_t>(heif.references_to(primary, fourcc("thmb")).size());

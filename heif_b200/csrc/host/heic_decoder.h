@@ -19,6 +19,7 @@ struct ImageStorage {
   std::vector<std::vector<uint8_t>> rbsp;  // un-escaped slice RBSP per tile (owned)
   std::vector<std::vector<uint8_t>> nal;   // escaped VCL NAL unit per tile incl. 2-byte header
   std::vector<uint8_t> vps_nal, sps_nal, pps_nal;  // escaped parameter-set NAL units from hvcC
+  heic_image_transform transform;                  // the item's clap / irot / imir in normal form
   uint32_t item_id = 0;
 };
 

@@ -36,6 +36,74 @@ const ItemProperty* Heif::property_of(uint32_t item_id, uint32_t kind) const {
   return nullptr;
 }
 
+std::vector<const ItemProperty*> Heif::properties_of(uint32_t item_id) const {
+  std::vector<const ItemProperty*> out;
+  for (auto& a : associations) {
+    if (a.item_id != item_id) continue;
+    for (auto& e : a.entries)
+      if (e.second != 0 && e.second <= properties.size()) out.push_back(&properties[e.second - 1]);
+  }
+  return out;
+}
+
+namespace {
+
+// floor(n / d) for d > 0
+__int128 floor_div(__int128 n, __int128 d) { return n >= 0 ? n / d : -((-n + d - 1) / d); }
+
+// Pixel (x, y) of a w x h block whose image after orientation o (see heic_image_transform) has pixel (ox, oy) there.
+// Forward: 1: (y, w - 1 - x)  2: (w - 1 - x, h - 1 - y)  3: (h - 1 - y, x), then ox -> width - 1 - ox when o & 4.
+void unorient(uint32_t o, int64_t w, int64_t h, int64_t ox, int64_t oy, int64_t& x, int64_t& y) {
+  if (o & 4) ox = ((o & 1) ? h : w) - 1 - ox;
+  switch (o & 3) {
+    case 0: x = ox, y = oy; break;
+    case 1: y = ox, x = w - 1 - oy; break;
+    case 2: x = w - 1 - ox, y = h - 1 - oy; break;
+    default: y = h - 1 - ox, x = oy; break;
+  }
+}
+
+}  // namespace
+
+heic_image_transform compose_transform(uint32_t canvas_w, uint32_t canvas_h, const std::vector<const ItemProperty*>& props) {
+  heic_image_transform t{0, 0, canvas_w, canvas_h, 0};
+  for (const ItemProperty* p : props) {
+    uint32_t rot = t.orientation & 3, mir = t.orientation >> 2;
+    if (p->kind == fourcc("irot")) {
+      // a turn after a mirror is the mirror after the opposite turn
+      rot = mir ? (rot - p->irot_angle) & 3 : (rot + p->irot_angle) & 3;
+      t.orientation = rot | (mir << 2);
+    } else if (p->kind == fourcc("imir")) {
+      // left <-> right toggles the mirror; top <-> bottom is a half turn and then left <-> right
+      const uint32_t m = kImirOrientation[p->imir_axis & 1];
+      rot = mir ? (rot - (m & 3)) & 3 : (rot + (m & 3)) & 3;
+      t.orientation = rot | ((mir ^ 1u) << 2);
+    } else if (p->kind == fourcc("clap")) {
+      const int64_t W = (t.orientation & 1) ? t.crop_h : t.crop_w, H = (t.orientation & 1) ? t.crop_w : t.crop_h;
+      if (!p->clap_width_d || !p->clap_height_d || !p->clap_horiz_off_d || !p->clap_vert_off_d)
+        bail(HEIC_E_BITSTREAM, "clap with a zero denominator");
+      // Exact rationals: left = horizOff + (W - cleanW) / 2, rounded down; the width rounded to the nearest integer (halves
+      // up).  The rounding of non-integral values is this library's choice; it has not been compared with libheif's.
+      const __int128 wn = p->clap_width_n, wd = p->clap_width_d, hn = p->clap_height_n, hd = p->clap_height_d;
+      const __int128 xn = p->clap_horiz_off_n, xd = p->clap_horiz_off_d, yn = p->clap_vert_off_n, yd = p->clap_vert_off_d;
+      const __int128 cw = floor_div(2 * wn + wd, 2 * wd), ch = floor_div(2 * hn + hd, 2 * hd);
+      const __int128 left = floor_div(2 * xn * wd + ((__int128)W * wd - wn) * xd, 2 * xd * wd);
+      const __int128 top = floor_div(2 * yn * hd + ((__int128)H * hd - hn) * yd, 2 * yd * hd);
+      if (cw <= 0 || ch <= 0 || left < 0 || top < 0 || left + cw > W || top + ch > H)
+        bail(HEIC_E_BITSTREAM, "clap clean aperture is empty or not inside the image");
+      // the rectangle's corners back in crop coordinates
+      int64_t x0, y0, x1, y1;
+      unorient(t.orientation, t.crop_w, t.crop_h, (int64_t)left, (int64_t)top, x0, y0);
+      unorient(t.orientation, t.crop_w, t.crop_h, (int64_t)(left + cw - 1), (int64_t)(top + ch - 1), x1, y1);
+      t.crop_x += (uint32_t)std::min(x0, x1);
+      t.crop_y += (uint32_t)std::min(y0, y1);
+      t.crop_w = (uint32_t)(std::max(x0, x1) - std::min(x0, x1) + 1);
+      t.crop_h = (uint32_t)(std::max(y0, y1) - std::min(y0, y1) + 1);
+    }
+  }
+  return t;
+}
+
 std::vector<uint32_t> Heif::references_from(uint32_t from, uint32_t type) const {
   std::vector<uint32_t> out;
   for (auto& r : item_references)
@@ -250,6 +318,16 @@ void HeifReader::read_iprp(Heif& h, const BoxHeader& box) const {
             break;
           case fourcc("irot"): prop.irot_angle = static_cast<uint32_t>(be(c.payload, 1, c.end)) & 3; break;
           case fourcc("imir"): prop.imir_axis = static_cast<uint32_t>(be(c.payload, 1, c.end)) & 1; break;
+          case fourcc("clap"):
+            prop.clap_width_n = static_cast<uint32_t>(be(c.payload, 4, c.end));
+            prop.clap_width_d = static_cast<uint32_t>(be(c.payload + 4, 4, c.end));
+            prop.clap_height_n = static_cast<uint32_t>(be(c.payload + 8, 4, c.end));
+            prop.clap_height_d = static_cast<uint32_t>(be(c.payload + 12, 4, c.end));
+            prop.clap_horiz_off_n = static_cast<int32_t>(static_cast<uint32_t>(be(c.payload + 16, 4, c.end)));
+            prop.clap_horiz_off_d = static_cast<uint32_t>(be(c.payload + 20, 4, c.end));
+            prop.clap_vert_off_n = static_cast<int32_t>(static_cast<uint32_t>(be(c.payload + 24, 4, c.end)));
+            prop.clap_vert_off_d = static_cast<uint32_t>(be(c.payload + 28, 4, c.end));
+            break;
           case fourcc("pixi"): {
             uint32_t n = static_cast<uint32_t>(be(c.payload + 4, 1, c.end));
             for (uint32_t i = 0; i < n; ++i) prop.pixi_bits.push_back(static_cast<uint8_t>(be(c.payload + 5 + i, 1, c.end)));

@@ -67,6 +67,10 @@ struct ItemProperty {
   uint32_t ispe_width = 0, ispe_height = 0;     // 'ispe'
   uint32_t irot_angle = 0;                      // 'irot' (ccw quarter turns)
   uint32_t imir_axis = 0;                       // 'imir'
+  // 'clap' (ISO/IEC 14496-12 12.1.4): cleanApertureWidthN/D, cleanApertureHeightN/D, horizOffN/D, vertOffN/D
+  uint32_t clap_width_n = 0, clap_width_d = 0, clap_height_n = 0, clap_height_d = 0;
+  int32_t clap_horiz_off_n = 0, clap_vert_off_n = 0;
+  uint32_t clap_horiz_off_d = 0, clap_vert_off_d = 0;
   std::vector<uint8_t> pixi_bits;               // 'pixi'
   uint32_t colr_type = 0;                       // 'colr': 'nclx' / 'prof' / 'rICC'
   uint32_t nclx_primaries = 2, nclx_transfer = 2, nclx_matrix = 2, nclx_full_range = 0;
@@ -110,9 +114,22 @@ struct Heif {
   const HEVCDecoderConfigurationRecord* hevc_configuration_record() const;
   // The hvcC (or any property kind) actually associated with an item through ipma.
   const ItemProperty* property_of(uint32_t item_id, uint32_t kind) const;
+  // Every property of an item, in the order its ipma entries list them.
+  std::vector<const ItemProperty*> properties_of(uint32_t item_id) const;
   std::vector<uint32_t> references_from(uint32_t from_item_id, uint32_t reference_type) const;
   std::vector<uint32_t> references_to(uint32_t to_item_id, uint32_t reference_type) const;
 };
+
+// imir axis_type -> orientation bits of heic_image_transform: axis 0 mirrors top <-> bottom (6 = half turn, then
+// left <-> right), axis 1 mirrors left <-> right (4).  This follows libheif's reading and the later editions of
+// ISO/IEC 23008-12; the 2017 wording ("vertical axis" for 0) can be read the other way round, in which case only this
+// table changes.
+constexpr uint32_t kImirOrientation[2] = {6, 4};
+
+// The transformative properties (clap, irot, imir) of an image of canvas_w x canvas_h, applied in the given order,
+// reduced to heic_image_transform's normal form.  Other property kinds are skipped.  Throws HEIC_E_BITSTREAM for a clap
+// with a zero denominator, an empty clean aperture, or one that does not lie inside the image it applies to.
+heic_image_transform compose_transform(uint32_t canvas_w, uint32_t canvas_h, const std::vector<const ItemProperty*>& props);
 
 class HeifReader {
  public:

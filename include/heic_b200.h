@@ -180,6 +180,17 @@ typedef struct heic_image_desc {
   const heic_tile_desc* tiles;           /* row-major */
 } heic_image_desc;
 
+/* Output geometry of one image, carried beside its heic_image_desc (whose layout is fixed by the ABI version):
+ *   out = canvas[crop_y : crop_y + crop_h, crop_x : crop_x + crop_w], then rotated anticlockwise by
+ *   (orientation & 3) quarter turns, then, when orientation & 4, mirrored left <-> right.
+ * The canvas is the output_width x output_height grid canvas.  This normal form covers every sequence of the
+ * HEIF transformative properties clap, irot and imir (heic_b200_file_image_transform composes them).
+ * The identity is {0, 0, output_width, output_height, 0}. */
+typedef struct heic_image_transform {
+  uint32_t crop_x, crop_y, crop_w, crop_h;  /* canvas coordinates, before the orientation */
+  uint32_t orientation;                     /* bits 0-1: ccw quarter turns; bit 2: then mirror left<->right */
+} heic_image_transform;
+
 typedef struct heic_tile_status {
   int32_t code;               /* heic_status for this tile; one bad tile does not poison a batch */
   uint32_t bins_decoded;      /* CABAC bins (decision + bypass + terminate) consumed */
@@ -251,13 +262,16 @@ typedef struct heic_file_info {
   uint32_t primary_item_id;
   uint32_t ispe_width, ispe_height;       /* ispe associated with the primary item */
   uint32_t rotation_ccw_quarter_turns;    /* irot.angle */
-  uint32_t rotated_width, rotated_height;
+  uint32_t rotated_width, rotated_height; /* size after every transformative property (clap, irot, imir) */
   uint32_t luma_bits, chroma_bits;
   uint32_t thumbnail_count;
   uint32_t item_count;
   uint32_t is_grid;
 } heic_file_info;
 int32_t heic_b200_file_info(const heic_b200_file* f, heic_file_info* out);
+/* The clap / irot / imir properties of an image item (image = -1: primary, >= 0: auxiliary), taken in the order its
+ * ipma lists them and reduced to the normal form of heic_image_transform.  Properties of grid tile items are not applied. */
+int32_t heic_b200_file_image_transform(const heic_b200_file* f, int32_t image, heic_image_transform* out);
 
 /* ---- the hot path ------------------------------------------------------------------------- */
 /* Replacement for the tile loop + SliceSegmentReader::read_data (decoder.rs:114-119, slice.rs:206):
@@ -281,13 +295,28 @@ int32_t heic_b200_decode_grids_submit(heic_b200_ctx* ctx, const heic_image_desc*
                                       int32_t apply_transforms, heic_tile_status* status, heic_b200_job** out_job);
 int32_t heic_b200_job_wait(heic_b200_job* job);
 
+/* decode_grids / decode_grids_submit with an output geometry per image (xforms: n_imgs entries): image i is written as
+ * heic_image_transform describes, crop_w x crop_h, or crop_h x crop_w for odd quarter turns.  A transform whose crop
+ * does not lie inside its canvas, or whose orientation is above 7, fails the whole call with HEIC_E_INVALID_ARG before
+ * anything is queued.  The calls without xforms are these with {whole canvas, rotation_ccw_quarter_turns & 3} per image
+ * when apply_transforms != 0, and with the identity otherwise. */
+int32_t heic_b200_decode_grids_transformed(heic_b200_ctx* ctx, const heic_image_desc* imgs, const heic_image_transform* xforms,
+                                           uint32_t n_imgs, uint8_t* rgb_out, size_t pitch, size_t image_stride,
+                                           heic_tile_status* status);
+int32_t heic_b200_decode_grids_submit_transformed(heic_b200_ctx* ctx, const heic_image_desc* imgs,
+                                                  const heic_image_transform* xforms, uint32_t n_imgs, uint8_t* rgb_out,
+                                                  size_t pitch, size_t image_stride, heic_tile_status* status,
+                                                  heic_b200_job** out_job);
+
 /* Same, planar YCbCr out (tile mosaic cropped to the output canvas, no colour conversion): Y plane
- * output_width x output_height, then Cb, Cr at half resolution (rounded up), per image.  */
+ * output_width x output_height, then Cb, Cr at half resolution (rounded up), per image.  Tiles are stitched at their
+ * conformance-window size; no transform is applied.  */
 int32_t heic_b200_decode_grids_yuv(heic_b200_ctx* ctx, const heic_image_desc* imgs, uint32_t n_imgs,
                                    uint8_t* y_out, uint8_t* cb_out, uint8_t* cr_out,
                                    heic_tile_status* status);
 
 /* Convenience: HeicDecoder::decode(&[u8]) that actually returns the image (decoder.rs:12 returns ()).
+ * With apply_transforms != 0 the file's own transform (heic_b200_file_image_transform) is applied.
  * Query the size first with heic_b200_file_info (rotated_* when apply_transforms, else ispe_*). */
 int32_t heic_b200_decode_file(heic_b200_ctx* ctx, const uint8_t* data, size_t len, uint8_t* rgb_out,
                               size_t pitch, int32_t apply_transforms);
@@ -301,6 +330,9 @@ int32_t heic_b200_batch_create(heic_b200_ctx* ctx, const heic_image_desc* imgs, 
 /* The same with apply_transforms != 0: the RGB output of every image is rotated by its irot (as heic_b200_decode_grids does). */
 int32_t heic_b200_batch_create_ex(heic_b200_ctx* ctx, const heic_image_desc* imgs, uint32_t n_imgs, int32_t apply_transforms,
                                   heic_b200_batch** out);
+/* The same with an output geometry per image (see heic_b200_decode_grids_transformed). */
+int32_t heic_b200_batch_create_transformed(heic_b200_ctx* ctx, const heic_image_desc* imgs, const heic_image_transform* xforms,
+                                           uint32_t n_imgs, heic_b200_batch** out);
 void    heic_b200_batch_destroy(heic_b200_batch* b);
 /* Runs slice data -> RGB for the whole batch on the context's stream; does not synchronise. */
 int32_t heic_b200_batch_decode(heic_b200_batch* b);

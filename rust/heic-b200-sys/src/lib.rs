@@ -319,6 +319,18 @@ pub struct heic_image_desc {
     pub tiles: *const heic_tile_desc,
 }
 
+/// Output geometry of one image: the crop of the canvas, then `orientation & 3` anticlockwise quarter turns, then a
+/// left<->right mirror when `orientation & 4`.
+#[repr(C)]
+#[derive(Clone, Copy, Default)]
+pub struct heic_image_transform {
+    pub crop_x: u32,
+    pub crop_y: u32,
+    pub crop_w: u32,
+    pub crop_h: u32,
+    pub orientation: u32,
+}
+
 #[repr(C)]
 #[derive(Clone, Copy, Default)]
 pub struct heic_tile_status {
@@ -414,6 +426,7 @@ extern "C" {
         f: *const heic_b200_file, image: i32, tile: u32, data: *mut *const u8, len: *mut usize,
     ) -> i32;
     pub fn heic_b200_file_info(f: *const heic_b200_file, out: *mut heic_file_info) -> i32;
+    pub fn heic_b200_file_image_transform(f: *const heic_b200_file, image: i32, out: *mut heic_image_transform) -> i32;
     // ---- the hot path ----
     pub fn heic_b200_decode_grids(
         ctx: *mut heic_b200_ctx, imgs: *const heic_image_desc, n_imgs: u32, rgb_out: *mut u8, pitch: usize,
@@ -424,6 +437,14 @@ extern "C" {
         image_stride: usize, apply_transforms: c_int, status: *mut heic_tile_status, out_job: *mut *mut heic_b200_job,
     ) -> i32;
     pub fn heic_b200_job_wait(job: *mut heic_b200_job) -> i32;
+    pub fn heic_b200_decode_grids_transformed(
+        ctx: *mut heic_b200_ctx, imgs: *const heic_image_desc, xforms: *const heic_image_transform, n_imgs: u32,
+        rgb_out: *mut u8, pitch: usize, image_stride: usize, status: *mut heic_tile_status,
+    ) -> i32;
+    pub fn heic_b200_decode_grids_submit_transformed(
+        ctx: *mut heic_b200_ctx, imgs: *const heic_image_desc, xforms: *const heic_image_transform, n_imgs: u32,
+        rgb_out: *mut u8, pitch: usize, image_stride: usize, status: *mut heic_tile_status, out_job: *mut *mut heic_b200_job,
+    ) -> i32;
     pub fn heic_b200_decode_grids_yuv(
         ctx: *mut heic_b200_ctx, imgs: *const heic_image_desc, n_imgs: u32, y_out: *mut u8, cb_out: *mut u8,
         cr_out: *mut u8, status: *mut heic_tile_status,
@@ -437,6 +458,10 @@ extern "C" {
     ) -> i32;
     pub fn heic_b200_batch_create_ex(
         ctx: *mut heic_b200_ctx, imgs: *const heic_image_desc, n_imgs: u32, apply_transforms: i32, out: *mut *mut heic_b200_batch,
+    ) -> i32;
+    pub fn heic_b200_batch_create_transformed(
+        ctx: *mut heic_b200_ctx, imgs: *const heic_image_desc, xforms: *const heic_image_transform, n_imgs: u32,
+        out: *mut *mut heic_b200_batch,
     ) -> i32;
     pub fn heic_b200_batch_destroy(b: *mut heic_b200_batch);
     pub fn heic_b200_batch_decode(b: *mut heic_b200_batch) -> i32;
