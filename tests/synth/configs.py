@@ -71,3 +71,43 @@ EXTREME_CONFIGS = [
     ("big_monochrome", dict(_BIG, init_qp_minus26=25, chroma_format_idc=0)),
 ]
 EXTREME_SEEDS = (0, 1)
+
+# Directed intra-prediction streams, kept apart from CONFIGS (tests/test_intra_reference.py, test_gpu_intra.py).  Random
+# syntax alone puts the picture edge through a below-left or above-right neighbour a handful of times and rarely codes
+# large blocks; these pictures do it on purpose:
+# - widths and heights = 8, 16 or 24 (mod 32) and 40 .. 56 (mod 64) at CTB 16 / 32 / 64, so that the picture's right and
+#   bottom edges cut the above-right and below-left samples of 16x16 / 32x32 luma and 8x8 / 16x16 chroma blocks;
+# - few CU splits with MaxTb 32 (many 32x32 luma and 16x16 chroma blocks), and min TB 4 with many 8x8 CUs (NxN
+#   partitions: 4x4 luma units, chroma 4x4 of a split 8x8);
+# - few coded blocks (cbf_prob) for smooth pictures on which strong intra smoothing passes its flatness tests, each such
+#   stream once with strong smoothing on and once off (the same slice data: the walk does not depend on the flag);
+# - one CTB row, one CTB column, 8x8 and 4:0:0 pictures;
+# - about half with deblocking and SAO off: FFmpeg's output then is the intra reconstruction itself.
+_BIG32 = dict(log2_max_tb=5, split_cu_prob=0.1)
+_NO_LF = dict(deblocking_disabled=1, sao=0)
+_SMOOTH64 = dict(_BIG32, log2_ctb=6, width=512, height=304, cbf_prob=0.15)
+_SMOOTH32 = dict(_BIG32, width=480, height=272, cbf_prob=0.3)
+INTRA_CONFIGS = [
+    ("ctb64_big_520x296", dict(_BIG32, log2_ctb=6, width=520, height=296)),
+    ("ctb64_big_584x360_no_lf", dict(_BIG32, **_NO_LF, log2_ctb=6, width=584, height=360)),
+    ("ctb64_big_616x312_no_wpp", dict(_BIG32, log2_ctb=6, width=616, height=312, wpp=0)),
+    ("ctb32_big_520x280_no_lf", dict(_BIG32, **_NO_LF, width=520, height=280)),
+    ("ctb32_big_464x344", dict(_BIG32, width=464, height=344)),
+    ("ctb64_smooth_strong_no_lf", dict(_SMOOTH64, **_NO_LF, strong_intra_smoothing=1)),
+    ("ctb64_smooth_no_strong_no_lf", dict(_SMOOTH64, **_NO_LF, strong_intra_smoothing=0)),
+    ("ctb32_smooth_strong", dict(_SMOOTH32, strong_intra_smoothing=1)),
+    ("ctb32_smooth_no_strong", dict(_SMOOTH32, strong_intra_smoothing=0)),
+    ("ctb16_208x136_no_lf", dict(_NO_LF, log2_ctb=4, log2_max_tb=4, width=208, height=136, split_cu_prob=0.3)),
+    ("ctb32_mid_328x248_mpm", dict(width=328, height=248, split_cu_prob=0.4, log2_max_tb=4, prev_intra_prob=0.8)),
+    ("ctb64_mid_344x280_no_lf", dict(_NO_LF, log2_ctb=6, width=344, height=280, split_cu_prob=0.4, log2_max_tb=4,
+                                     prev_intra_prob=0.2)),
+    ("nxn_264x200", dict(width=264, height=200, split_cu_prob=0.9)),
+    ("nxn_ctb16_136x120_no_lf", dict(_NO_LF, log2_ctb=4, log2_max_tb=4, width=136, height=120, split_cu_prob=0.9)),
+    ("one_ctb_row_ctb64_584x56_no_lf", dict(_BIG32, **_NO_LF, log2_ctb=6, width=584, height=56)),
+    ("one_ctb_column_24x328", dict(_BIG32, width=24, height=328)),
+    ("one_ctb_column_ctb64_40x264_no_lf", dict(_BIG32, **_NO_LF, log2_ctb=6, width=40, height=264)),
+    ("tiny_8x8_no_lf", dict(_NO_LF, width=8, height=8)),
+    ("monochrome_ctb64_520x296", dict(_BIG32, log2_ctb=6, width=520, height=296, chroma_format_idc=0, strong_intra_smoothing=1,
+                                      cbf_prob=0.2)),
+]
+INTRA_SEEDS = (0, 1)

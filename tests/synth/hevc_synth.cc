@@ -114,10 +114,12 @@ struct EncEngine {
   Rng* rng = nullptr;
   double lps_gain = 1.0;          // > 1 makes LPS decisions more likely (busier streams)
   int max_bypass_ones = 6;        // caps unary / Exp-Golomb prefixes so values stay conformant
-  // Optional overrides of P(bin = 1) for two elements whose random-walk statistics are far from an encoder's choices
-  // (< 0: off, the context's own probability is used): real streams switch SAO on for a few per cent of the CTBs and
-  // smooth pictures rarely split their coding units.
-  double sao_on_prob = -1.0, split_cu_prob = -1.0;
+  // Optional overrides of P(bin = 1) for elements whose random-walk statistics are far from an encoder's choices
+  // (< 0: off, the context's own probability is used and no extra number is drawn): real streams switch SAO on for a few
+  // per cent of the CTBs and smooth pictures rarely split their coding units.  Few coded blocks (cbf_luma / cbf_cb /
+  // cbf_cr) give smooth, prediction-dominated pictures, on which strong intra smoothing passes its flatness tests;
+  // prev_intra_luma_pred_flag moves the luma modes between the most probable ones and the remaining 32.
+  double sao_on_prob = -1.0, split_cu_prob = -1.0, cbf_prob = -1.0, prev_intra_prob = -1.0;
   // With this probability a coeff_abs_level_remaining takes a chosen value (large_level_target) instead of the random walk:
   // its bins are queued and served to the next bypass() calls without the ones cap.
   double big_level_prob = 0.0;
@@ -209,6 +211,8 @@ struct EncEngine {
     double forced = -1.0;
     if (ctx_hint == CTX_SAO_TYPE) forced = sao_on_prob;
     else if (ctx_hint >= CTX_SPLIT_CU && ctx_hint < CTX_SPLIT_CU + 3) forced = split_cu_prob;
+    else if (ctx_hint >= CTX_CBF_LUMA && ctx_hint < CTX_CBF_CHROMA + 4) forced = cbf_prob;  // CBF_CHROMA follows CBF_LUMA
+    else if (ctx_hint == CTX_PREV_INTRA) forced = prev_intra_prob;
     ctx_hint = -1;
     if (forced >= 0.0) {
       const int bin = rng->uniform() < forced ? 1 : 0;
@@ -366,6 +370,7 @@ struct synth_config {
   double sao_on_prob, split_cu_prob;   // < 0: unbiased (see EncEngine)
   double big_level_prob;               // 0: every coeff_abs_level_remaining from the random walk (see EncEngine)
   uint32_t scaling_list_min, scaling_list_max;  // range of the explicit scaling-list entries (0, 0: 8..63)
+  double cbf_prob, prev_intra_prob;    // < 0: unbiased (see EncEngine)
 };
 
 // Writes the four NAL units (2-byte header + escaped payload) of one IDR_N_LP picture.  Each out_* buffer has `cap`
@@ -468,6 +473,8 @@ int synth_encode_picture(const synth_config* cfg, uint64_t seed, uint8_t* out_vp
     P.e.sao_on_prob = cfg->sao_on_prob;
     P.e.split_cu_prob = cfg->split_cu_prob;
     P.e.big_level_prob = cfg->big_level_prob;
+    P.e.cbf_prob = cfg->cbf_prob;
+    P.e.prev_intra_prob = cfg->prev_intra_prob;
     P.T = &tabs;
     P.ctx = ctx.data();
     P.pp = &pp;

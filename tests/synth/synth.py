@@ -24,7 +24,8 @@ class Config(C.Structure):
         ("slice_sao_luma", C.c_uint32), ("slice_sao_chroma", C.c_uint32), ("full_range", C.c_uint32),
         ("matrix_coeffs", C.c_uint32), ("lps_gain", C.c_double), ("max_bypass_ones", C.c_uint32),
         ("sao_on_prob", C.c_double), ("split_cu_prob", C.c_double), ("big_level_prob", C.c_double),
-        ("scaling_list_min", C.c_uint32), ("scaling_list_max", C.c_uint32),
+        ("scaling_list_min", C.c_uint32), ("scaling_list_max", C.c_uint32), ("cbf_prob", C.c_double),
+        ("prev_intra_prob", C.c_double),
     ]
 
 
@@ -33,7 +34,8 @@ DEFAULTS = dict(width=128, height=128, chroma_format_idc=1, log2_min_cb=3, log2_
                 transform_skip=0, cu_qp_delta=0, diff_cu_qp_delta_depth=0, init_qp_minus26=0, slice_qp_delta=0, cb_qp_offset=0,
                 cr_qp_offset=0, slice_cb_qp_offset=0, slice_cr_qp_offset=0, wpp=1, deblocking_disabled=0, beta_offset_div2=0,
                 tc_offset_div2=0, slice_sao_luma=1, slice_sao_chroma=1, full_range=1, matrix_coeffs=6, lps_gain=1.0,
-                max_bypass_ones=0, sao_on_prob=-1.0, split_cu_prob=-1.0, big_level_prob=0.0, scaling_list_min=8, scaling_list_max=63)
+                max_bypass_ones=0, sao_on_prob=-1.0, split_cu_prob=-1.0, big_level_prob=0.0, scaling_list_min=8, scaling_list_max=63,
+                cbf_prob=-1.0, prev_intra_prob=-1.0)
 
 _lib = None
 
