@@ -184,10 +184,25 @@ def _transform(t) -> K.ImageTransform:
     return t if isinstance(t, K.ImageTransform) else K.ImageTransform(*t)
 
 
-def _canvas(img: K.ImageDesc, apply_transforms: bool = False, transform=None):
-    """(width, height) of an image's output: the transform's crop, turned for odd quarter turns."""
+def _canvas(img: K.ImageDesc, apply_transforms: bool = False, transform=None, reduce: int = 1):
+    """(width, height) of an image's output: the transform's crop, turned for odd quarter turns, then reduced by the box
+    reduction factor to ceil(w / reduce) x ceil(h / reduce).  (A factor outside 1..16 is left for the library to reject.)"""
     t = _transform(transform) if transform is not None else canvas_transform(img, apply_transforms)
-    return (t.crop_h, t.crop_w) if t.orientation & 1 else (t.crop_w, t.crop_h)
+    w, h = (t.crop_h, t.crop_w) if t.orientation & 1 else (t.crop_w, t.crop_h)
+    k = max(int(reduce), 1)
+    return -(-w // k), -(-h // k)
+
+
+def _reduce_list(reduce, n: int):
+    """One box reduction factor per image from an int or a sequence."""
+    ks = [int(reduce)] * n if isinstance(reduce, (int, np.integer)) else [int(k) for k in reduce]
+    if len(ks) != n:
+        raise ValueError("one reduction factor per image")
+    return ks
+
+
+def _reduce_array(ks):
+    return (K.u32 * len(ks))(*[k & 0xFFFFFFFF for k in ks])
 
 
 def _transform_array(transforms, n: int):
@@ -210,16 +225,25 @@ def _desc_array(images):
 class Batch:
     """A resident batch: bitstreams, descriptors and every intermediate live in HBM (heic_b200_batch_*)."""
 
-    def __init__(self, dec: "HeicDecoder", images, apply_transforms: bool = False, transforms=None):
+    def __init__(self, dec: "HeicDecoder", images, apply_transforms: bool = False, transforms=None, reduce=1):
         """transforms: one heic_image_transform (K.ImageTransform or (x, y, w, h, orientation)) per image; when None,
-        apply_transforms selects the irot turn of every image or none."""
+        apply_transforms selects the irot turn of every image or none.  reduce: box reduction factor (1..16), one int for
+        every image or one per image: image i is PIL.Image.reduce(reduce[i]) of its transformed RGB (heic_b200.h,
+        heic_b200_decode_grids_reduced)."""
         self._lib = dec._lib
         self._dec = dec
         self.images = list(images)
         self.apply_transforms = bool(apply_transforms)
+        self.reduce = _reduce_list(reduce, len(self.images))
         self._arr = _desc_array(self.images)
         self._h = C.c_void_p()
-        if transforms is None:
+        if any(k != 1 for k in self.reduce):
+            xf = transforms if transforms is not None else [canvas_transform(im, self.apply_transforms) for im in self.images]
+            self._xf = _transform_array(xf, len(self.images))
+            self.transforms = list(self._xf)
+            K.check(self._lib.heic_b200_batch_create_reduced(dec._h, self._arr, self._xf, _reduce_array(self.reduce), len(self.images),
+                                                             C.byref(self._h)))
+        elif transforms is None:
             self.transforms = [canvas_transform(im, self.apply_transforms) for im in self.images]
             K.check(self._lib.heic_b200_batch_create_ex(dec._h, self._arr, len(self.images), int(self.apply_transforms), C.byref(self._h)))
         else:
@@ -275,7 +299,7 @@ class Batch:
         return int(p.value or 0), pitch.value, stride.value
 
     def download_rgb(self, out: np.ndarray | None = None) -> np.ndarray:
-        w, h = _canvas(self.images[0], transform=self.transforms[0])
+        w, h = _canvas(self.images[0], transform=self.transforms[0], reduce=self.reduce[0])
         if out is None:
             out = np.empty((len(self.images), h, w, 3), np.uint8)
         K.check(self._lib.heic_b200_batch_download_rgb(self._h, out.ctypes.data, out.strides[1], out.strides[0]))
@@ -283,7 +307,7 @@ class Batch:
 
     def download_image(self, index: int) -> np.ndarray:
         """RGB of one image of the batch (H, W, 3)."""
-        w, h = _canvas(self.images[index], transform=self.transforms[index])
+        w, h = _canvas(self.images[index], transform=self.transforms[index], reduce=self.reduce[index])
         out = np.empty((h, w, 3), np.uint8)
         K.check(self._lib.heic_b200_batch_download_image(self._h, index, out.ctypes.data, out.strides[0]))
         return out
@@ -356,21 +380,24 @@ class HeicDecoder:
     def launch_count(self) -> int:
         return int(self._lib.heic_b200_launch_count(self._h))
 
-    def decode(self, data, apply_transforms: bool = False) -> np.ndarray:
-        """bytes | HeicFile -> (H, W, 3) uint8 RGB of the primary item; apply_transforms: with the file's clap / irot / imir."""
+    def decode(self, data, apply_transforms: bool = False, reduce: int = 1) -> np.ndarray:
+        """bytes | HeicFile -> (H, W, 3) uint8 RGB of the primary item; apply_transforms: with the file's clap / irot / imir;
+        reduce: box reduction factor 1..16 (see Batch)."""
         f = data if isinstance(data, HeicFile) else HeicFile(data)
         if apply_transforms:
-            return self.decode_grids([f.primary], transforms=[f.transform()])[0]
-        return self.decode_grids([f.primary])[0]
+            return self.decode_grids([f.primary], transforms=[f.transform()], reduce=reduce)[0]
+        return self.decode_grids([f.primary], reduce=reduce)[0]
 
     def decode_grids(self, images, out: np.ndarray | None = None, apply_transforms: bool = False, return_status: bool = False,
-                     transforms=None):
+                     transforms=None, reduce=1):
         """Batch of image descriptors (host) -> (n, H, W, 3) uint8 RGB (host).  All outputs must share one size.
-        transforms: one heic_image_transform per image (see Batch); when None, apply_transforms selects irot or nothing."""
+        transforms: one heic_image_transform per image (see Batch); when None, apply_transforms selects irot or nothing.
+        reduce: box reduction factor (1..16), one for every image or one per image (see Batch)."""
         images = list(images)
         arr = _desc_array(images)
         xf = [None] * len(images) if transforms is None else list(transforms)
-        sizes = [_canvas(im, apply_transforms, t) for im, t in zip(images, xf)]
+        ks = _reduce_list(reduce, len(images))
+        sizes = [_canvas(im, apply_transforms, t, k) for im, t, k in zip(images, xf, ks)]
         w, h = sizes[0]
         if any(s != (w, h) for s in sizes[1:]):
             raise ValueError("decode_grids packs the images into one (n, H, W, 3) array: all outputs (after the transform) must be equal")
@@ -378,7 +405,11 @@ class HeicDecoder:
             out = np.empty((len(images), h, w, 3), np.uint8)
         n_tiles = sum(im.n_tiles for im in images)
         st = (K.TileStatus * n_tiles)()
-        if transforms is None:
+        if any(k != 1 for k in ks):
+            xf = [canvas_transform(im, apply_transforms) if t is None else t for im, t in zip(images, xf)]
+            rc = self._lib.heic_b200_decode_grids_reduced(self._h, arr, _transform_array(xf, len(images)), _reduce_array(ks), len(images),
+                                                          out.ctypes.data, out.strides[1], out.strides[0], st)
+        elif transforms is None:
             rc = self._lib.heic_b200_decode_grids(self._h, arr, len(images), out.ctypes.data, out.strides[1], out.strides[0],
                                                   1 if apply_transforms else 0, st)
         else:
@@ -389,14 +420,20 @@ class HeicDecoder:
         K.check(rc)
         return out
 
-    def submit_grids(self, images, out: np.ndarray, apply_transforms: bool = False, transforms=None):
+    def submit_grids(self, images, out: np.ndarray, apply_transforms: bool = False, transforms=None, reduce=1):
         """Asynchronous decode_grids: returns a job; call ``wait_job(job)`` before reading ``out``."""
         images = list(images)
         arr = _desc_array(images)
         n_tiles = sum(im.n_tiles for im in images)
         st = (K.TileStatus * n_tiles)()
         job = C.c_void_p()
-        if transforms is None:
+        ks = _reduce_list(reduce, len(images))
+        if any(k != 1 for k in ks):
+            xf = transforms if transforms is not None else [canvas_transform(im, apply_transforms) for im in images]
+            K.check(self._lib.heic_b200_decode_grids_submit_reduced(self._h, arr, _transform_array(xf, len(images)), _reduce_array(ks),
+                                                                    len(images), out.ctypes.data, out.strides[1], out.strides[0], st,
+                                                                    C.byref(job)))
+        elif transforms is None:
             K.check(self._lib.heic_b200_decode_grids_submit(self._h, arr, len(images), out.ctypes.data, out.strides[1], out.strides[0],
                                                             1 if apply_transforms else 0, st, C.byref(job)))
         else:
@@ -438,8 +475,8 @@ class HeicDecoder:
             co += cw * ch
         return res
 
-    def batch(self, images, apply_transforms: bool = False, transforms=None) -> Batch:
-        return Batch(self, images, apply_transforms, transforms)
+    def batch(self, images, apply_transforms: bool = False, transforms=None, reduce=1) -> Batch:
+        return Batch(self, images, apply_transforms, transforms, reduce)
 
     def color_stitch(self, dev_planes: int, n_images, grid_rows, grid_cols, tile_w, tile_h, out_w, out_h, dev_rgb: int,
                      pitch: int, image_stride: int, full_range: int = 1, matrix_coeffs: int = 6):

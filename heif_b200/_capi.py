@@ -178,12 +178,19 @@ SYMBOLS = [
      [_vp, C.POINTER(ImageDesc), C.POINTER(ImageTransform), u32, _vp, _sz, _sz, C.POINTER(TileStatus)]),
     ("heic_b200_decode_grids_submit_transformed", i32,
      [_vp, C.POINTER(ImageDesc), C.POINTER(ImageTransform), u32, _vp, _sz, _sz, C.POINTER(TileStatus), C.POINTER(_vp)]),
+    ("heic_b200_decode_grids_reduced", i32,
+     [_vp, C.POINTER(ImageDesc), C.POINTER(ImageTransform), C.POINTER(u32), u32, _vp, _sz, _sz, C.POINTER(TileStatus)]),
+    ("heic_b200_decode_grids_submit_reduced", i32,
+     [_vp, C.POINTER(ImageDesc), C.POINTER(ImageTransform), C.POINTER(u32), u32, _vp, _sz, _sz, C.POINTER(TileStatus),
+      C.POINTER(_vp)]),
     ("heic_b200_decode_grids_yuv", i32,
      [_vp, C.POINTER(ImageDesc), u32, _vp, _vp, _vp, C.POINTER(TileStatus)]),
     ("heic_b200_decode_file", i32, [_vp, C.c_char_p, _sz, _vp, _sz, i32]),
     ("heic_b200_batch_create", i32, [_vp, C.POINTER(ImageDesc), u32, C.POINTER(_vp)]),
     ("heic_b200_batch_create_ex", i32, [_vp, C.POINTER(ImageDesc), u32, i32, C.POINTER(_vp)]),
     ("heic_b200_batch_create_transformed", i32, [_vp, C.POINTER(ImageDesc), C.POINTER(ImageTransform), u32, C.POINTER(_vp)]),
+    ("heic_b200_batch_create_reduced", i32,
+     [_vp, C.POINTER(ImageDesc), C.POINTER(ImageTransform), C.POINTER(u32), u32, C.POINTER(_vp)]),
     ("heic_b200_batch_destroy", None, [_vp]),
     ("heic_b200_batch_decode", i32, [_vp]),
     ("heic_b200_batch_run_stages", i32, [_vp, u32]),

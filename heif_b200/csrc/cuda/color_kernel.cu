@@ -354,9 +354,152 @@ __global__ void __launch_bounds__(kColorThreads) color_geom_kernel(ColorJob J, C
   }
 }
 
+// Box reduction by k = 2..16 fused into the colour pass: the output is PIL.Image.reduce(k) of the RGB color_geom_kernel
+// writes, i.e. of T = the crop turned and mirrored.  Output pixel = block of n = rows x cols pixels of T (k x k, fewer in
+// its last row and column) with channel sums S, out = (((S + n / 2) * M(n)) mod 2^32) >> 24, M(n) = trunc(float32(2^32) /
+// float32(256 n)) (Pillow's fixed-point division, not the rounded mean).
+// The sums are taken in crop order and each finished block is placed at its oriented position: along a crop axis that
+// the orientation reverses, T's block grid starts at the crop's high edge, so block b covers crop positions
+// [b k - p, b k - p + k) with the phase p = (k - L % k) % k on that axis (0 on the others), and the grid of blocks is
+// oriented like the grid of pixels.
+// A CTA takes a region of kReduceRegionW x kReduceRegionH crop pixels rounded down to whole blocks.  Its threads convert
+// crop-aligned 16 x 2 groups (convert_block or gather_block, as color_geom_kernel), add each run of pixels of one block
+// in registers -- R + (G << 16) and B: a block sum is at most 256 x 255 < 2^16 -- and add the run into shared memory; then
+// the finished pixels are laid down in output orientation and leave as 16-byte stores.
+struct ReduceGeom {
+  uint32_t k, px, py;        // factor; phase of the block grid along crop x / y
+  uint32_t nbx, nby;         // blocks across / down the crop: ceil(crop_w / k), ceil(crop_h / k)
+  uint32_t bw, bh;           // blocks of a CTA's region
+  uint32_t regions_x, regions_y;
+};
+constexpr int kReduceRegionW = 256, kReduceRegionH = 32;
+constexpr int kReduceBlocks = (kReduceRegionW / 2) * (kReduceRegionH / 2);
+constexpr int kReduceSums = kReduceBlocks + kReduceBlocks / 32;  // block i at i + i / 32: a warp's adds hit distinct banks
+// the oriented region, rows padded to 16 bytes plus the destination's offset in its 16 bytes: at most 8192 bytes
+// (k = 2, odd quarter turn: 128 rows of up(15 + 16 x 3, 16))
+constexpr int kReduceStage = 8192;
+
+__device__ __forceinline__ uint32_t reduce_slot(uint32_t i) { return i + (i >> 5); }
+
+// Adds pixels i0..i1-1 of the group's rows in `rows` (bit r: row r) into consecutive blocks from slot `idx`; pixel i0 is
+// pixel `c` of its block.
+__device__ __forceinline__ void reduce_run(const uint32_t (&w)[2][12], uint32_t rows, uint32_t i0, uint32_t i1, uint32_t c,
+                                           uint32_t k, uint32_t idx, uint32_t* sum_rg, uint32_t* sum_b) {
+  uint32_t rg = 0, b = 0;
+#pragma unroll
+  for (int i = 0; i < 16; i++) {
+    if ((uint32_t)i < i0 || (uint32_t)i >= i1) continue;
+#pragma unroll
+    for (int r = 0; r < 2; r++) {
+      if (!((rows >> r) & 1u)) continue;
+      // R to byte 0 and G to byte 2 (from the one or two words holding them), B alone
+      rg += __byte_perm(w[r][(3 * i) >> 2], w[r][(3 * i + 1) >> 2], ((3 * i) & 3) | ((4 + ((3 * i + 1) & 3)) << 8)) & 0x00ff00ffu;
+      b += __byte_perm(w[r][(3 * i + 2) >> 2], 0u, 0x4440 | ((3 * i + 2) & 3));
+    }
+    if (++c == k || (uint32_t)i + 1 == i1) {
+      atomicAdd(sum_rg + reduce_slot(idx), rg);
+      atomicAdd(sum_b + reduce_slot(idx), b);
+      rg = b = 0;
+      c = 0;
+      idx++;
+    }
+  }
+}
+
+template <bool FULL, bool FUSED>
+__global__ void __launch_bounds__(kColorThreads) color_reduce_kernel(ColorJob J, ColorWindow G, Coeffs K, ReduceGeom R, uint32_t aligned) {
+  __shared__ uint32_t sum_rg[kReduceSums], sum_b[kReduceSums];
+  __shared__ __align__(16) uint8_t stage[kReduceStage];
+  const uint32_t per_image = R.regions_x * R.regions_y;
+  const uint32_t image = blockIdx.x / per_image, rem = blockIdx.x % per_image;
+  const uint32_t bx0 = (rem % R.regions_x) * R.bw, by0 = (rem / R.regions_x) * R.bh;  // first block of the region
+  const uint32_t bw = min(R.bw, R.nbx - bx0), bh = min(R.bh, R.nby - by0);
+  const int k = (int)R.k, W = (int)G.crop_w, H = (int)G.crop_h;
+  const uint32_t n_slots = reduce_slot(R.bw * bh - 1) + 1;
+  for (uint32_t i = threadIdx.x; i < n_slots; i += kColorThreads) sum_rg[i] = sum_b[i] = 0u;
+  // the region's pixels in crop coordinates, and the crop-aligned 16 x 2 groups that cover them
+  const int xs = max(0, (int)bx0 * k - (int)R.px), xe = min(W, (int)(bx0 + bw) * k - (int)R.px);
+  const int ys = max(0, (int)by0 * k - (int)R.py), ye = min(H, (int)(by0 + bh) * k - (int)R.py);
+  const uint32_t gx0 = (uint32_t)xs / 16, gy0 = (uint32_t)ys / 2;
+  const uint32_t ngx = (uint32_t)(xe - 1) / 16 - gx0 + 1, ngy = (uint32_t)(ye - 1) / 2 - gy0 + 1;
+  __syncthreads();
+  for (uint32_t g = threadIdx.x; g < ngx * ngy; g += kColorThreads) {
+    const int sx0 = (int)(gx0 + g % ngx) * 16, sy0 = (int)(gy0 + g / ngx) * 2;
+    const uint32_t cx = G.crop_x + (uint32_t)sx0, cy = G.crop_y + (uint32_t)sy0;
+    uint32_t w[2][12];
+    if (aligned) convert_block<FULL, FUSED>(J, K, image, cx, cy, cy + 1 < J.out_h, w);
+    else gather_block<FUSED>(J, G, K, image, cx, cy, (uint32_t)min(16, W - sx0), sy0 + 1 < H ? 2u : 1u, w);
+    const int x_first = max(xs, sx0);
+    const uint32_t i0 = (uint32_t)(x_first - sx0), i1 = (uint32_t)(min(xe, sx0 + 16) - sx0);
+    const uint32_t c = (uint32_t)(x_first + (int)R.px) % (uint32_t)k;
+    const uint32_t lbx = (uint32_t)(x_first + (int)R.px) / (uint32_t)k - bx0;
+    const bool r0 = sy0 >= ys, r1 = sy0 + 1 < ye;  // rows of the group inside the region
+    const uint32_t lby0 = (uint32_t)(sy0 + (int)R.py) / (uint32_t)k - by0, lby1 = (uint32_t)(sy0 + 1 + (int)R.py) / (uint32_t)k - by0;
+    if (r0 && r1 && lby0 == lby1) {
+      reduce_run(w, 3u, i0, i1, c, (uint32_t)k, lby0 * R.bw + lbx, sum_rg, sum_b);
+    } else {
+      if (r0) reduce_run(w, 1u, i0, i1, c, (uint32_t)k, lby0 * R.bw + lbx, sum_rg, sum_b);
+      if (r1) reduce_run(w, 2u, i0, i1, c, (uint32_t)k, lby1 * R.bw + lbx, sum_rg, sum_b);
+    }
+  }
+  __syncthreads();
+  // the region in output orientation: the block grid is oriented as color_geom_kernel orients the pixel grid
+  const uint32_t rot = J.orientation & 3u;
+  const bool mir = (J.orientation & 4u) != 0;
+  const uint32_t n_cols = (rot & 1u) ? bh : bw, n_rows = (rot & 1u) ? bw : bh;
+  uint32_t dx0, dy0;
+  if (rot == 0) dx0 = bx0, dy0 = by0;
+  else if (rot == 1) dx0 = by0, dy0 = R.nbx - bx0 - bw;
+  else if (rot == 2) dx0 = R.nbx - bx0 - bw, dy0 = R.nby - by0 - bh;
+  else dx0 = R.nby - by0 - bh, dy0 = bx0;
+  if (mir) dx0 = ((rot & 1u) ? R.nby : R.nbx) - dx0 - n_cols;
+  uint8_t* dst = J.rgb + (size_t)image * J.image_stride + (size_t)dy0 * J.pitch + (size_t)dx0 * 3;
+  // staging rows start at the destination's offset inside its 16 bytes, so that whole 16-byte words go out as one store
+  const bool wide = ((J.pitch | J.image_stride | (uint64_t)(uintptr_t)J.rgb) & 15u) == 0;
+  const uint32_t a = wide ? (uint32_t)((uintptr_t)dst & 15u) : 0u;
+  const uint32_t row_bytes = n_cols * 3, rs = (a + row_bytes + 15u) & ~15u;
+  for (uint32_t t = threadIdx.x; t < bw * bh; t += kColorThreads) {
+    const uint32_t lbx = t % bw, lby = t / bw;
+    const int x0 = (int)(bx0 + lbx) * k - (int)R.px, y0 = (int)(by0 + lby) * k - (int)R.py;
+    const uint32_t n = (uint32_t)((min(x0 + k, W) - max(x0, 0)) * (min(y0 + k, H) - max(y0, 0)));
+    const uint32_t m = __float2uint_rz(__fdiv_rn(4294967296.0f, (float)(256u * n))), half = n >> 1;
+    const uint32_t s = reduce_slot(lby * R.bw + lbx), rg = sum_rg[s], b = sum_b[s];
+    uint32_t row, col;
+    if (rot == 0) row = lby, col = lbx;
+    else if (rot == 1) row = bw - 1 - lbx, col = lby;
+    else if (rot == 2) row = bh - 1 - lby, col = bw - 1 - lbx;
+    else row = lbx, col = bh - 1 - lby;
+    if (mir) col = n_cols - 1 - col;
+    uint8_t* o = stage + row * rs + a + col * 3;
+    o[0] = (uint8_t)((((rg & 0xffffu) + half) * m) >> 24);
+    o[1] = (uint8_t)((((rg >> 16) + half) * m) >> 24);
+    o[2] = (uint8_t)(((b + half) * m) >> 24);
+  }
+  __syncthreads();
+  if (wide) {
+    uint8_t* base = dst - a;  // 16-byte aligned; the row's bytes are [a, a + row_bytes) of each staging row
+    const uint32_t chunks = rs >> 4;
+    for (uint32_t q = threadIdx.x; q < n_rows * chunks; q += kColorThreads) {
+      const uint32_t row = q / chunks, b0 = (q - row * chunks) * 16;
+      uint8_t* d = base + (size_t)row * J.pitch;
+      const uint8_t* s = stage + row * rs;
+      if (b0 >= a && b0 + 16 <= a + row_bytes) {
+        *reinterpret_cast<uint4*>(d + b0) = *reinterpret_cast<const uint4*>(s + b0);
+      } else {  // the row's partial first and last 16 bytes: the neighbouring regions write the rest
+        for (uint32_t j = max(b0, a); j < min(b0 + 16, a + row_bytes); j++) d[j] = s[j];
+      }
+    }
+  } else {
+    for (uint32_t q = threadIdx.x; q < n_rows * row_bytes; q += kColorThreads) {
+      const uint32_t row = q / row_bytes, c = q - row * row_bytes;
+      dst[(size_t)row * J.pitch + c] = stage[row * rs + c];
+    }
+  }
+}
+
 }  // namespace
 
-cudaError_t launch_color(const ColorJob& job, const ColorWindow& win, cudaStream_t stream) {
+cudaError_t launch_color(const ColorJob& job, const ColorWindow& win, uint32_t reduce, cudaStream_t stream) {
   if (!job.n_images || !job.out_w || !job.out_h || !win.crop_w || !win.crop_h) return cudaSuccess;
   Coeffs k;
   const bool bt709 = job.matrix_coeffs == 1;
@@ -374,6 +517,32 @@ cudaError_t launch_color(const ColorJob& job, const ColorWindow& win, cudaStream
   // seams between tiles at multiples of 8 columns and of 2 rows (or none): the first and the second 8 pixels of a
   // 16-pixel group may lie in different tiles, not within one, and the two rows of a thread lie in one tile
   const bool seams = (job.tile_w % 8 == 0 || job.grid_cols == 1) && (job.tile_h % 2 == 0 || job.grid_rows == 1);
+  if (reduce > 1) {
+    const uint32_t rot = job.orientation & 3u;
+    const bool mir = (job.orientation & 4u) != 0;
+    // crop axes that the orientation reverses (see color_reduce_kernel)
+    const bool rev_x = rot == 1 || (rot == 0 && mir) || (rot == 2 && !mir), rev_y = rot == 2 || (rot == 1 && mir) || (rot == 3 && !mir);
+    ReduceGeom r;
+    r.k = reduce;
+    r.px = rev_x ? (reduce - win.crop_w % reduce) % reduce : 0u;
+    r.py = rev_y ? (reduce - win.crop_h % reduce) % reduce : 0u;
+    r.nbx = (win.crop_w + reduce - 1) / reduce;
+    r.nby = (win.crop_h + reduce - 1) / reduce;
+    r.bw = (uint32_t)kReduceRegionW / reduce;  // k <= 16: at least 16 x 2 blocks
+    r.bh = (uint32_t)kReduceRegionH / reduce;
+    r.regions_x = (r.nbx + r.bw - 1) / r.bw;
+    r.regions_y = (r.nby + r.bh - 1) / r.bh;
+    const unsigned grid = job.n_images * r.regions_x * r.regions_y;
+    const uint32_t aligned = !win.win_x && !win.win_y && seams && win.crop_x % 8 == 0 && win.crop_y % 2 == 0;
+    if (job.fused) {
+      if (job.full_range) color_reduce_kernel<true, true><<<grid, kColorThreads, 0, stream>>>(job, win, k, r, aligned);
+      else color_reduce_kernel<false, true><<<grid, kColorThreads, 0, stream>>>(job, win, k, r, aligned);
+    } else {
+      if (job.full_range) color_reduce_kernel<true, false><<<grid, kColorThreads, 0, stream>>>(job, win, k, r, aligned);
+      else color_reduce_kernel<false, false><<<grid, kColorThreads, 0, stream>>>(job, win, k, r, aligned);
+    }
+    return cudaGetLastError();
+  }
   if (job.orientation != 0 || win.crop_x || win.crop_y || win.win_x || win.win_y || !seams) {
     const uint32_t tiles_x = (win.crop_w + kRotTile - 1) / kRotTile, tiles_y = (win.crop_h + kRotTile - 1) / kRotTile;
     const unsigned rgrid = job.n_images * tiles_x * tiles_y;

@@ -72,9 +72,11 @@ struct ColorWindow {
   uint32_t crop_x, crop_y, crop_w, crop_h;  // output rectangle in canvas coordinates, before the orientation
   uint32_t win_x, win_y;                    // origin of a tile's stitched part inside its decoded picture (luma samples)
 };
-// Identity orientation, crop and window at the origin, tiles stitched at multiples of 8 pixels: color_stitch_kernel.
-// Everything else: color_geom_kernel.
-cudaError_t launch_color(const ColorJob& job, const ColorWindow& win, cudaStream_t stream);
+// reduce = 1: identity orientation, crop and window at the origin, tiles stitched at multiples of 8 pixels:
+// color_stitch_kernel; everything else: color_geom_kernel.
+// reduce = 2..16: color_reduce_kernel writes PIL.Image.reduce(reduce) of that output (include/heic_b200.h,
+// heic_b200_decode_grids_reduced): ceil(w / reduce) x ceil(h / reduce) pixels.
+cudaError_t launch_color(const ColorJob& job, const ColorWindow& win, uint32_t reduce, cudaStream_t stream);
 
 }  // namespace dev
 }  // namespace heic

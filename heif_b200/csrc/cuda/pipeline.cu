@@ -138,9 +138,10 @@ struct heic_b200_ctx {
 
 struct ImageInfo {
   uint32_t first_tile, n_tiles, pic;
-  uint32_t grid_rows, grid_cols, out_w, out_h, rot_w, rot_h;
+  uint32_t grid_rows, grid_cols, out_w, out_h, rot_w, rot_h;  // rot_w x rot_h: the RGB output (oriented, then reduced)
   uint32_t tile_w, tile_h, win_x, win_y;                    // conformance window of every tile (luma samples)
   uint32_t crop_x, crop_y, crop_w, crop_h, orientation;     // heic_image_transform
+  uint32_t reduce;                                          // box reduction factor (1: none)
   uint32_t full_range, matrix_coeffs;
 };
 
@@ -176,6 +177,21 @@ void check_transform(const heic_image_transform& x, uint32_t out_w, uint32_t out
   if (x.orientation > 7 || !x.crop_w || !x.crop_h || (uint64_t)x.crop_x + x.crop_w > out_w || (uint64_t)x.crop_y + x.crop_h > out_h)
     bail(HEIC_E_INVALID_ARG, "image transform: crop rectangle not inside the canvas, or orientation above 7");
 }
+
+void check_reduce(uint32_t k) {
+  if (k < 1 || k > 16) bail(HEIC_E_INVALID_ARG, "reduction factor outside 1..16");
+}
+
+// Size of the RGB output of a transform and a reduction factor: the crop, turned for odd quarter turns, then
+// ceil(w / k) x ceil(h / k).
+void output_size(const heic_image_transform& x, uint32_t k, uint32_t& w, uint32_t& h) {
+  const uint32_t ow = (x.orientation & 1u) ? x.crop_h : x.crop_w, oh = (x.orientation & 1u) ? x.crop_w : x.crop_h;
+  w = (ow + k - 1) / k;
+  h = (oh + k - 1) / k;
+}
+
+// What the calls without reduction factors apply: 1 for every image.
+std::vector<uint32_t> no_reduction(uint32_t n_imgs) { return std::vector<uint32_t>(std::max(n_imgs, 1u), 1u); }
 
 // What the calls without transforms apply: the whole canvas, turned by irot when apply_transforms is set.
 std::vector<heic_image_transform> canvas_transforms(const heic_image_desc* imgs, uint32_t n_imgs, int32_t apply_transforms) {
@@ -248,7 +264,7 @@ struct heic_b200_batch {
     for (int k = 0; k < LIST_CLASSES; k++) a.list_off[k] = list_off[k];
     return a;
   }
-  void load(const heic_image_desc* imgs, const heic_image_transform* xforms, uint32_t n_imgs, bool with_rgb);
+  void load(const heic_image_desc* imgs, const heic_image_transform* xforms, const uint32_t* reduce, uint32_t n_imgs, bool with_rgb);
   void run(uint32_t mask);
 };
 
@@ -267,7 +283,8 @@ heic_b200_ctx::~heic_b200_ctx() {
 }
 
 // ---- batch construction --------------------------------------------------------------------------------
-void heic_b200_batch::load(const heic_image_desc* imgs, const heic_image_transform* xforms, uint32_t n_imgs, bool with_rgb) {
+void heic_b200_batch::load(const heic_image_desc* imgs, const heic_image_transform* xforms, const uint32_t* reduce, uint32_t n_imgs,
+                           bool with_rgb) {
   pics.clear();
   scaling.clear();
   tiles.clear();
@@ -297,6 +314,7 @@ void heic_b200_batch::load(const heic_image_desc* imgs, const heic_image_transfo
     image_geometry(im, pp, win, out_w, out_h);
     const heic_image_transform& xf = xforms[i];
     check_transform(xf, out_w, out_h);
+    check_reduce(reduce[i]);
     ScalingSet ss;
     build_scaling_set(im.sps, im.pps, ss);
     size_t s = 0;
@@ -324,8 +342,8 @@ void heic_b200_batch::load(const heic_image_desc* imgs, const heic_image_transfo
     info.crop_w = xf.crop_w;
     info.crop_h = xf.crop_h;
     info.orientation = xf.orientation;
-    info.rot_w = (xf.orientation & 1u) ? xf.crop_h : xf.crop_w;
-    info.rot_h = (xf.orientation & 1u) ? xf.crop_w : xf.crop_h;
+    info.reduce = reduce[i];
+    output_size(xf, reduce[i], info.rot_w, info.rot_h);
     info.full_range = im.sps.vui_parameters_present_flag ? im.sps.video_full_range_flag : 0u;
     info.matrix_coeffs = im.sps.vui_parameters_present_flag ? im.sps.matrix_coeffs : 2u;
     images.push_back(info);
@@ -641,7 +659,8 @@ void heic_b200_batch::run(uint32_t mask) {
         return a.pic == b.pic && a.n_tiles == b.n_tiles && a.grid_cols == b.grid_cols && a.out_w == b.out_w &&
                a.out_h == b.out_h && a.tile_w == b.tile_w && a.tile_h == b.tile_h && a.win_x == b.win_x && a.win_y == b.win_y &&
                a.crop_x == b.crop_x && a.crop_y == b.crop_y && a.crop_w == b.crop_w && a.crop_h == b.crop_h &&
-               a.orientation == b.orientation && a.full_range == b.full_range && a.matrix_coeffs == b.matrix_coeffs;
+               a.orientation == b.orientation && a.full_range == b.full_range && a.matrix_coeffs == b.matrix_coeffs &&
+               a.reduce == b.reduce;
       };
       while (j < images.size() && same(images[i], images[j])) j++;
       const ImageInfo& im = images[i];
@@ -677,7 +696,7 @@ void heic_b200_batch::run(uint32_t mask) {
       job.pitch = rgb_pitch;
       job.image_stride = rgb_image_stride;
       const ColorWindow win = {im.crop_x, im.crop_y, im.crop_w, im.crop_h, im.win_x, im.win_y};
-      CU(launch_color(job, win, st));
+      CU(launch_color(job, win, im.reduce, st));
       ctx->launches++;
       i = j;
     }
@@ -759,15 +778,15 @@ int32_t heic_b200_batch_create(heic_b200_ctx* ctx, const heic_image_desc* imgs, 
   return heic_b200_batch_create_ex(ctx, imgs, n_imgs, 0, out);
 }
 
-static int64_t batch_create(heic_b200_ctx* ctx, const heic_image_desc* imgs, const heic_image_transform* xforms, uint32_t n_imgs,
-                            heic_b200_batch** out) {
-  if (!ctx || !imgs || !xforms || !out || !n_imgs) bail(HEIC_E_INVALID_ARG, "null argument");
+static int64_t batch_create(heic_b200_ctx* ctx, const heic_image_desc* imgs, const heic_image_transform* xforms, const uint32_t* reduce,
+                            uint32_t n_imgs, heic_b200_batch** out) {
+  if (!ctx || !imgs || !xforms || !reduce || !out || !n_imgs) bail(HEIC_E_INVALID_ARG, "null argument");
   *out = nullptr;
   CU(cudaSetDevice(ctx->device));
   auto b = std::make_unique<heic_b200_batch>();
   b->ctx = ctx;
   b->stream = ctx->stream;
-  b->load(imgs, xforms, n_imgs, true);
+  b->load(imgs, xforms, reduce, n_imgs, true);
   CU(cudaStreamSynchronize(ctx->stream));
   *out = b.release();
   return 0;
@@ -778,13 +797,18 @@ int32_t heic_b200_batch_create_ex(heic_b200_ctx* ctx, const heic_image_desc* img
   return static_cast<int32_t>(guard([&]() -> int64_t {
     if (!ctx || !imgs || !out || !n_imgs) bail(HEIC_E_INVALID_ARG, "null argument");
     *out = nullptr;
-    return batch_create(ctx, imgs, canvas_transforms(imgs, n_imgs, apply_transforms).data(), n_imgs, out);
+    return batch_create(ctx, imgs, canvas_transforms(imgs, n_imgs, apply_transforms).data(), no_reduction(n_imgs).data(), n_imgs, out);
   }));
 }
 
 int32_t heic_b200_batch_create_transformed(heic_b200_ctx* ctx, const heic_image_desc* imgs, const heic_image_transform* xforms,
                                            uint32_t n_imgs, heic_b200_batch** out) {
-  return static_cast<int32_t>(guard([&]() -> int64_t { return batch_create(ctx, imgs, xforms, n_imgs, out); }));
+  return static_cast<int32_t>(guard([&]() -> int64_t { return batch_create(ctx, imgs, xforms, no_reduction(n_imgs).data(), n_imgs, out); }));
+}
+
+int32_t heic_b200_batch_create_reduced(heic_b200_ctx* ctx, const heic_image_desc* imgs, const heic_image_transform* xforms,
+                                       const uint32_t* reduce, uint32_t n_imgs, heic_b200_batch** out) {
+  return static_cast<int32_t>(guard([&]() -> int64_t { return batch_create(ctx, imgs, xforms, reduce, n_imgs, out); }));
 }
 
 void heic_b200_batch_destroy(heic_b200_batch* b) {
@@ -957,9 +981,9 @@ static void harvest_slot(heic_b200_ctx* ctx, int slot) {
 
 // xforms: one output geometry per image (RGB output; ignored for the planar output, which applies none)
 static heic_b200_job* submit_grids(heic_b200_ctx* ctx, const heic_image_desc* imgs, const heic_image_transform* xforms,
-                                   uint32_t n_imgs, uint8_t* rgb_out, size_t pitch, size_t image_stride, uint8_t* y_out,
-                                   uint8_t* cb_out, uint8_t* cr_out, heic_tile_status* status) {
-  if (!ctx || !imgs || !xforms || !n_imgs) bail(HEIC_E_INVALID_ARG, "null argument");
+                                   const uint32_t* reduce, uint32_t n_imgs, uint8_t* rgb_out, size_t pitch, size_t image_stride,
+                                   uint8_t* y_out, uint8_t* cb_out, uint8_t* cr_out, heic_tile_status* status) {
+  if (!ctx || !imgs || !xforms || !reduce || !n_imgs) bail(HEIC_E_INVALID_ARG, "null argument");
   CU(cudaSetDevice(ctx->device));
   // validate every descriptor before any work is queued, so a bad image rejects the call as a whole
   std::vector<size_t> first_tile(n_imgs + 1, 0), y_off(n_imgs + 1, 0), c_off(n_imgs + 1, 0);
@@ -970,14 +994,15 @@ static heic_b200_job* submit_grids(heic_b200_ctx* ctx, const heic_image_desc* im
     uint32_t out_w, out_h;
     image_geometry(im, pp, win, out_w, out_h);
     check_transform(xforms[i], out_w, out_h);
+    check_reduce(reduce[i]);
     TileParams tp;
     for (uint32_t t = 0; t < im.n_tiles; t++) make_tile_params(pp, im.pps, im.tiles[t], tp);
     const size_t ow = out_w, oh = out_h;
     if (rgb_out) {  // the caller's buffer layout, checked for every image before anything is queued
-      const bool turn = xforms[i].orientation & 1u;
-      const size_t rw = turn ? xforms[i].crop_h : xforms[i].crop_w, rh = turn ? xforms[i].crop_w : xforms[i].crop_h;
-      if (pitch < rw * 3) bail(HEIC_E_INVALID_ARG, "output pitch smaller than a row of RGB");
-      if (n_imgs > 1 && rh * pitch > image_stride) bail(HEIC_E_INVALID_ARG, "image_stride smaller than one image (rows x pitch)");
+      uint32_t rw, rh;
+      output_size(xforms[i], reduce[i], rw, rh);
+      if (pitch < (size_t)rw * 3) bail(HEIC_E_INVALID_ARG, "output pitch smaller than a row of RGB");
+      if (n_imgs > 1 && (size_t)rh * pitch > image_stride) bail(HEIC_E_INVALID_ARG, "image_stride smaller than one image (rows x pitch)");
     }
     first_tile[i + 1] = first_tile[i] + im.n_tiles;
     y_off[i + 1] = y_off[i] + ow * oh;
@@ -1032,7 +1057,7 @@ static heic_b200_job* submit_grids(heic_b200_ctx* ctx, const heic_image_desc* im
     heic_b200_batch* b = ctx->pipe_batch[slot].get();
     cudaStream_t st = b->stream;
     t0 = clk::now();
-    b->load(imgs + i0, xforms + i0, cnt, rgb_out != nullptr);
+    b->load(imgs + i0, xforms + i0, reduce + i0, cnt, rgb_out != nullptr);
     t_load += ms_since(t0);
     t0 = clk::now();
     PipePending& pend = ctx->pipe_pending[slot];
@@ -1153,17 +1178,17 @@ static int64_t job_wait(heic_b200_job* job) {
 }
 
 static int64_t decode_grids_impl(heic_b200_ctx* ctx, const heic_image_desc* imgs, const heic_image_transform* xforms,
-                                 uint32_t n_imgs, uint8_t* rgb_out, size_t pitch, size_t image_stride, uint8_t* y_out,
-                                 uint8_t* cb_out, uint8_t* cr_out, heic_tile_status* status) {
-  return job_wait(submit_grids(ctx, imgs, xforms, n_imgs, rgb_out, pitch, image_stride, y_out, cb_out, cr_out, status));
+                                 const uint32_t* reduce, uint32_t n_imgs, uint8_t* rgb_out, size_t pitch, size_t image_stride,
+                                 uint8_t* y_out, uint8_t* cb_out, uint8_t* cr_out, heic_tile_status* status) {
+  return job_wait(submit_grids(ctx, imgs, xforms, reduce, n_imgs, rgb_out, pitch, image_stride, y_out, cb_out, cr_out, status));
 }
 
 int32_t heic_b200_decode_grids(heic_b200_ctx* ctx, const heic_image_desc* imgs, uint32_t n_imgs, uint8_t* rgb_out,
                                size_t pitch, size_t image_stride, int32_t apply_transforms, heic_tile_status* status) {
   return static_cast<int32_t>(guard([&]() -> int64_t {
     if (!ctx || !rgb_out) bail(HEIC_E_INVALID_ARG, "null argument");
-    return decode_grids_impl(ctx, imgs, canvas_transforms(imgs, n_imgs, apply_transforms).data(), n_imgs, rgb_out, pitch,
-                             image_stride, nullptr, nullptr, nullptr, status);
+    return decode_grids_impl(ctx, imgs, canvas_transforms(imgs, n_imgs, apply_transforms).data(), no_reduction(n_imgs).data(), n_imgs,
+                             rgb_out, pitch, image_stride, nullptr, nullptr, nullptr, status);
   }));
 }
 
@@ -1172,7 +1197,17 @@ int32_t heic_b200_decode_grids_transformed(heic_b200_ctx* ctx, const heic_image_
                                            heic_tile_status* status) {
   return static_cast<int32_t>(guard([&]() -> int64_t {
     if (!rgb_out) bail(HEIC_E_INVALID_ARG, "null output buffer");
-    return decode_grids_impl(ctx, imgs, xforms, n_imgs, rgb_out, pitch, image_stride, nullptr, nullptr, nullptr, status);
+    return decode_grids_impl(ctx, imgs, xforms, no_reduction(n_imgs).data(), n_imgs, rgb_out, pitch, image_stride, nullptr, nullptr,
+                             nullptr, status);
+  }));
+}
+
+int32_t heic_b200_decode_grids_reduced(heic_b200_ctx* ctx, const heic_image_desc* imgs, const heic_image_transform* xforms,
+                                       const uint32_t* reduce, uint32_t n_imgs, uint8_t* rgb_out, size_t pitch, size_t image_stride,
+                                       heic_tile_status* status) {
+  return static_cast<int32_t>(guard([&]() -> int64_t {
+    if (!rgb_out) bail(HEIC_E_INVALID_ARG, "null output buffer");
+    return decode_grids_impl(ctx, imgs, xforms, reduce, n_imgs, rgb_out, pitch, image_stride, nullptr, nullptr, nullptr, status);
   }));
 }
 
@@ -1181,8 +1216,8 @@ int32_t heic_b200_decode_grids_submit(heic_b200_ctx* ctx, const heic_image_desc*
                                       heic_b200_job** out_job) {
   return static_cast<int32_t>(guard([&]() -> int64_t {
     if (!ctx || !rgb_out || !out_job) bail(HEIC_E_INVALID_ARG, "null argument");
-    *out_job = submit_grids(ctx, imgs, canvas_transforms(imgs, n_imgs, apply_transforms).data(), n_imgs, rgb_out, pitch,
-                            image_stride, nullptr, nullptr, nullptr, status);
+    *out_job = submit_grids(ctx, imgs, canvas_transforms(imgs, n_imgs, apply_transforms).data(), no_reduction(n_imgs).data(), n_imgs,
+                            rgb_out, pitch, image_stride, nullptr, nullptr, nullptr, status);
     return 0;
   }));
 }
@@ -1193,7 +1228,18 @@ int32_t heic_b200_decode_grids_submit_transformed(heic_b200_ctx* ctx, const heic
                                                   heic_b200_job** out_job) {
   return static_cast<int32_t>(guard([&]() -> int64_t {
     if (!rgb_out || !out_job) bail(HEIC_E_INVALID_ARG, "null argument");
-    *out_job = submit_grids(ctx, imgs, xforms, n_imgs, rgb_out, pitch, image_stride, nullptr, nullptr, nullptr, status);
+    *out_job = submit_grids(ctx, imgs, xforms, no_reduction(n_imgs).data(), n_imgs, rgb_out, pitch, image_stride, nullptr, nullptr,
+                            nullptr, status);
+    return 0;
+  }));
+}
+
+int32_t heic_b200_decode_grids_submit_reduced(heic_b200_ctx* ctx, const heic_image_desc* imgs, const heic_image_transform* xforms,
+                                              const uint32_t* reduce, uint32_t n_imgs, uint8_t* rgb_out, size_t pitch,
+                                              size_t image_stride, heic_tile_status* status, heic_b200_job** out_job) {
+  return static_cast<int32_t>(guard([&]() -> int64_t {
+    if (!rgb_out || !out_job) bail(HEIC_E_INVALID_ARG, "null argument");
+    *out_job = submit_grids(ctx, imgs, xforms, reduce, n_imgs, rgb_out, pitch, image_stride, nullptr, nullptr, nullptr, status);
     return 0;
   }));
 }
@@ -1209,8 +1255,8 @@ int32_t heic_b200_decode_grids_yuv(heic_b200_ctx* ctx, const heic_image_desc* im
                                    uint8_t* cb_out, uint8_t* cr_out, heic_tile_status* status) {
   return static_cast<int32_t>(guard([&]() -> int64_t {
     if (!ctx || !y_out) bail(HEIC_E_INVALID_ARG, "null argument");
-    return decode_grids_impl(ctx, imgs, canvas_transforms(imgs, n_imgs, 0).data(), n_imgs, nullptr, 0, 0, y_out, cb_out, cr_out,
-                             status);
+    return decode_grids_impl(ctx, imgs, canvas_transforms(imgs, n_imgs, 0).data(), no_reduction(n_imgs).data(), n_imgs, nullptr, 0, 0,
+                             y_out, cb_out, cr_out, status);
   }));
 }
 
@@ -1220,7 +1266,8 @@ int32_t heic_b200_decode_file(heic_b200_ctx* ctx, const uint8_t* data, size_t le
     if (!ctx || !data || !rgb_out) bail(HEIC_E_INVALID_ARG, "null argument");
     std::unique_ptr<HeicFile> f = HeicDecoder::open(data, len);
     const heic_image_transform xf = apply_transforms ? f->primary.transform : canvas_transforms(&f->primary.desc, 1, 0)[0];
-    return decode_grids_impl(ctx, &f->primary.desc, &xf, 1, rgb_out, pitch, 0, nullptr, nullptr, nullptr, nullptr);
+    const uint32_t k = 1;
+    return decode_grids_impl(ctx, &f->primary.desc, &xf, &k, 1, rgb_out, pitch, 0, nullptr, nullptr, nullptr, nullptr);
   }));
 }
 
@@ -1311,7 +1358,7 @@ int32_t heic_b200_color_stitch(heic_b200_ctx* ctx, const void* dev_planes, uint3
     job.rgb = (uint8_t*)dev_rgb;
     job.pitch = pitch;
     job.image_stride = image_stride;
-    CU(launch_color(job, ColorWindow{0, 0, out_w, out_h, 0, 0}, ctx->stream));
+    CU(launch_color(job, ColorWindow{0, 0, out_w, out_h, 0, 0}, 1, ctx->stream));
     ctx->launches++;
     CU(cudaStreamSynchronize(ctx->stream));
     return 0;

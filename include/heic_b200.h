@@ -308,6 +308,24 @@ int32_t heic_b200_decode_grids_submit_transformed(heic_b200_ctx* ctx, const heic
                                                   size_t pitch, size_t image_stride, heic_tile_status* status,
                                                   heic_b200_job** out_job);
 
+/* decode_grids_transformed / decode_grids_submit_transformed with a box reduction per image (reduce: n_imgs factors,
+ * 1..16): image i is PIL.Image.fromarray(T).reduce(reduce[i]) of the RGB8 image T that the _transformed call writes for
+ * xforms[i].  Its size is ceil(w / k) x ceil(h / k) for the w x h of T and k = reduce[i].  Each output pixel and channel
+ * comes from the block of n = rows x cols pixels of T it covers (k x k, fewer in the last output row and column), with
+ * channel sum S:
+ *     out = (((S + n / 2) * M(n)) mod 2^32) >> 24,   M(n) = trunc(float32(2^32) / float32(256 * n))
+ * (Pillow's fixed-point division; it differs from the rounded mean (S + n / 2) / n at some ties when n is not a power of
+ * two).  Decoding is unchanged; only the colour stage and the output shrink.  Factors of 1 give the _transformed output
+ * (those calls are these with every factor 1); factors may differ between images.  A factor of 0 or above 16 fails the
+ * whole call with HEIC_E_INVALID_ARG before anything is queued. */
+int32_t heic_b200_decode_grids_reduced(heic_b200_ctx* ctx, const heic_image_desc* imgs, const heic_image_transform* xforms,
+                                       const uint32_t* reduce, uint32_t n_imgs, uint8_t* rgb_out, size_t pitch,
+                                       size_t image_stride, heic_tile_status* status);
+int32_t heic_b200_decode_grids_submit_reduced(heic_b200_ctx* ctx, const heic_image_desc* imgs,
+                                              const heic_image_transform* xforms, const uint32_t* reduce, uint32_t n_imgs,
+                                              uint8_t* rgb_out, size_t pitch, size_t image_stride, heic_tile_status* status,
+                                              heic_b200_job** out_job);
+
 /* Same, planar YCbCr out (tile mosaic cropped to the output canvas, no colour conversion): Y plane
  * output_width x output_height, then Cb, Cr at half resolution (rounded up), per image.  Tiles are stitched at their
  * conformance-window size; no transform is applied.  */
@@ -333,6 +351,10 @@ int32_t heic_b200_batch_create_ex(heic_b200_ctx* ctx, const heic_image_desc* img
 /* The same with an output geometry per image (see heic_b200_decode_grids_transformed). */
 int32_t heic_b200_batch_create_transformed(heic_b200_ctx* ctx, const heic_image_desc* imgs, const heic_image_transform* xforms,
                                            uint32_t n_imgs, heic_b200_batch** out);
+/* The same with a box reduction factor per image (1..16; see heic_b200_decode_grids_reduced for the definition): the
+ * batch's RGB output, its pitch and its image stride are those of the reduced images. */
+int32_t heic_b200_batch_create_reduced(heic_b200_ctx* ctx, const heic_image_desc* imgs, const heic_image_transform* xforms,
+                                       const uint32_t* reduce, uint32_t n_imgs, heic_b200_batch** out);
 void    heic_b200_batch_destroy(heic_b200_batch* b);
 /* Runs slice data -> RGB for the whole batch on the context's stream; does not synchronise. */
 int32_t heic_b200_batch_decode(heic_b200_batch* b);

@@ -445,6 +445,15 @@ extern "C" {
         ctx: *mut heic_b200_ctx, imgs: *const heic_image_desc, xforms: *const heic_image_transform, n_imgs: u32,
         rgb_out: *mut u8, pitch: usize, image_stride: usize, status: *mut heic_tile_status, out_job: *mut *mut heic_b200_job,
     ) -> i32;
+    pub fn heic_b200_decode_grids_reduced(
+        ctx: *mut heic_b200_ctx, imgs: *const heic_image_desc, xforms: *const heic_image_transform, reduce: *const u32,
+        n_imgs: u32, rgb_out: *mut u8, pitch: usize, image_stride: usize, status: *mut heic_tile_status,
+    ) -> i32;
+    pub fn heic_b200_decode_grids_submit_reduced(
+        ctx: *mut heic_b200_ctx, imgs: *const heic_image_desc, xforms: *const heic_image_transform, reduce: *const u32,
+        n_imgs: u32, rgb_out: *mut u8, pitch: usize, image_stride: usize, status: *mut heic_tile_status,
+        out_job: *mut *mut heic_b200_job,
+    ) -> i32;
     pub fn heic_b200_decode_grids_yuv(
         ctx: *mut heic_b200_ctx, imgs: *const heic_image_desc, n_imgs: u32, y_out: *mut u8, cb_out: *mut u8,
         cr_out: *mut u8, status: *mut heic_tile_status,
@@ -462,6 +471,10 @@ extern "C" {
     pub fn heic_b200_batch_create_transformed(
         ctx: *mut heic_b200_ctx, imgs: *const heic_image_desc, xforms: *const heic_image_transform, n_imgs: u32,
         out: *mut *mut heic_b200_batch,
+    ) -> i32;
+    pub fn heic_b200_batch_create_reduced(
+        ctx: *mut heic_b200_ctx, imgs: *const heic_image_desc, xforms: *const heic_image_transform, reduce: *const u32,
+        n_imgs: u32, out: *mut *mut heic_b200_batch,
     ) -> i32;
     pub fn heic_b200_batch_destroy(b: *mut heic_b200_batch);
     pub fn heic_b200_batch_decode(b: *mut heic_b200_batch) -> i32;
