@@ -16,12 +16,14 @@ import ctypes as C
 import numpy as np
 
 from . import _capi as K
+from ._capi import RESAMPLE_BICUBIC, RESAMPLE_BILINEAR, RESAMPLE_BOX, RESAMPLE_HAMMING, RESAMPLE_LANCZOS
 from ._capi import HeicError, STAGE_ALL, STAGE_CABAC, STAGE_COLOR, STAGE_DEBLOCK, STAGE_INTRA, STAGE_SAO, STAGE_TRANSFORM
 
 __all__ = [
     "HeicDecoder", "HeicFile", "HeifReader", "Batch", "HeicError", "remove_emulation_prevention", "parse_sps", "parse_pps",
     "parse_slice_header", "parse_slice_header_raw", "read_ue", "read_se", "STAGE_ALL", "STAGE_CABAC", "STAGE_TRANSFORM", "STAGE_INTRA", "STAGE_DEBLOCK", "STAGE_SAO",
-    "STAGE_COLOR",
+    "STAGE_COLOR", "RESAMPLE_LANCZOS", "RESAMPLE_BILINEAR", "RESAMPLE_BICUBIC", "RESAMPLE_BOX", "RESAMPLE_HAMMING",
+    "resample_coeffs",
 ]
 
 
@@ -184,13 +186,61 @@ def _transform(t) -> K.ImageTransform:
     return t if isinstance(t, K.ImageTransform) else K.ImageTransform(*t)
 
 
-def _canvas(img: K.ImageDesc, apply_transforms: bool = False, transform=None, reduce: int = 1):
+def _canvas(img: K.ImageDesc, apply_transforms: bool = False, transform=None, reduce: int = 1, resize=None):
     """(width, height) of an image's output: the transform's crop, turned for odd quarter turns, then reduced by the box
-    reduction factor to ceil(w / reduce) x ceil(h / reduce).  (A factor outside 1..16 is left for the library to reject.)"""
+    reduction factor to ceil(w / reduce) x ceil(h / reduce), then the resize's (W, H) when there is one.  (A factor outside
+    1..16 or an invalid resize is left for the library to reject.)"""
+    if resize is not None and tuple(resize) != (0, 0):
+        return int(resize[0]), int(resize[1])
     t = _transform(transform) if transform is not None else canvas_transform(img, apply_transforms)
     w, h = (t.crop_h, t.crop_w) if t.orientation & 1 else (t.crop_w, t.crop_h)
     k = max(int(reduce), 1)
     return -(-w // k), -(-h // k)
+
+
+def resample_coeffs(n_in: int, n_out: int, resample: int = RESAMPLE_BICUBIC):
+    """The fixed-point table of one resampling axis (heic_b200_resample_coeffs, host only): (bounds, coeffs) with bounds an
+    (n_out, 2) int32 array of (xmin, n) and coeffs the int32 weights of every output index back to back."""
+    lib = _lib()
+    f = int(resample)
+    n = K.check(int(lib.heic_b200_resample_coeffs(n_in, n_out, f, None, None, 0)))
+    bounds = np.zeros((n_out, 2), np.int32)
+    coeffs = np.zeros(max(n, 1), np.int32)
+    K.check(int(lib.heic_b200_resample_coeffs(n_in, n_out, f, bounds.ctypes.data_as(C.POINTER(K.i32)),
+                                              coeffs.ctypes.data_as(C.POINTER(K.i32)), coeffs.size)))
+    return bounds, coeffs[:n]
+
+
+def _is_size(x) -> bool:
+    return isinstance(x, (tuple, list)) and len(x) == 2 and all(isinstance(v, (int, np.integer)) for v in x)
+
+
+def _resize_list(resize, n: int):
+    """One (W, H) or None per image from None, one (W, H) for every image, or a sequence with one entry per image."""
+    if resize is None:
+        return [None] * n
+    if _is_size(resize):
+        return [(int(resize[0]), int(resize[1]))] * n
+    rs = [None if r is None else (int(r[0]), int(r[1])) for r in resize]
+    if len(rs) != n:
+        raise ValueError("one resize per image")
+    return rs
+
+
+def _resample_list(resample, n: int):
+    """One filter per image from an int or PIL.Image.Resampling member (an IntEnum; Pillow is not imported), or a sequence."""
+    fs = [int(resample)] * n if isinstance(resample, (int, np.integer)) else [int(f) for f in resample]
+    if len(fs) != n:
+        raise ValueError("one resampling filter per image")
+    return fs
+
+
+def _resize_array(sizes, filters):
+    arr = (K.Resize * len(sizes))()
+    for i, (s, f) in enumerate(zip(sizes, filters)):
+        if s is not None:
+            arr[i] = K.Resize(s[0] & 0xFFFFFFFF, s[1] & 0xFFFFFFFF, f & 0xFFFFFFFF)
+    return arr
 
 
 def _reduce_list(reduce, n: int):
@@ -225,19 +275,30 @@ def _desc_array(images):
 class Batch:
     """A resident batch: bitstreams, descriptors and every intermediate live in HBM (heic_b200_batch_*)."""
 
-    def __init__(self, dec: "HeicDecoder", images, apply_transforms: bool = False, transforms=None, reduce=1):
+    def __init__(self, dec: "HeicDecoder", images, apply_transforms: bool = False, transforms=None, reduce=1, resize=None,
+                 resample=RESAMPLE_BICUBIC):
         """transforms: one heic_image_transform (K.ImageTransform or (x, y, w, h, orientation)) per image; when None,
         apply_transforms selects the irot turn of every image or none.  reduce: box reduction factor (1..16), one int for
         every image or one per image: image i is PIL.Image.reduce(reduce[i]) of its transformed RGB (heic_b200.h,
-        heic_b200_decode_grids_reduced)."""
+        heic_b200_decode_grids_reduced).  resize: None, one (W, H) for every image, or one (W, H) or None per image: image
+        i is then PIL.Image.resize((W, H), resample) of that (heic_b200_decode_grids_resized); resample: a filter number
+        or PIL.Image.Resampling member (LANCZOS, BILINEAR, BICUBIC, BOX, HAMMING; not NEAREST), or one per image."""
         self._lib = dec._lib
         self._dec = dec
         self.images = list(images)
         self.apply_transforms = bool(apply_transforms)
         self.reduce = _reduce_list(reduce, len(self.images))
+        self.resize = _resize_list(resize, len(self.images))
         self._arr = _desc_array(self.images)
         self._h = C.c_void_p()
-        if any(k != 1 for k in self.reduce):
+        if any(r is not None for r in self.resize):
+            xf = transforms if transforms is not None else [canvas_transform(im, self.apply_transforms) for im in self.images]
+            self._xf = _transform_array(xf, len(self.images))
+            self.transforms = list(self._xf)
+            rs = _resize_array(self.resize, _resample_list(resample, len(self.images)))
+            K.check(self._lib.heic_b200_batch_create_resized(dec._h, self._arr, self._xf, _reduce_array(self.reduce), rs,
+                                                             len(self.images), C.byref(self._h)))
+        elif any(k != 1 for k in self.reduce):
             xf = transforms if transforms is not None else [canvas_transform(im, self.apply_transforms) for im in self.images]
             self._xf = _transform_array(xf, len(self.images))
             self.transforms = list(self._xf)
@@ -299,7 +360,7 @@ class Batch:
         return int(p.value or 0), pitch.value, stride.value
 
     def download_rgb(self, out: np.ndarray | None = None) -> np.ndarray:
-        w, h = _canvas(self.images[0], transform=self.transforms[0], reduce=self.reduce[0])
+        w, h = _canvas(self.images[0], transform=self.transforms[0], reduce=self.reduce[0], resize=self.resize[0])
         if out is None:
             out = np.empty((len(self.images), h, w, 3), np.uint8)
         K.check(self._lib.heic_b200_batch_download_rgb(self._h, out.ctypes.data, out.strides[1], out.strides[0]))
@@ -307,7 +368,7 @@ class Batch:
 
     def download_image(self, index: int) -> np.ndarray:
         """RGB of one image of the batch (H, W, 3)."""
-        w, h = _canvas(self.images[index], transform=self.transforms[index], reduce=self.reduce[index])
+        w, h = _canvas(self.images[index], transform=self.transforms[index], reduce=self.reduce[index], resize=self.resize[index])
         out = np.empty((h, w, 3), np.uint8)
         K.check(self._lib.heic_b200_batch_download_image(self._h, index, out.ctypes.data, out.strides[0]))
         return out
@@ -380,24 +441,26 @@ class HeicDecoder:
     def launch_count(self) -> int:
         return int(self._lib.heic_b200_launch_count(self._h))
 
-    def decode(self, data, apply_transforms: bool = False, reduce: int = 1) -> np.ndarray:
+    def decode(self, data, apply_transforms: bool = False, reduce: int = 1, resize=None, resample=RESAMPLE_BICUBIC) -> np.ndarray:
         """bytes | HeicFile -> (H, W, 3) uint8 RGB of the primary item; apply_transforms: with the file's clap / irot / imir;
-        reduce: box reduction factor 1..16 (see Batch)."""
+        reduce: box reduction factor 1..16; resize: (W, H) or None, with the filter `resample` (see Batch)."""
         f = data if isinstance(data, HeicFile) else HeicFile(data)
         if apply_transforms:
-            return self.decode_grids([f.primary], transforms=[f.transform()], reduce=reduce)[0]
-        return self.decode_grids([f.primary], reduce=reduce)[0]
+            return self.decode_grids([f.primary], transforms=[f.transform()], reduce=reduce, resize=resize, resample=resample)[0]
+        return self.decode_grids([f.primary], reduce=reduce, resize=resize, resample=resample)[0]
 
     def decode_grids(self, images, out: np.ndarray | None = None, apply_transforms: bool = False, return_status: bool = False,
-                     transforms=None, reduce=1):
+                     transforms=None, reduce=1, resize=None, resample=RESAMPLE_BICUBIC):
         """Batch of image descriptors (host) -> (n, H, W, 3) uint8 RGB (host).  All outputs must share one size.
         transforms: one heic_image_transform per image (see Batch); when None, apply_transforms selects irot or nothing.
-        reduce: box reduction factor (1..16), one for every image or one per image (see Batch)."""
+        reduce: box reduction factor (1..16), one for every image or one per image; resize / resample: the resize after it
+        (see Batch)."""
         images = list(images)
         arr = _desc_array(images)
         xf = [None] * len(images) if transforms is None else list(transforms)
         ks = _reduce_list(reduce, len(images))
-        sizes = [_canvas(im, apply_transforms, t, k) for im, t, k in zip(images, xf, ks)]
+        rs = _resize_list(resize, len(images))
+        sizes = [_canvas(im, apply_transforms, t, k, r) for im, t, k, r in zip(images, xf, ks, rs)]
         w, h = sizes[0]
         if any(s != (w, h) for s in sizes[1:]):
             raise ValueError("decode_grids packs the images into one (n, H, W, 3) array: all outputs (after the transform) must be equal")
@@ -405,7 +468,12 @@ class HeicDecoder:
             out = np.empty((len(images), h, w, 3), np.uint8)
         n_tiles = sum(im.n_tiles for im in images)
         st = (K.TileStatus * n_tiles)()
-        if any(k != 1 for k in ks):
+        if any(r is not None for r in rs):
+            xf = [canvas_transform(im, apply_transforms) if t is None else t for im, t in zip(images, xf)]
+            rc = self._lib.heic_b200_decode_grids_resized(self._h, arr, _transform_array(xf, len(images)), _reduce_array(ks),
+                                                          _resize_array(rs, _resample_list(resample, len(images))), len(images),
+                                                          out.ctypes.data, out.strides[1], out.strides[0], st)
+        elif any(k != 1 for k in ks):
             xf = [canvas_transform(im, apply_transforms) if t is None else t for im, t in zip(images, xf)]
             rc = self._lib.heic_b200_decode_grids_reduced(self._h, arr, _transform_array(xf, len(images)), _reduce_array(ks), len(images),
                                                           out.ctypes.data, out.strides[1], out.strides[0], st)
@@ -420,7 +488,8 @@ class HeicDecoder:
         K.check(rc)
         return out
 
-    def submit_grids(self, images, out: np.ndarray, apply_transforms: bool = False, transforms=None, reduce=1):
+    def submit_grids(self, images, out: np.ndarray, apply_transforms: bool = False, transforms=None, reduce=1, resize=None,
+                     resample=RESAMPLE_BICUBIC):
         """Asynchronous decode_grids: returns a job; call ``wait_job(job)`` before reading ``out``."""
         images = list(images)
         arr = _desc_array(images)
@@ -428,7 +497,14 @@ class HeicDecoder:
         st = (K.TileStatus * n_tiles)()
         job = C.c_void_p()
         ks = _reduce_list(reduce, len(images))
-        if any(k != 1 for k in ks):
+        rs = _resize_list(resize, len(images))
+        if any(r is not None for r in rs):
+            xf = transforms if transforms is not None else [canvas_transform(im, apply_transforms) for im in images]
+            K.check(self._lib.heic_b200_decode_grids_submit_resized(self._h, arr, _transform_array(xf, len(images)), _reduce_array(ks),
+                                                                    _resize_array(rs, _resample_list(resample, len(images))),
+                                                                    len(images), out.ctypes.data, out.strides[1], out.strides[0], st,
+                                                                    C.byref(job)))
+        elif any(k != 1 for k in ks):
             xf = transforms if transforms is not None else [canvas_transform(im, apply_transforms) for im in images]
             K.check(self._lib.heic_b200_decode_grids_submit_reduced(self._h, arr, _transform_array(xf, len(images)), _reduce_array(ks),
                                                                     len(images), out.ctypes.data, out.strides[1], out.strides[0], st,
@@ -475,8 +551,9 @@ class HeicDecoder:
             co += cw * ch
         return res
 
-    def batch(self, images, apply_transforms: bool = False, transforms=None, reduce=1) -> Batch:
-        return Batch(self, images, apply_transforms, transforms, reduce)
+    def batch(self, images, apply_transforms: bool = False, transforms=None, reduce=1, resize=None,
+              resample=RESAMPLE_BICUBIC) -> Batch:
+        return Batch(self, images, apply_transforms, transforms, reduce, resize, resample)
 
     def color_stitch(self, dev_planes: int, n_images, grid_rows, grid_cols, tile_w, tile_h, out_w, out_h, dev_rgb: int,
                      pitch: int, image_stride: int, full_range: int = 1, matrix_coeffs: int = 6):

@@ -22,6 +22,9 @@ HEIC_E_NOMEM = -6
 STAGE_CABAC, STAGE_TRANSFORM, STAGE_INTRA, STAGE_DEBLOCK, STAGE_SAO, STAGE_COLOR = 1, 2, 4, 8, 16, 32
 STAGE_ALL = 63
 
+# heic_resize::filter: Pillow's Image.Resampling numbers (NEAREST = 0 is not offered)
+RESAMPLE_LANCZOS, RESAMPLE_BILINEAR, RESAMPLE_BICUBIC, RESAMPLE_BOX, RESAMPLE_HAMMING = 1, 2, 3, 4, 5
+
 u8, u32, i32 = C.c_uint8, C.c_uint32, C.c_int32
 
 
@@ -114,6 +117,11 @@ class ImageTransform(C.Structure):
     _fields_ = _u32_fields("crop_x,crop_y,crop_w,crop_h,orientation")
 
 
+class Resize(C.Structure):
+    """heic_resize: output width x height and filter (RESAMPLE_*); {0, 0, 0} is no resize."""
+    _fields_ = _u32_fields("width,height,filter")
+
+
 class TileStatus(C.Structure):
     _fields_ = [("code", i32), ("bins_decoded", u32), ("ctus_decoded", u32), ("reserved", u32)]
 
@@ -183,6 +191,13 @@ SYMBOLS = [
     ("heic_b200_decode_grids_submit_reduced", i32,
      [_vp, C.POINTER(ImageDesc), C.POINTER(ImageTransform), C.POINTER(u32), u32, _vp, _sz, _sz, C.POINTER(TileStatus),
       C.POINTER(_vp)]),
+    ("heic_b200_decode_grids_resized", i32,
+     [_vp, C.POINTER(ImageDesc), C.POINTER(ImageTransform), C.POINTER(u32), C.POINTER(Resize), u32, _vp, _sz, _sz,
+      C.POINTER(TileStatus)]),
+    ("heic_b200_decode_grids_submit_resized", i32,
+     [_vp, C.POINTER(ImageDesc), C.POINTER(ImageTransform), C.POINTER(u32), C.POINTER(Resize), u32, _vp, _sz, _sz,
+      C.POINTER(TileStatus), C.POINTER(_vp)]),
+    ("heic_b200_resample_coeffs", C.c_int64, [u32, u32, u32, C.POINTER(i32), C.POINTER(i32), _sz]),
     ("heic_b200_decode_grids_yuv", i32,
      [_vp, C.POINTER(ImageDesc), u32, _vp, _vp, _vp, C.POINTER(TileStatus)]),
     ("heic_b200_decode_file", i32, [_vp, C.c_char_p, _sz, _vp, _sz, i32]),
@@ -191,6 +206,8 @@ SYMBOLS = [
     ("heic_b200_batch_create_transformed", i32, [_vp, C.POINTER(ImageDesc), C.POINTER(ImageTransform), u32, C.POINTER(_vp)]),
     ("heic_b200_batch_create_reduced", i32,
      [_vp, C.POINTER(ImageDesc), C.POINTER(ImageTransform), C.POINTER(u32), u32, C.POINTER(_vp)]),
+    ("heic_b200_batch_create_resized", i32,
+     [_vp, C.POINTER(ImageDesc), C.POINTER(ImageTransform), C.POINTER(u32), C.POINTER(Resize), u32, C.POINTER(_vp)]),
     ("heic_b200_batch_destroy", None, [_vp]),
     ("heic_b200_batch_decode", i32, [_vp]),
     ("heic_b200_batch_run_stages", i32, [_vp, u32]),

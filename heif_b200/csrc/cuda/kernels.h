@@ -78,5 +78,35 @@ struct ColorWindow {
 // heic_b200_decode_grids_reduced): ceil(w / reduce) x ceil(h / reduce) pixels.
 cudaError_t launch_color(const ColorJob& job, const ColorWindow& win, uint32_t reduce, cudaStream_t stream);
 
+// Resampling after the colour stage: PIL.Image.resize of the colour stage's RGB (include/heic_b200.h,
+// heic_b200_decode_grids_resized), one launch per pass for a run of images with equal (source size, target size, filter).
+constexpr int kResampleBand = 32;  // output indices per band: a warp's lanes
+// One axis' fixed-point table in device memory, built on the host (host/resample.h) and laid out for the kernels.
+struct ResampleAxis {
+  const int4* out;        // per output index: {xmin, n, index of its tap 0 in coeffs (taps kResampleBand apart), 0}
+  const int4* band;       // per band of kResampleBand outputs: {xmin of its first output, input samples the band reads,
+                          //  taps (the band's largest n), index of the band's coefficients}
+  const int32_t* coeffs;  // band-major, then tap-major: output j's tap x at band.w + x * kResampleBand + j % kResampleBand;
+                          // 0 for x >= n, so a band can run its largest n for every output
+  uint32_t n_out, n_bands;
+  uint32_t max_taps;      // largest taps over the bands
+  uint32_t max_row_bytes; // largest shared-memory row a band of resample_h_kernel needs (16-byte multiple)
+};
+struct ResampleJob {
+  const uint8_t* src;     // image i at src + i * src_image_stride, RGB8 rows of src_pitch bytes (16-byte aligned)
+  uint64_t src_pitch, src_image_stride;
+  uint8_t* dst;           // the same for the output
+  uint64_t dst_pitch, dst_image_stride;
+  uint32_t n_images;
+  uint32_t out_w;         // output width in pixels
+  uint32_t rows;          // horizontal pass: rows it writes; vertical pass: output rows
+  uint32_t row0;          // horizontal pass: first source row it reads; vertical pass: shift subtracted from every xmin
+};
+// Horizontal pass: dst row r = the src row row0 + r resampled to out_w pixels (resample_h_kernel with the band's
+// coefficients and input span in shared memory, or resample_h_wide_kernel from global memory when they do not fit).
+cudaError_t launch_resample_h(const ResampleJob& job, const ResampleAxis& ax, cudaStream_t stream);
+// Vertical pass: dst row yy from the src rows [xmin - row0, xmin - row0 + n) of the table's entry yy.
+cudaError_t launch_resample_v(const ResampleJob& job, const ResampleAxis& ax, cudaStream_t stream);
+
 }  // namespace dev
 }  // namespace heic

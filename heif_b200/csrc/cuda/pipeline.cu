@@ -20,6 +20,7 @@
 
 #include "../host/capi_common.h"
 #include "../host/heic_decoder.h"
+#include "../host/resample.h"
 #include "cabac_tables.h"
 #include "host_params.h"
 #include "kernels.h"
@@ -138,10 +139,13 @@ struct heic_b200_ctx {
 
 struct ImageInfo {
   uint32_t first_tile, n_tiles, pic;
-  uint32_t grid_rows, grid_cols, out_w, out_h, rot_w, rot_h;  // rot_w x rot_h: the RGB output (oriented, then reduced)
+  uint32_t grid_rows, grid_cols, out_w, out_h, rot_w, rot_h;  // rot_w x rot_h: the RGB output (oriented, reduced, resized)
   uint32_t tile_w, tile_h, win_x, win_y;                    // conformance window of every tile (luma samples)
   uint32_t crop_x, crop_y, crop_w, crop_h, orientation;     // heic_image_transform
   uint32_t reduce;                                          // box reduction factor (1: none)
+  uint32_t src_w, src_h;                                    // size of the colour stage's output (oriented, reduced)
+  uint32_t filter;                                          // resize filter (HEIC_RESAMPLE_*); 0: rot_w x rot_h = src_w x src_h
+  uint32_t src_slot;                                        // resized images: index in the batch's source arena
   uint32_t full_range, matrix_coeffs;
 };
 
@@ -193,6 +197,22 @@ void output_size(const heic_image_transform& x, uint32_t k, uint32_t& w, uint32_
 // What the calls without reduction factors apply: 1 for every image.
 std::vector<uint32_t> no_reduction(uint32_t n_imgs) { return std::vector<uint32_t>(std::max(n_imgs, 1u), 1u); }
 
+void check_resize(const heic_resize& r) {
+  if ((r.width == 0) != (r.height == 0) || r.width > kResampleMaxSide || r.height > kResampleMaxSide ||
+      (r.width && (r.filter < HEIC_RESAMPLE_LANCZOS || r.filter > HEIC_RESAMPLE_HAMMING)))
+    bail(HEIC_E_INVALID_ARG, "resize: exactly one side 0, a side above 32768, or a filter outside 1..5");
+}
+
+// Size of the RGB output after the resize: the resize's size, or the colour stage's w x h when there is none.
+void resized_size(const heic_resize& r, uint32_t& w, uint32_t& h) {
+  if (r.width) w = r.width, h = r.height;
+}
+
+// What the calls without resizes apply: none.
+std::vector<heic_resize> no_resize(uint32_t n_imgs) {
+  return std::vector<heic_resize>(std::max(n_imgs, 1u), heic_resize{0, 0, 0});
+}
+
 // What the calls without transforms apply: the whole canvas, turned by irot when apply_transforms is set.
 std::vector<heic_image_transform> canvas_transforms(const heic_image_desc* imgs, uint32_t n_imgs, int32_t apply_transforms) {
   if (!imgs) bail(HEIC_E_INVALID_ARG, "null argument");
@@ -209,6 +229,21 @@ std::vector<heic_image_transform> canvas_transforms(const heic_image_desc* imgs,
 
 }  // namespace
 
+// Images in a row of a batch with equal (source size, target size, filter): one launch per resampling pass.
+// One distinct coefficient table of a load: its device layout sits in heic_b200_batch::rs_tables at these int32 offsets.
+struct ResampleTableRef {
+  ResampleAxis ax;              // the pointers are filled in by run()
+  size_t o_out, o_band, o_coef;
+  uint32_t row0, row_end;       // as a vertical table: the first and one past the last source row it reads
+};
+
+struct ResampleRun {
+  uint32_t first, count;      // images
+  int h_table, v_table;       // index into heic_b200_batch::rs_axes; -1: that pass does not run
+  uint32_t row0, rows;        // horizontal pass: source rows it reads (the vertical pass's first and last used rows)
+  size_t tmp_off, tmp_pitch, tmp_stride;  // uint8 intermediate of the two-pass case
+};
+
 struct CabacClass {  // tiles launched together: same wavefront shape
   int n_slots, hctb;
   uint32_t order_off, n_groups, n_tiles;
@@ -224,6 +259,11 @@ struct heic_b200_batch {
   std::vector<ImageInfo> images;
   std::vector<uint32_t> substreams, order, heavy_first;
   std::vector<CabacClass> classes;
+  std::vector<ResampleRun> rs_runs;
+  std::vector<ResampleTableRef> rs_axes;
+  std::vector<int32_t> rs_tables;     // device layout of every distinct table of the load (ResampleAxis)
+  size_t src_pitch = 0, src_image_stride = 0, n_src = 0, tmp_bytes = 0;
+  size_t src_off = 0, tmp_off = 0;  // byte offsets of the source arena and the intermediate inside d_rgb's allocation
   size_t raw_bytes = 0;       // raw NAL payloads of the tiles shipped with emulation prevention bytes in place
   bool any_plain = false;
   size_t bs_bytes = 0, tu_words = 0, coeff_elems = 0, plane_bytes = 0, map4_bytes = 0, map8_bytes = 0, sao_words = 0, wpp_bytes = 0;
@@ -234,7 +274,12 @@ struct heic_b200_batch {
   bool final_stale = false;   // SAO ran fused into the colour kernel: the `final` planes were not written (dump_tile refreshes them)
   bool coeff_clean = false;   // the coefficient arena is all-zero (fresh memset, or the last intra stage cleared it)
   PinnedBuf h_bitstream, h_status, h_params;
-  size_t off_sub = 0, off_order = 0, off_heavy = 0, off_pics = 0, off_tiles = 0, off_scaling = 0;  // inside the parameter blob
+  // inside the parameter blob
+  size_t off_sub = 0, off_order = 0, off_heavy = 0, off_pics = 0, off_tiles = 0, off_scaling = 0, off_resample = 0;
+  // d_rgb's allocation also holds, after the RGB output, the source arena (the colour stage's output of the resized
+  // images; the output then holds the resized ones) and the uint8 rows of the horizontal pass of the two-pass images: one
+  // allocation, so a context that alternates resized and unresized calls keeps the larger of the two layouts, not both.
+  // pass's uint8 rows of the images that take both passes
   DevBuf d_bitstream, d_params, d_tu, d_coeff, d_recon, d_final, d_ipm, d_ctd,
       d_qp, d_sao, d_wpp, d_status, d_rgb, d_list, d_list_count, d_raw, d_counters;
   PinnedBuf h_raw;
@@ -264,7 +309,9 @@ struct heic_b200_batch {
     for (int k = 0; k < LIST_CLASSES; k++) a.list_off[k] = list_off[k];
     return a;
   }
-  void load(const heic_image_desc* imgs, const heic_image_transform* xforms, const uint32_t* reduce, uint32_t n_imgs, bool with_rgb);
+  void load(const heic_image_desc* imgs, const heic_image_transform* xforms, const uint32_t* reduce, const heic_resize* resize,
+            uint32_t n_imgs, bool with_rgb);
+  void plan_resample();
   void run(uint32_t mask);
 };
 
@@ -283,8 +330,8 @@ heic_b200_ctx::~heic_b200_ctx() {
 }
 
 // ---- batch construction --------------------------------------------------------------------------------
-void heic_b200_batch::load(const heic_image_desc* imgs, const heic_image_transform* xforms, const uint32_t* reduce, uint32_t n_imgs,
-                           bool with_rgb) {
+void heic_b200_batch::load(const heic_image_desc* imgs, const heic_image_transform* xforms, const uint32_t* reduce,
+                           const heic_resize* resize, uint32_t n_imgs, bool with_rgb) {
   pics.clear();
   scaling.clear();
   tiles.clear();
@@ -315,6 +362,7 @@ void heic_b200_batch::load(const heic_image_desc* imgs, const heic_image_transfo
     const heic_image_transform& xf = xforms[i];
     check_transform(xf, out_w, out_h);
     check_reduce(reduce[i]);
+    check_resize(resize[i]);
     ScalingSet ss;
     build_scaling_set(im.sps, im.pps, ss);
     size_t s = 0;
@@ -343,7 +391,14 @@ void heic_b200_batch::load(const heic_image_desc* imgs, const heic_image_transfo
     info.crop_h = xf.crop_h;
     info.orientation = xf.orientation;
     info.reduce = reduce[i];
-    output_size(xf, reduce[i], info.rot_w, info.rot_h);
+    output_size(xf, reduce[i], info.src_w, info.src_h);
+    info.rot_w = info.src_w;
+    info.rot_h = info.src_h;
+    resized_size(resize[i], info.rot_w, info.rot_h);
+    // a resize to the size it already has is Pillow's copy(): the colour stage writes the output
+    info.filter = (info.rot_w != info.src_w || info.rot_h != info.src_h) && with_rgb ? resize[i].filter : 0u;
+    if (!with_rgb) info.rot_w = info.src_w, info.rot_h = info.src_h;
+    info.src_slot = 0;
     info.full_range = im.sps.vui_parameters_present_flag ? im.sps.video_full_range_flag : 0u;
     info.matrix_coeffs = im.sps.vui_parameters_present_flag ? im.sps.matrix_coeffs : 2u;
     images.push_back(info);
@@ -405,6 +460,7 @@ void heic_b200_batch::load(const heic_image_desc* imgs, const heic_image_transfo
   rgb_pitch = max_rgb_pitch;
   // every image is written at the widest pitch: the stride holds the tallest image at that pitch
   rgb_image_stride = up(max_rgb_pitch * max_rgb_rows, 256);
+  plan_resample();
   if (tiles.size() >= (1u << 24)) bail(HEIC_E_UNSUPPORTED, "more than 2^24 tiles in one batch (the transform lists keep the tile index in 24 bits)");
 
   // ---- CABAC launch classes: tiles with the same wavefront shape, heaviest first, TILES per CTA ----------
@@ -558,7 +614,8 @@ void heic_b200_batch::load(const heic_image_desc* imgs, const heic_image_transfo
   off_pics = up(off_heavy + heavy_first.size() * 4, 256);
   off_tiles = up(off_pics + pics.size() * sizeof(PicParams), 256);
   off_scaling = up(off_tiles + tiles.size() * sizeof(TileParams), 256);
-  const size_t params_bytes = up(off_scaling + scaling.size() * sizeof(ScalingSet), 256);
+  off_resample = up(off_scaling + scaling.size() * sizeof(ScalingSet), 256);
+  const size_t params_bytes = up(off_resample + rs_tables.size() * sizeof(int32_t), 256);
   h_params.ensure(params_bytes);
   {
     uint8_t* hp = (uint8_t*)h_params.p;
@@ -568,6 +625,7 @@ void heic_b200_batch::load(const heic_image_desc* imgs, const heic_image_transfo
     std::memcpy(hp + off_pics, pics.data(), pics.size() * sizeof(PicParams));
     std::memcpy(hp + off_tiles, tiles.data(), tiles.size() * sizeof(TileParams));
     std::memcpy(hp + off_scaling, scaling.data(), scaling.size() * sizeof(ScalingSet));
+    std::memcpy(hp + off_resample, rs_tables.data(), rs_tables.size() * sizeof(int32_t));
   }
   d_bitstream.ensure(bs_bytes + 16);
   d_params.ensure(params_bytes);
@@ -586,11 +644,106 @@ void heic_b200_batch::load(const heic_image_desc* imgs, const heic_image_transfo
   d_wpp.ensure(wpp_bytes);
   d_status.ensure(tiles.size() * sizeof(TileStatusDev));
   h_status.ensure(tiles.size() * sizeof(TileStatusDev));
-  if (with_rgb) d_rgb.ensure(rgb_image_stride * images.size());
+  if (with_rgb) {
+    src_off = up(rgb_image_stride * images.size(), 256);
+    tmp_off = up(src_off + src_image_stride * n_src, 256);
+    d_rgb.ensure(tmp_off + tmp_bytes);
+  }
   d_raw.ensure(raw_bytes ? raw_bytes + 16 : 0);
   if (any_plain) CU(cudaMemcpyAsync(d_bitstream.p, h_bitstream.p, bs_bytes + 16, cudaMemcpyHostToDevice, st));
   if (raw_bytes) CU(cudaMemcpyAsync(d_raw.p, h_raw.p, raw_bytes + 16, cudaMemcpyHostToDevice, st));
   CU(cudaMemcpyAsync(d_params.p, h_params.p, params_bytes, cudaMemcpyHostToDevice, st));
+}
+
+// Source arena, coefficient tables and launch runs of the resized images of a load.  The colour stage writes a resized
+// image into the source arena at its full (oriented, reduced) size, and the resampling passes write d_rgb.  Tables are
+// shared by every image and axis with the same (input size, output size, filter).
+void heic_b200_batch::plan_resample() {
+  rs_runs.clear();
+  rs_axes.clear();
+  rs_tables.clear();
+  src_pitch = src_image_stride = n_src = tmp_bytes = 0;
+  size_t max_rows = 0;
+  for (ImageInfo& im : images) {
+    if (!im.filter) continue;
+    im.src_slot = (uint32_t)n_src++;
+    src_pitch = std::max(src_pitch, up((size_t)im.src_w * 3, 16));
+    max_rows = std::max(max_rows, (size_t)im.src_h);
+  }
+  if (!n_src) return;
+  src_image_stride = up(src_pitch * max_rows, 256);
+  std::map<std::tuple<uint32_t, uint32_t, uint32_t>, int> by_key;
+  auto table = [&](uint32_t n_in, uint32_t n_out, uint32_t filter) -> int {
+    const auto key = std::make_tuple(n_in, n_out, filter);
+    const auto it = by_key.find(key);
+    if (it != by_key.end()) return it->second;
+    ResampleTable t;
+    resample_coeffs(n_in, n_out, filter, t);
+    ResampleTableRef ref;
+    std::memset(&ref, 0, sizeof ref);
+    ref.ax.n_out = n_out;
+    ref.ax.n_bands = (n_out + kResampleBand - 1) / kResampleBand;
+    ref.row0 = (uint32_t)t.xmin[0];
+    ref.row_end = (uint32_t)(t.xmin[n_out - 1] + t.n[n_out - 1]);
+    // every part is a multiple of 4 words: the int4 entries and the coefficient bands start at 16-byte boundaries
+    ref.o_out = rs_tables.size();
+    ref.o_band = ref.o_out + 4 * (size_t)n_out;
+    ref.o_coef = ref.o_band + 4 * (size_t)ref.ax.n_bands;
+    rs_tables.resize(ref.o_coef, 0);
+    for (uint32_t b = 0; b < ref.ax.n_bands; b++) {
+      const uint32_t j0 = b * kResampleBand, j1 = std::min(n_out, j0 + kResampleBand);
+      int32_t taps = 0, end = 0;
+      for (uint32_t j = j0; j < j1; j++) taps = std::max(taps, t.n[j]), end = std::max(end, t.xmin[j] + t.n[j]);
+      const size_t cb = rs_tables.size();
+      rs_tables.resize(cb + (size_t)taps * kResampleBand, 0);
+      for (uint32_t j = j0; j < j1; j++) {
+        for (int32_t x = 0; x < t.n[j]; x++) rs_tables[cb + (size_t)x * kResampleBand + (j - j0)] = t.coeffs[t.off[j] + x];
+        int32_t* e = &rs_tables[ref.o_out + 4 * (size_t)j];
+        e[0] = t.xmin[j];
+        e[1] = t.n[j];
+        e[2] = (int32_t)(cb - ref.o_coef + (j - j0));
+      }
+      const int32_t x0 = t.xmin[j0];
+      int32_t* e = &rs_tables[ref.o_band + 4 * (size_t)b];
+      e[0] = x0;
+      e[1] = end - x0;
+      e[2] = taps;
+      e[3] = (int32_t)(cb - ref.o_coef);
+      ref.ax.max_taps = std::max(ref.ax.max_taps, (uint32_t)taps);
+      // resample_h_kernel's row buffer holds the span from its 16-byte aligned start, and the band's last output reads
+      // `taps` pixels from its xmin
+      const size_t lead = (3u * (uint32_t)x0) & 15u;
+      const size_t need = std::max(lead + 3 * (size_t)(t.xmin[j1 - 1] - x0 + taps), lead + 3 * (size_t)(end - x0) + 15);
+      ref.ax.max_row_bytes = std::max(ref.ax.max_row_bytes, (uint32_t)up(need, 16));
+    }
+    rs_axes.push_back(ref);
+    return by_key[key] = (int)rs_axes.size() - 1;
+  };
+  for (size_t i = 0; i < images.size();) {
+    if (!images[i].filter) {
+      i++;
+      continue;
+    }
+    const ImageInfo& im = images[i];
+    size_t j = i + 1;
+    while (j < images.size() && images[j].filter == im.filter && images[j].src_w == im.src_w && images[j].src_h == im.src_h &&
+           images[j].rot_w == im.rot_w && images[j].rot_h == im.rot_h)
+      j++;
+    ResampleRun r;
+    r.first = (uint32_t)i;
+    r.count = (uint32_t)(j - i);
+    r.h_table = im.rot_w != im.src_w ? table(im.src_w, im.rot_w, im.filter) : -1;
+    r.v_table = im.rot_h != im.src_h ? table(im.src_h, im.rot_h, im.filter) : -1;
+    r.row0 = 0;
+    r.rows = im.src_h;
+    if (r.v_table >= 0) r.row0 = rs_axes[r.v_table].row0, r.rows = rs_axes[r.v_table].row_end - r.row0;
+    r.tmp_off = tmp_bytes;
+    r.tmp_pitch = up((size_t)im.rot_w * 3, 16);
+    r.tmp_stride = up(r.tmp_pitch * r.rows, 256);
+    if (r.h_table >= 0 && r.v_table >= 0) tmp_bytes += r.tmp_stride * r.count;
+    rs_runs.push_back(r);
+    i = j;
+  }
 }
 
 // ---- stage sequencing ----------------------------------------------------------------------------------
@@ -660,7 +813,7 @@ void heic_b200_batch::run(uint32_t mask) {
                a.out_h == b.out_h && a.tile_w == b.tile_w && a.tile_h == b.tile_h && a.win_x == b.win_x && a.win_y == b.win_y &&
                a.crop_x == b.crop_x && a.crop_y == b.crop_y && a.crop_w == b.crop_w && a.crop_h == b.crop_h &&
                a.orientation == b.orientation && a.full_range == b.full_range && a.matrix_coeffs == b.matrix_coeffs &&
-               a.reduce == b.reduce;
+               a.reduce == b.reduce && (a.filter != 0) == (b.filter != 0);
       };
       while (j < images.size() && same(images[i], images[j])) j++;
       const ImageInfo& im = images[i];
@@ -692,13 +845,62 @@ void heic_b200_batch::run(uint32_t mask) {
       job.full_range = im.full_range;
       job.matrix_coeffs = im.matrix_coeffs;
       job.orientation = im.orientation;
-      job.rgb = (uint8_t*)d_rgb.p + i * rgb_image_stride;
-      job.pitch = rgb_pitch;
-      job.image_stride = rgb_image_stride;
+      if (im.filter) {  // resized: the source arena, where consecutive resized images have consecutive slots
+        job.rgb = (uint8_t*)d_rgb.p + src_off + (size_t)im.src_slot * src_image_stride;
+        job.pitch = src_pitch;
+        job.image_stride = src_image_stride;
+      } else {
+        job.rgb = (uint8_t*)d_rgb.p + i * rgb_image_stride;
+        job.pitch = rgb_pitch;
+        job.image_stride = rgb_image_stride;
+      }
       const ColorWindow win = {im.crop_x, im.crop_y, im.crop_w, im.crop_h, im.win_x, im.win_y};
       CU(launch_color(job, win, im.reduce, st));
       ctx->launches++;
       i = j;
+    }
+    // resampling: horizontal pass first (into the intermediate when the vertical pass follows), then vertical, per run of images
+    const uint8_t* tabs = (const uint8_t*)d_params.p + off_resample;
+    auto axis = [&](int t) {
+      ResampleAxis a = rs_axes[t].ax;
+      a.out = (const int4*)(tabs + rs_axes[t].o_out * 4);
+      a.band = (const int4*)(tabs + rs_axes[t].o_band * 4);
+      a.coeffs = (const int32_t*)(tabs + rs_axes[t].o_coef * 4);
+      return a;
+    };
+    for (const ResampleRun& r : rs_runs) {
+      const ImageInfo& im = images[r.first];
+      ResampleJob rj;
+      rj.src = (const uint8_t*)d_rgb.p + src_off + (size_t)im.src_slot * src_image_stride;
+      rj.src_pitch = src_pitch;
+      rj.src_image_stride = src_image_stride;
+      rj.n_images = r.count;
+      rj.out_w = im.rot_w;
+      uint8_t* out = (uint8_t*)d_rgb.p + (size_t)r.first * rgb_image_stride;
+      const bool two = r.h_table >= 0 && r.v_table >= 0;
+      if (r.h_table >= 0) {
+        rj.dst = two ? (uint8_t*)d_rgb.p + tmp_off + r.tmp_off : out;
+        rj.dst_pitch = two ? r.tmp_pitch : rgb_pitch;
+        rj.dst_image_stride = two ? r.tmp_stride : rgb_image_stride;
+        rj.rows = r.rows;
+        rj.row0 = r.row0;
+        CU(launch_resample_h(rj, axis(r.h_table), st));
+        ctx->launches++;
+      }
+      if (r.v_table >= 0) {
+        if (two) {  // the intermediate starts at the first used row: the vertical bounds shift by it
+          rj.src = rj.dst;
+          rj.src_pitch = rj.dst_pitch;
+          rj.src_image_stride = rj.dst_image_stride;
+        }
+        rj.dst = out;
+        rj.dst_pitch = rgb_pitch;
+        rj.dst_image_stride = rgb_image_stride;
+        rj.rows = im.rot_h;
+        rj.row0 = two ? r.row0 : 0;
+        CU(launch_resample_v(rj, axis(r.v_table), st));
+        ctx->launches++;
+      }
     }
   }
   stages_run |= mask;
@@ -779,14 +981,14 @@ int32_t heic_b200_batch_create(heic_b200_ctx* ctx, const heic_image_desc* imgs, 
 }
 
 static int64_t batch_create(heic_b200_ctx* ctx, const heic_image_desc* imgs, const heic_image_transform* xforms, const uint32_t* reduce,
-                            uint32_t n_imgs, heic_b200_batch** out) {
-  if (!ctx || !imgs || !xforms || !reduce || !out || !n_imgs) bail(HEIC_E_INVALID_ARG, "null argument");
+                            const heic_resize* resize, uint32_t n_imgs, heic_b200_batch** out) {
+  if (!ctx || !imgs || !xforms || !reduce || !resize || !out || !n_imgs) bail(HEIC_E_INVALID_ARG, "null argument");
   *out = nullptr;
   CU(cudaSetDevice(ctx->device));
   auto b = std::make_unique<heic_b200_batch>();
   b->ctx = ctx;
   b->stream = ctx->stream;
-  b->load(imgs, xforms, reduce, n_imgs, true);
+  b->load(imgs, xforms, reduce, resize, n_imgs, true);
   CU(cudaStreamSynchronize(ctx->stream));
   *out = b.release();
   return 0;
@@ -797,18 +999,28 @@ int32_t heic_b200_batch_create_ex(heic_b200_ctx* ctx, const heic_image_desc* img
   return static_cast<int32_t>(guard([&]() -> int64_t {
     if (!ctx || !imgs || !out || !n_imgs) bail(HEIC_E_INVALID_ARG, "null argument");
     *out = nullptr;
-    return batch_create(ctx, imgs, canvas_transforms(imgs, n_imgs, apply_transforms).data(), no_reduction(n_imgs).data(), n_imgs, out);
+    return batch_create(ctx, imgs, canvas_transforms(imgs, n_imgs, apply_transforms).data(), no_reduction(n_imgs).data(),
+                        no_resize(n_imgs).data(), n_imgs, out);
   }));
 }
 
 int32_t heic_b200_batch_create_transformed(heic_b200_ctx* ctx, const heic_image_desc* imgs, const heic_image_transform* xforms,
                                            uint32_t n_imgs, heic_b200_batch** out) {
-  return static_cast<int32_t>(guard([&]() -> int64_t { return batch_create(ctx, imgs, xforms, no_reduction(n_imgs).data(), n_imgs, out); }));
+  return static_cast<int32_t>(guard([&]() -> int64_t {
+    return batch_create(ctx, imgs, xforms, no_reduction(n_imgs).data(), no_resize(n_imgs).data(), n_imgs, out);
+  }));
 }
 
 int32_t heic_b200_batch_create_reduced(heic_b200_ctx* ctx, const heic_image_desc* imgs, const heic_image_transform* xforms,
                                        const uint32_t* reduce, uint32_t n_imgs, heic_b200_batch** out) {
-  return static_cast<int32_t>(guard([&]() -> int64_t { return batch_create(ctx, imgs, xforms, reduce, n_imgs, out); }));
+  return static_cast<int32_t>(guard([&]() -> int64_t {
+    return batch_create(ctx, imgs, xforms, reduce, no_resize(n_imgs).data(), n_imgs, out);
+  }));
+}
+
+int32_t heic_b200_batch_create_resized(heic_b200_ctx* ctx, const heic_image_desc* imgs, const heic_image_transform* xforms,
+                                       const uint32_t* reduce, const heic_resize* resize, uint32_t n_imgs, heic_b200_batch** out) {
+  return static_cast<int32_t>(guard([&]() -> int64_t { return batch_create(ctx, imgs, xforms, reduce, resize, n_imgs, out); }));
 }
 
 void heic_b200_batch_destroy(heic_b200_batch* b) {
@@ -981,9 +1193,9 @@ static void harvest_slot(heic_b200_ctx* ctx, int slot) {
 
 // xforms: one output geometry per image (RGB output; ignored for the planar output, which applies none)
 static heic_b200_job* submit_grids(heic_b200_ctx* ctx, const heic_image_desc* imgs, const heic_image_transform* xforms,
-                                   const uint32_t* reduce, uint32_t n_imgs, uint8_t* rgb_out, size_t pitch, size_t image_stride,
-                                   uint8_t* y_out, uint8_t* cb_out, uint8_t* cr_out, heic_tile_status* status) {
-  if (!ctx || !imgs || !xforms || !reduce || !n_imgs) bail(HEIC_E_INVALID_ARG, "null argument");
+                                   const uint32_t* reduce, const heic_resize* resize, uint32_t n_imgs, uint8_t* rgb_out, size_t pitch,
+                                   size_t image_stride, uint8_t* y_out, uint8_t* cb_out, uint8_t* cr_out, heic_tile_status* status) {
+  if (!ctx || !imgs || !xforms || !reduce || !resize || !n_imgs) bail(HEIC_E_INVALID_ARG, "null argument");
   CU(cudaSetDevice(ctx->device));
   // validate every descriptor before any work is queued, so a bad image rejects the call as a whole
   std::vector<size_t> first_tile(n_imgs + 1, 0), y_off(n_imgs + 1, 0), c_off(n_imgs + 1, 0);
@@ -995,12 +1207,14 @@ static heic_b200_job* submit_grids(heic_b200_ctx* ctx, const heic_image_desc* im
     image_geometry(im, pp, win, out_w, out_h);
     check_transform(xforms[i], out_w, out_h);
     check_reduce(reduce[i]);
+    check_resize(resize[i]);
     TileParams tp;
     for (uint32_t t = 0; t < im.n_tiles; t++) make_tile_params(pp, im.pps, im.tiles[t], tp);
     const size_t ow = out_w, oh = out_h;
     if (rgb_out) {  // the caller's buffer layout, checked for every image before anything is queued
       uint32_t rw, rh;
       output_size(xforms[i], reduce[i], rw, rh);
+      resized_size(resize[i], rw, rh);
       if (pitch < (size_t)rw * 3) bail(HEIC_E_INVALID_ARG, "output pitch smaller than a row of RGB");
       if (n_imgs > 1 && (size_t)rh * pitch > image_stride) bail(HEIC_E_INVALID_ARG, "image_stride smaller than one image (rows x pitch)");
     }
@@ -1057,7 +1271,7 @@ static heic_b200_job* submit_grids(heic_b200_ctx* ctx, const heic_image_desc* im
     heic_b200_batch* b = ctx->pipe_batch[slot].get();
     cudaStream_t st = b->stream;
     t0 = clk::now();
-    b->load(imgs + i0, xforms + i0, reduce + i0, cnt, rgb_out != nullptr);
+    b->load(imgs + i0, xforms + i0, reduce + i0, resize + i0, cnt, rgb_out != nullptr);
     t_load += ms_since(t0);
     t0 = clk::now();
     PipePending& pend = ctx->pipe_pending[slot];
@@ -1178,17 +1392,17 @@ static int64_t job_wait(heic_b200_job* job) {
 }
 
 static int64_t decode_grids_impl(heic_b200_ctx* ctx, const heic_image_desc* imgs, const heic_image_transform* xforms,
-                                 const uint32_t* reduce, uint32_t n_imgs, uint8_t* rgb_out, size_t pitch, size_t image_stride,
-                                 uint8_t* y_out, uint8_t* cb_out, uint8_t* cr_out, heic_tile_status* status) {
-  return job_wait(submit_grids(ctx, imgs, xforms, reduce, n_imgs, rgb_out, pitch, image_stride, y_out, cb_out, cr_out, status));
+                                 const uint32_t* reduce, const heic_resize* resize, uint32_t n_imgs, uint8_t* rgb_out, size_t pitch,
+                                 size_t image_stride, uint8_t* y_out, uint8_t* cb_out, uint8_t* cr_out, heic_tile_status* status) {
+  return job_wait(submit_grids(ctx, imgs, xforms, reduce, resize, n_imgs, rgb_out, pitch, image_stride, y_out, cb_out, cr_out, status));
 }
 
 int32_t heic_b200_decode_grids(heic_b200_ctx* ctx, const heic_image_desc* imgs, uint32_t n_imgs, uint8_t* rgb_out,
                                size_t pitch, size_t image_stride, int32_t apply_transforms, heic_tile_status* status) {
   return static_cast<int32_t>(guard([&]() -> int64_t {
     if (!ctx || !rgb_out) bail(HEIC_E_INVALID_ARG, "null argument");
-    return decode_grids_impl(ctx, imgs, canvas_transforms(imgs, n_imgs, apply_transforms).data(), no_reduction(n_imgs).data(), n_imgs,
-                             rgb_out, pitch, image_stride, nullptr, nullptr, nullptr, status);
+    return decode_grids_impl(ctx, imgs, canvas_transforms(imgs, n_imgs, apply_transforms).data(), no_reduction(n_imgs).data(),
+                             no_resize(n_imgs).data(), n_imgs, rgb_out, pitch, image_stride, nullptr, nullptr, nullptr, status);
   }));
 }
 
@@ -1197,8 +1411,8 @@ int32_t heic_b200_decode_grids_transformed(heic_b200_ctx* ctx, const heic_image_
                                            heic_tile_status* status) {
   return static_cast<int32_t>(guard([&]() -> int64_t {
     if (!rgb_out) bail(HEIC_E_INVALID_ARG, "null output buffer");
-    return decode_grids_impl(ctx, imgs, xforms, no_reduction(n_imgs).data(), n_imgs, rgb_out, pitch, image_stride, nullptr, nullptr,
-                             nullptr, status);
+    return decode_grids_impl(ctx, imgs, xforms, no_reduction(n_imgs).data(), no_resize(n_imgs).data(), n_imgs, rgb_out, pitch,
+                             image_stride, nullptr, nullptr, nullptr, status);
   }));
 }
 
@@ -1207,7 +1421,18 @@ int32_t heic_b200_decode_grids_reduced(heic_b200_ctx* ctx, const heic_image_desc
                                        heic_tile_status* status) {
   return static_cast<int32_t>(guard([&]() -> int64_t {
     if (!rgb_out) bail(HEIC_E_INVALID_ARG, "null output buffer");
-    return decode_grids_impl(ctx, imgs, xforms, reduce, n_imgs, rgb_out, pitch, image_stride, nullptr, nullptr, nullptr, status);
+    return decode_grids_impl(ctx, imgs, xforms, reduce, no_resize(n_imgs).data(), n_imgs, rgb_out, pitch, image_stride, nullptr,
+                             nullptr, nullptr, status);
+  }));
+}
+
+int32_t heic_b200_decode_grids_resized(heic_b200_ctx* ctx, const heic_image_desc* imgs, const heic_image_transform* xforms,
+                                       const uint32_t* reduce, const heic_resize* resize, uint32_t n_imgs, uint8_t* rgb_out,
+                                       size_t pitch, size_t image_stride, heic_tile_status* status) {
+  return static_cast<int32_t>(guard([&]() -> int64_t {
+    if (!rgb_out) bail(HEIC_E_INVALID_ARG, "null output buffer");
+    return decode_grids_impl(ctx, imgs, xforms, reduce, resize, n_imgs, rgb_out, pitch, image_stride, nullptr, nullptr, nullptr,
+                             status);
   }));
 }
 
@@ -1216,8 +1441,8 @@ int32_t heic_b200_decode_grids_submit(heic_b200_ctx* ctx, const heic_image_desc*
                                       heic_b200_job** out_job) {
   return static_cast<int32_t>(guard([&]() -> int64_t {
     if (!ctx || !rgb_out || !out_job) bail(HEIC_E_INVALID_ARG, "null argument");
-    *out_job = submit_grids(ctx, imgs, canvas_transforms(imgs, n_imgs, apply_transforms).data(), no_reduction(n_imgs).data(), n_imgs,
-                            rgb_out, pitch, image_stride, nullptr, nullptr, nullptr, status);
+    *out_job = submit_grids(ctx, imgs, canvas_transforms(imgs, n_imgs, apply_transforms).data(), no_reduction(n_imgs).data(),
+                            no_resize(n_imgs).data(), n_imgs, rgb_out, pitch, image_stride, nullptr, nullptr, nullptr, status);
     return 0;
   }));
 }
@@ -1228,8 +1453,8 @@ int32_t heic_b200_decode_grids_submit_transformed(heic_b200_ctx* ctx, const heic
                                                   heic_b200_job** out_job) {
   return static_cast<int32_t>(guard([&]() -> int64_t {
     if (!rgb_out || !out_job) bail(HEIC_E_INVALID_ARG, "null argument");
-    *out_job = submit_grids(ctx, imgs, xforms, no_reduction(n_imgs).data(), n_imgs, rgb_out, pitch, image_stride, nullptr, nullptr,
-                            nullptr, status);
+    *out_job = submit_grids(ctx, imgs, xforms, no_reduction(n_imgs).data(), no_resize(n_imgs).data(), n_imgs, rgb_out, pitch,
+                            image_stride, nullptr, nullptr, nullptr, status);
     return 0;
   }));
 }
@@ -1239,7 +1464,18 @@ int32_t heic_b200_decode_grids_submit_reduced(heic_b200_ctx* ctx, const heic_ima
                                               size_t image_stride, heic_tile_status* status, heic_b200_job** out_job) {
   return static_cast<int32_t>(guard([&]() -> int64_t {
     if (!rgb_out || !out_job) bail(HEIC_E_INVALID_ARG, "null argument");
-    *out_job = submit_grids(ctx, imgs, xforms, reduce, n_imgs, rgb_out, pitch, image_stride, nullptr, nullptr, nullptr, status);
+    *out_job = submit_grids(ctx, imgs, xforms, reduce, no_resize(n_imgs).data(), n_imgs, rgb_out, pitch, image_stride, nullptr,
+                            nullptr, nullptr, status);
+    return 0;
+  }));
+}
+
+int32_t heic_b200_decode_grids_submit_resized(heic_b200_ctx* ctx, const heic_image_desc* imgs, const heic_image_transform* xforms,
+                                              const uint32_t* reduce, const heic_resize* resize, uint32_t n_imgs, uint8_t* rgb_out,
+                                              size_t pitch, size_t image_stride, heic_tile_status* status, heic_b200_job** out_job) {
+  return static_cast<int32_t>(guard([&]() -> int64_t {
+    if (!rgb_out || !out_job) bail(HEIC_E_INVALID_ARG, "null argument");
+    *out_job = submit_grids(ctx, imgs, xforms, reduce, resize, n_imgs, rgb_out, pitch, image_stride, nullptr, nullptr, nullptr, status);
     return 0;
   }));
 }
@@ -1255,8 +1491,8 @@ int32_t heic_b200_decode_grids_yuv(heic_b200_ctx* ctx, const heic_image_desc* im
                                    uint8_t* cb_out, uint8_t* cr_out, heic_tile_status* status) {
   return static_cast<int32_t>(guard([&]() -> int64_t {
     if (!ctx || !y_out) bail(HEIC_E_INVALID_ARG, "null argument");
-    return decode_grids_impl(ctx, imgs, canvas_transforms(imgs, n_imgs, 0).data(), no_reduction(n_imgs).data(), n_imgs, nullptr, 0, 0,
-                             y_out, cb_out, cr_out, status);
+    return decode_grids_impl(ctx, imgs, canvas_transforms(imgs, n_imgs, 0).data(), no_reduction(n_imgs).data(),
+                             no_resize(n_imgs).data(), n_imgs, nullptr, 0, 0, y_out, cb_out, cr_out, status);
   }));
 }
 
@@ -1267,7 +1503,8 @@ int32_t heic_b200_decode_file(heic_b200_ctx* ctx, const uint8_t* data, size_t le
     std::unique_ptr<HeicFile> f = HeicDecoder::open(data, len);
     const heic_image_transform xf = apply_transforms ? f->primary.transform : canvas_transforms(&f->primary.desc, 1, 0)[0];
     const uint32_t k = 1;
-    return decode_grids_impl(ctx, &f->primary.desc, &xf, &k, 1, rgb_out, pitch, 0, nullptr, nullptr, nullptr, nullptr);
+    const heic_resize none = {0, 0, 0};
+    return decode_grids_impl(ctx, &f->primary.desc, &xf, &k, &none, 1, rgb_out, pitch, 0, nullptr, nullptr, nullptr, nullptr);
   }));
 }
 

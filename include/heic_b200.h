@@ -326,6 +326,46 @@ int32_t heic_b200_decode_grids_submit_reduced(heic_b200_ctx* ctx, const heic_ima
                                               uint8_t* rgb_out, size_t pitch, size_t image_stride, heic_tile_status* status,
                                               heic_b200_job** out_job);
 
+/* Output size and filter of a resize (Pillow's Image.Resampling numbers).  {0, 0, 0}: no resize. */
+typedef struct heic_resize {
+  uint32_t width, height, filter;
+} heic_resize;
+enum { HEIC_RESAMPLE_LANCZOS = 1, HEIC_RESAMPLE_BILINEAR = 2, HEIC_RESAMPLE_BICUBIC = 3, HEIC_RESAMPLE_BOX = 4, HEIC_RESAMPLE_HAMMING = 5 };
+
+/* decode_grids_reduced / decode_grids_submit_reduced with a resize per image (resize: n_imgs entries): image i is
+ *     PIL.Image.fromarray(T).resize((W, H), filter, reducing_gap=None)
+ * of the RGB8 image T that the _reduced call writes for xforms[i] and reduce[i] (so reduce(k) then resize, as Pillow's
+ * img.reduce(k).resize(size, filter)), with (W, H, filter) = resize[i].  Filters and their support: LANCZOS 3,
+ * BILINEAR 1, BICUBIC 2 (a = -0.5), BOX 0.5 (1 on (-0.5, 0.5]), HAMMING 1 (sinc(x) * (0.54f + 0.46f * cos(pi x)), its
+ * constants float32 as in Pillow); sinc(0) = 1.
+ * Per axis, with input size n_in and output size n_out, in IEEE double:
+ *     scale = n_in / n_out, fs = max(scale, 1), support = filter_support * fs
+ *     output xx: center = (xx + 0.5) * scale, xmin = max((int)(center - support + 0.5), 0),
+ *                n = min((int)(center + support + 0.5), n_in) - xmin,
+ *                w[x] = filter((x + xmin - center + 0.5) * (1 / fs)) for x < n, each divided by their sum when it is not 0,
+ *                k[x] = (int)(w[x] * 2^22 + 0.5) for w >= 0, (int)(w[x] * 2^22 - 0.5) for w < 0
+ * A pass computes, per channel, s = 2^21 + sum_x in[xmin + x] * k[x] in int32 and writes clamp(s >> 22, 0, 255).  The
+ * horizontal pass runs first, when W != w, on the rows [first vertical xmin, last vertical xmin + n) of T only, into a
+ * uint8 image; the vertical bounds are then shifted by that first row.  The vertical pass runs when H != h.  (W, H) = (w, h)
+ * is T unchanged.  heic_b200_resample_coeffs gives the tables.  Decoding and the colour stage are unchanged: the
+ * resampling runs after them on the GPU.  Resizes of {0, 0, 0} give the _reduced output (those calls are these with
+ * every resize {0, 0, 0}); sizes, filters, factors and transforms may differ between images.  Exactly one side 0, a side
+ * above 32768, or a filter outside 1..5 (HEIC_RESAMPLE_*) fails the whole call with HEIC_E_INVALID_ARG before anything is
+ * queued.  (NEAREST, reducing_gap and fractional source boxes are not offered.) */
+int32_t heic_b200_decode_grids_resized(heic_b200_ctx* ctx, const heic_image_desc* imgs, const heic_image_transform* xforms,
+                                       const uint32_t* reduce, const heic_resize* resize, uint32_t n_imgs, uint8_t* rgb_out,
+                                       size_t pitch, size_t image_stride, heic_tile_status* status);
+int32_t heic_b200_decode_grids_submit_resized(heic_b200_ctx* ctx, const heic_image_desc* imgs,
+                                              const heic_image_transform* xforms, const uint32_t* reduce,
+                                              const heic_resize* resize, uint32_t n_imgs, uint8_t* rgb_out, size_t pitch,
+                                              size_t image_stride, heic_tile_status* status, heic_b200_job** out_job);
+/* The fixed-point table of one axis n_in -> n_out under a filter (HOST only; no device needed): bounds (2 * n_out entries,
+ * may be NULL) receives (xmin, n) per output index; coeffs (may be NULL) receives the k[x] of every output index back to
+ * back, output 0 first.  Returns the number of coefficients, or HEIC_E_INVALID_ARG for n_in = 0, n_out outside 1..32768,
+ * a filter outside 1..5 or coeffs_cap smaller than the count. */
+int64_t heic_b200_resample_coeffs(uint32_t n_in, uint32_t n_out, uint32_t filter, int32_t* bounds, int32_t* coeffs,
+                                  size_t coeffs_cap);
+
 /* Same, planar YCbCr out (tile mosaic cropped to the output canvas, no colour conversion): Y plane
  * output_width x output_height, then Cb, Cr at half resolution (rounded up), per image.  Tiles are stitched at their
  * conformance-window size; no transform is applied.  */
@@ -355,6 +395,11 @@ int32_t heic_b200_batch_create_transformed(heic_b200_ctx* ctx, const heic_image_
  * batch's RGB output, its pitch and its image stride are those of the reduced images. */
 int32_t heic_b200_batch_create_reduced(heic_b200_ctx* ctx, const heic_image_desc* imgs, const heic_image_transform* xforms,
                                        const uint32_t* reduce, uint32_t n_imgs, heic_b200_batch** out);
+/* The same with a resize per image (see heic_b200_decode_grids_resized for the definition): the batch's RGB output, its
+ * pitch and its image stride are those of the resized images. */
+int32_t heic_b200_batch_create_resized(heic_b200_ctx* ctx, const heic_image_desc* imgs, const heic_image_transform* xforms,
+                                       const uint32_t* reduce, const heic_resize* resize, uint32_t n_imgs,
+                                       heic_b200_batch** out);
 void    heic_b200_batch_destroy(heic_b200_batch* b);
 /* Runs slice data -> RGB for the whole batch on the context's stream; does not synchronise. */
 int32_t heic_b200_batch_decode(heic_b200_batch* b);

@@ -25,6 +25,12 @@ pub const HEIC_STAGE_ALL: u32 = 63;
 
 pub const HEIC_MAX_ENTRY_POINTS: usize = 255;
 
+pub const HEIC_RESAMPLE_LANCZOS: u32 = 1;
+pub const HEIC_RESAMPLE_BILINEAR: u32 = 2;
+pub const HEIC_RESAMPLE_BICUBIC: u32 = 3;
+pub const HEIC_RESAMPLE_BOX: u32 = 4;
+pub const HEIC_RESAMPLE_HAMMING: u32 = 5;
+
 #[repr(C)]
 #[derive(Clone, Copy)]
 pub struct heic_scaling_list {
@@ -331,6 +337,15 @@ pub struct heic_image_transform {
     pub orientation: u32,
 }
 
+/// Output size and filter (`HEIC_RESAMPLE_*`) of a resize; all zero: no resize.
+#[repr(C)]
+#[derive(Clone, Copy, Default)]
+pub struct heic_resize {
+    pub width: u32,
+    pub height: u32,
+    pub filter: u32,
+}
+
 #[repr(C)]
 #[derive(Clone, Copy, Default)]
 pub struct heic_tile_status {
@@ -454,6 +469,19 @@ extern "C" {
         n_imgs: u32, rgb_out: *mut u8, pitch: usize, image_stride: usize, status: *mut heic_tile_status,
         out_job: *mut *mut heic_b200_job,
     ) -> i32;
+    pub fn heic_b200_decode_grids_resized(
+        ctx: *mut heic_b200_ctx, imgs: *const heic_image_desc, xforms: *const heic_image_transform, reduce: *const u32,
+        resize: *const heic_resize, n_imgs: u32, rgb_out: *mut u8, pitch: usize, image_stride: usize,
+        status: *mut heic_tile_status,
+    ) -> i32;
+    pub fn heic_b200_decode_grids_submit_resized(
+        ctx: *mut heic_b200_ctx, imgs: *const heic_image_desc, xforms: *const heic_image_transform, reduce: *const u32,
+        resize: *const heic_resize, n_imgs: u32, rgb_out: *mut u8, pitch: usize, image_stride: usize,
+        status: *mut heic_tile_status, out_job: *mut *mut heic_b200_job,
+    ) -> i32;
+    pub fn heic_b200_resample_coeffs(
+        n_in: u32, n_out: u32, filter: u32, bounds: *mut i32, coeffs: *mut i32, coeffs_cap: usize,
+    ) -> i64;
     pub fn heic_b200_decode_grids_yuv(
         ctx: *mut heic_b200_ctx, imgs: *const heic_image_desc, n_imgs: u32, y_out: *mut u8, cb_out: *mut u8,
         cr_out: *mut u8, status: *mut heic_tile_status,
@@ -475,6 +503,10 @@ extern "C" {
     pub fn heic_b200_batch_create_reduced(
         ctx: *mut heic_b200_ctx, imgs: *const heic_image_desc, xforms: *const heic_image_transform, reduce: *const u32,
         n_imgs: u32, out: *mut *mut heic_b200_batch,
+    ) -> i32;
+    pub fn heic_b200_batch_create_resized(
+        ctx: *mut heic_b200_ctx, imgs: *const heic_image_desc, xforms: *const heic_image_transform, reduce: *const u32,
+        resize: *const heic_resize, n_imgs: u32, out: *mut *mut heic_b200_batch,
     ) -> i32;
     pub fn heic_b200_batch_destroy(b: *mut heic_b200_batch);
     pub fn heic_b200_batch_decode(b: *mut heic_b200_batch) -> i32;
