@@ -19,10 +19,61 @@ namespace dev {
 
 namespace {
 
-__constant__ int8_t kIntraPredAngle[35] = {0,   0,   32,  26,  21,  17, 13, 9,  5,  2,  0,  -2, -5, -9, -13, -17, -21, -26,
-                                               -32, -26, -21, -17, -13, -9, -5, -2, 0,  2,  5,  9,  13, 17, 21,  26,  32};
-__constant__ int16_t kInvAngle[15] = {-4096, -1638, -910, -630, -482, -390, -315, -256,
-                                          -315,  -390,  -482, -630, -910, -1638, -4096};  // modes 11..25
+struct Angles {
+  int8_t angle[35];
+  int16_t inv[15];  // modes 11..25
+};
+constexpr Angles kAngles = {{0,   0,   32,  26,  21,  17, 13, 9,  5,  2,  0,  -2, -5, -9, -13, -17, -21, -26,
+                             -32, -26, -21, -17, -13, -9, -5, -2, 0,  2,  5,  9,  13, 17, 21,  26,  32},
+                            {-4096, -1638, -910, -630, -482, -390, -315, -256, -315, -390, -482, -630, -910, -1638, -4096}};
+__constant__ Angles kAng = kAngles;
+
+// ---- 4x4 prediction as a table: for mode m and output sample p = (x, y) = (p & 3, p >> 2), word [m * 16 + p] holds
+//   bits 0-4 / 8-12   the lanes A and B of the two reference samples the sample is weighed from (lane s holds scan
+//                     position s: left(i) = lane 8 - i, top(i) = lane 8 + i), as shuffle source lanes;
+//   bits 16-23 / 24-31 their weights wA and wB;
+//   bits 5-7          DC: the weight of the DC value in the luma edge filter (8.4.4.2.5);
+//   bit 13            modes 10 / 26: the sample lies on the luma edge the filter of 8.4.4.2.6 adjusts.
+// Angular (8.4.4.2.6): A, B = ref[iIdx + 1], ref[iIdx + 2] (negative indices projected onto the other edge), wA = 32 - iFact,
+// wB = iFact; for modes 10 and 26 (iFact = 0) B is the opposite edge's sample the edge filter needs.  Planar and DC: A =
+// left(y + 1), B = top(x + 1); planar weights (3 - x, 3 - y), DC (x == 0, y == 0).  A lane's whole mode-dependent set-up is one
+// load instead of a branch per mode class.
+struct Pred4Table {
+  uint32_t w[35 * 16];
+};
+constexpr Pred4Table make_pred4_table() {
+  Pred4Table t{};
+  for (int m = 0; m < 35; m++) {
+    for (int p = 0; p < 16; p++) {
+      const int x = p & 3, y = p >> 2;
+      int la = 7 - y, lb = 9 + x, wa = 0, wb = 0, low = 0;  // planar / DC: left(y + 1), top(x + 1)
+      if (m == 0) {
+        wa = 3 - x, wb = 3 - y;
+      } else if (m == 1) {
+        wa = x == 0, wb = y == 0, low = (4 - wa - wb) << 5;
+      } else {
+        const int angle = kAngles.angle[m];
+        const bool vertical = m >= 18;
+        const int dir = vertical ? 1 : -1;
+        const int tt = ((vertical ? y : x) + 1) * angle, fact = tt & 31;
+        const int t1 = (vertical ? x : y) + (tt >> 5) + 1;
+        la = 8 + dir * t1;
+        lb = la + dir;
+        if (angle < 0) {
+          const int inv = kAngles.inv[m - 11];
+          if (t1 < 0) la = 8 - dir * ((t1 * inv + 128) >> 8);
+          if (t1 + 1 < 0) lb = 8 - dir * (((t1 + 1) * inv + 128) >> 8);
+        }
+        wa = 32 - fact, wb = fact;
+        if (m == 26) lb = 7 - y, low = x == 0 ? 1 << 13 : 0;  // v = top(1) + ((left(y + 1) - corner) >> 1) at x = 0
+        if (m == 10) lb = 9 + x, low = y == 0 ? 1 << 13 : 0;  // v = left(1) + ((top(x + 1) - corner) >> 1) at y = 0
+      }
+      t.w[m * 16 + p] = (uint32_t)(la & 31) | ((uint32_t)(lb & 31) << 8) | (uint32_t)low | ((uint32_t)wa << 16) | ((uint32_t)wb << 24);
+    }
+  }
+  return t;
+}
+__device__ const Pred4Table kPred4 = make_pred4_table();
 
 __device__ __forceinline__ uint32_t compact1(uint32_t v) {
   v &= 0x55u;
@@ -94,8 +145,65 @@ __device__ __forceinline__ uint32_t block_availability(const Ctu& c, int sub, in
   return (uint32_t)lo | ((uint32_t)hi << 8);
 }
 
-// Predicts and reconstructs the N x N block at (bx, by) (plane samples, CTU-relative) of one plane, or — `pair` — of
-// the two chroma planes together (same geometry and mode; buffers `buf_delta` and residuals `res_delta` apart), which
+// Fields of a transform unit's per-plane word (luma, or the chroma pair), packed for 32 units at a time by the CTU walk:
+// mode in bits 14-19, cbf (Cb's for a pair) in bit 29, Cr's cbf in bit 30, and
+//   bit 31 set (4x4 block): bits 0-13 the CTU-buffer offset of the block's corner sample (-1, -1), bits 20-23 / 24-28 the
+//                           available reference interval (lo, hi) of block_availability();
+//   bit 31 clear (larger):  bits 0-3 / 4-7 the block position bx / 4, by / 4, bits 8-10 log2 of its size; (lo, hi) in a
+//                           separate word.
+constexpr uint32_t kW4 = 1u << 31, kWCbfA = 1u << 29, kWCbfB = 1u << 30;
+
+// Predicts and reconstructs a 4x4 block of one plane, or — `pair` — the Cb and Cr blocks of a chroma pair (same geometry and
+// mode; buffers `buf_delta` and residuals `res_delta` apart).  The 17 reference samples sit in lanes 0..16 (lane s holds scan
+// position s; a pair's Cr sample in the upper halfword beside the Cb one, so one shuffle and one multiply serve both
+// blocks), lane p < 16 predicts sample (p & 3, p >> 2) with what kPred4 says for it; no reference arrays, no smoothing at
+// this size, one warp barrier.  The edge filters of DC / horizontal / vertical are luma only.
+__device__ __forceinline__ void predict4(int lane, bool pair, uint8_t* buf, int buf_delta, int stride, uint32_t w, int mode,
+                                         const int16_t* __restrict__ resid, int res_delta) {
+  const uint8_t* corner = buf + (w & 0x3fffu);  // sample (-1, -1)
+  const int lo = (w >> 20) & 15, hi = (w >> 24) & 31;
+  const uint32_t tw = __ldg(&kPred4.w[mode * 16 + (lane & 15)]);
+  uint32_t r;
+  {
+    const int d = min(max(lane, lo), hi) - 8;  // lanes above 16 fetch position hi again: in bounds, unused
+    const int off = d <= 0 ? -d * stride : d;
+    r = corner[off];
+    if (pair) r |= (uint32_t)corner[off + buf_delta] << 16;
+    if (lo > hi) r = pair ? 0x800080u : 0x80u;  // nothing available: 1 << (bitDepth - 1)
+  }
+  const uint32_t a = __shfl_sync(0xffffffffu, r, (int)tw), b = __shfl_sync(0xffffffffu, r, (int)(tw >> 8));
+  uint32_t acc = ((tw >> 16) & 0xffu) * a + (tw >> 24) * b;  // per halfword: below 2^16
+  int v0, v1;
+  if (mode >= 2) {  // 8.4.4.2.6
+    acc += 0x100010u;
+    v0 = (int)((acc & 0xffffu) >> 5), v1 = (int)(acc >> 21);
+    if (!pair && (mode == 10 || mode == 26)) {
+      const int c0 = __shfl_sync(0xffffffffu, (int)r, 8);
+      if (tw & (1u << 13)) v0 = clip8((int)a + (((int)b - c0) >> 1));
+    }
+  } else if (mode == 0) {  // 8.4.4.2.4
+    const uint32_t tr = __shfl_sync(0xffffffffu, r, 13), bl = __shfl_sync(0xffffffffu, r, 3);
+    acc += (uint32_t)((lane & 3) + 1) * tr + (uint32_t)(((lane >> 2) & 3) + 1) * bl + 0x40004u;
+    v0 = (int)((acc & 0xffffu) >> 3), v1 = (int)(acc >> 19);
+  } else {  // 8.4.4.2.5: both blocks of a pair summed in one reduction (each sum < 2^11)
+    const uint32_t sums = __reduce_add_sync(0xffffffffu, ((0x1ef0u >> lane) & 1u) ? r : 0u);  // lanes 4..7, 9..12
+    v0 = (int)(((sums & 0xffffu) + 4) >> 3), v1 = (int)(((sums >> 16) + 4) >> 3);
+    if (!pair) v0 = (int)(acc + ((tw >> 5) & 7u) * (uint32_t)v0 + 2) >> 2;
+  }
+  if (lane < 16) {
+    uint8_t* o = buf + (w & 0x3fffu) + 1 + ((lane >> 2) + 1) * stride + (lane & 3);
+    if (w & kWCbfA) v0 = clip8(v0 + (int)resid[lane]);
+    o[0] = (uint8_t)v0;
+    if (pair) {
+      if (w & kWCbfB) v1 = clip8(v1 + (int)resid[res_delta + lane]);
+      o[buf_delta] = (uint8_t)v1;
+    }
+  }
+  __syncwarp();
+}
+
+// Predicts and reconstructs the N x N block at (bx, by) (plane samples, CTU-relative, N >= 8) of one plane, or — `pair` —
+// of the two chroma planes together (same geometry and mode; buffers `buf_delta` and residuals `res_delta` apart), which
 // shares the availability logic and the loop overheads between Cb and Cr.  A lane produces four horizontally adjacent
 // samples per step.  Deliberately one compact, size-generic body with a single call site: the kernel is
 // instruction-fetch bound when this code is replicated per size and per component.
@@ -106,78 +214,6 @@ __device__ __forceinline__ void predict_block(const Ctu& c, bool pair, uint8_t* 
   const int N = 1 << log2, lane = c.lane;
   const int total = 4 * N, cnt = total + 1;  // positions 0 .. 4N: s < 2N left column bottom-up, s = 2N corner, s > 2N top row
   uint8_t* ref = c.ref;
-  if (log2 == 2) {
-    // ---- 4x4 blocks (most calls): the 17 reference samples live in lanes 0..16 (lane s holds scan position s, so
-    // left(i) is lane 8 - i and top(i) lane 8 + i), the 16 samples in lanes 0..15, and shuffles replace the reference
-    // arrays, their loops and two warp barriers.  No smoothing at this size.  A chroma pair runs the same shuffles on a
-    // second register (same mode, same geometry); the edge filters of DC / horizontal / vertical are luma only.
-    const uint8_t* corner = buf + by * stride + bx + kApron - 1;  // sample (-1, -1)
-    int r = 128, r2 = 128;
-    if (lane <= 16 && lo <= hi) {
-      const int d = min(max(lane, lo), hi) - 8;
-      const int off = d <= 0 ? -d * stride : d;
-      r = corner[off];
-      if (pair) r2 = corner[off + buf_delta];
-    }
-    const int x = lane & 3, y = (lane >> 2) & 3;
-    const bool luma = !pair;
-    int v, v2 = 0;
-    const int L = __shfl_sync(0xffffffffu, r, 7 - y), T = __shfl_sync(0xffffffffu, r, 9 + x);  // left(1 + y), top(1 + x)
-    int L2 = 0, T2 = 0;
-    if (pair) L2 = __shfl_sync(0xffffffffu, r2, 7 - y), T2 = __shfl_sync(0xffffffffu, r2, 9 + x);
-    if (mode == 0) {
-      const int tr = __shfl_sync(0xffffffffu, r, 13), bl = __shfl_sync(0xffffffffu, r, 3);
-      v = ((3 - x) * L + (x + 1) * tr + (3 - y) * T + (y + 1) * bl + 4) >> 3;
-      if (pair) {
-        const int tr2 = __shfl_sync(0xffffffffu, r2, 13), bl2 = __shfl_sync(0xffffffffu, r2, 3);
-        v2 = ((3 - x) * L2 + (x + 1) * tr2 + (3 - y) * T2 + (y + 1) * bl2 + 4) >> 3;
-      }
-    } else if (mode == 1) {
-      const bool in_sum = (lane >= 4 && lane <= 7) || (lane >= 9 && lane <= 12);
-      // both sums in one reduction (each < 2^11)
-      const unsigned sums = __reduce_add_sync(0xffffffffu, in_sum ? (unsigned)r | ((unsigned)r2 << 16) : 0u);
-      const int dc = ((int)(sums & 0xffffu) + 4) >> 3;
-      v = dc;
-      v2 = ((int)(sums >> 16) + 4) >> 3;
-      if (luma) {
-        if (y == 0) v = x == 0 ? (L + 2 * dc + T + 2) >> 2 : (T + 3 * dc + 2) >> 2;
-        else if (x == 0) v = (L + 3 * dc + 2) >> 2;
-      }
-    } else {
-      const int angle = kIntraPredAngle[mode];
-      const bool vertical = mode >= 18;
-      const int dir = vertical ? 1 : -1;
-      const int t = ((vertical ? y : x) + 1) * angle, fact = t & 31;
-      const int t1 = (vertical ? x : y) + (t >> 5) + 1;
-      int la = 8 + dir * t1, lb = la + dir;
-      if (angle < 0) {  // negative positions of the angular array are projections of the other edge
-        const int inv = kInvAngle[mode - 11];
-        if (t1 < 0) la = 8 - dir * ((t1 * inv + 128) >> 8);
-        if (t1 + 1 < 0) lb = 8 - dir * (((t1 + 1) * inv + 128) >> 8);
-      }
-      const int a = __shfl_sync(0xffffffffu, r, la), b = __shfl_sync(0xffffffffu, r, lb);  // b unused when fact == 0
-      v = ((32 - fact) * a + fact * b + 16) >> 5;
-      if (pair) {
-        const int a2 = __shfl_sync(0xffffffffu, r2, la), b2 = __shfl_sync(0xffffffffu, r2, lb);
-        v2 = ((32 - fact) * a2 + fact * b2 + 16) >> 5;
-      } else if (mode == 26 || mode == 10) {
-        const int c0 = __shfl_sync(0xffffffffu, r, 8), t1s = __shfl_sync(0xffffffffu, r, 9), l1s = __shfl_sync(0xffffffffu, r, 7);
-        if (mode == 26 && x == 0) v = clip8(t1s + ((L - c0) >> 1));
-        if (mode == 10 && y == 0) v = clip8(l1s + ((T - c0) >> 1));
-      }
-    }
-    if (lane < 16) {
-      uint8_t* o = buf + (by + 1 + y) * stride + bx + kApron + x;
-      if (cbf_a) v = clip8(v + (int)resid[lane]);
-      o[0] = (uint8_t)v;
-      if (pair) {
-        if (cbf_b) v2 = clip8(v2 + (int)resid[res_delta + lane]);
-        o[buf_delta] = (uint8_t)v2;
-      }
-    }
-    __syncwarp();
-    return;
-  }
   {
     const uint8_t* corner = buf + by * stride + bx + kApron - 1;  // sample (-1, -1)
     const int n_ref = pair ? 2 * cnt : cnt;
@@ -231,7 +267,7 @@ __device__ __forceinline__ void predict_block(const Ctu& c, bool pair, uint8_t* 
   uint8_t* out = buf + (by + 1) * stride + bx + kApron;
   // mode-specific setup
   int dc_pack = 0;
-  const int angle = kIntraPredAngle[mode];
+  const int angle = kAng.angle[mode];
   const bool vertical = mode >= 18;
   if (mode == 1) {  // 8.4.4.2.5 DC: both blocks of a pair summed in one packed reduction (each sum < 2^16)
     if (lane < N) {
@@ -252,7 +288,7 @@ __device__ __forceinline__ void predict_block(const Ctu& c, bool pair, uint8_t* 
       if (angle < 0) {
         const int last = (N * angle) >> 5;
         const int i = -1 - lane;  // |last| <= N <= 32: one step
-        if (last < -1 && i >= last) ra[i] = Rp[-dir * ((i * (int)kInvAngle[mode - 11] + 128) >> 8)];
+        if (last < -1 && i >= last) ra[i] = Rp[-dir * ((i * (int)kAng.inv[mode - 11] + 128) >> 8)];
       }
     }
     __syncwarp();
@@ -462,47 +498,57 @@ __global__ void __maxnreg__(HEIC_INTRA_MAXNREG) intra_kernel(Arenas A, const uin
         }
       }
       // ---- transform units of this CTB in z-order -----------------------------------------------------
-      // Everything about a transform unit that is arithmetic on its tu_map word and position (block coordinates, modes,
-      // cbfs, the availability intervals of its luma block and of its chroma pair) is worked out for 32 units at a time,
-      // one lane per 4x4 unit; the sequential walk below then only fetches three words per unit with shuffles.
+      // Everything about a transform unit that is arithmetic on its tu_map word and position (block positions, modes, cbfs,
+      // the availability intervals of its luma block and of its chroma pair) is worked out for 32 units at a time, one lane
+      // per 4x4 unit, into the per-plane words described at kW4; the sequential walk below then fetches two words per unit
+      // with shuffles (a third one for a block larger than 4x4).
       {
         const int buf_delta = (int)(c.buf[2] - c.buf[1]), res_delta = (int)(c.res[2] - c.res[1]);
 #pragma unroll 1
         for (int base = 0; base < n4sq; base += 32) {
           const int idx_l = base + lane;
           const uint32_t wl = idx_l < n4sq ? c.tuw[idx_l] : 0u;
-          uint32_t pa = 0, pb = 0, pc = 0;
+          uint32_t pa = 0, pb = 0, pc = 0;  // luma word, availability of the larger blocks (luma | chroma << 16), chroma word
           if (wl & TU_ORIGIN) {
             const int lg = (int)tu_log2(wl);
             const int bxl = (int)compact1((uint32_t)idx_l) << 2, byl = (int)compact1((uint32_t)idx_l >> 1) << 2;
-            pa = (uint32_t)bxl | ((uint32_t)byl << 6) | ((uint32_t)lg << 12) | (tu_luma_mode(wl) << 15) | ((wl & TU_CBF_Y) ? 1u << 21 : 0u);
-            pb = block_availability(c, 0, bxl, byl, lg);
+            const uint32_t avl = block_availability(c, 0, bxl, byl, lg);
+            pa = (tu_luma_mode(wl) << 14) | ((wl & TU_CBF_Y) ? kWCbfA : 0u);
+            if (lg == 2) pa |= kW4 | ((avl & 15u) | (avl >> 4)) << 20 | (uint32_t)(byl * c.stride[0] + bxl + kApron - 1);
+            else pa |= (uint32_t)(bxl >> 2) | ((uint32_t)(byl >> 2) << 4) | ((uint32_t)lg << 8), pb = avl;
             if ((wl & TU_HAS_CHROMA) && n_planes == 3) {
               const int lgc = lg > 2 ? lg - 1 : 2;
               const int bxc = (lg > 2 ? bxl : bxl - 4) >> 1, byc = (lg > 2 ? byl : byl - 4) >> 1;
-              pa |= (1u << 22) | ((wl & TU_CBF_CB) ? 1u << 23 : 0u) | ((wl & TU_CBF_CR) ? 1u << 24 : 0u);
-              pb |= block_availability(c, 1, bxc, byc, lgc) << 16;
-              pc = tu_chroma_mode(wl) | ((uint32_t)bxc << 6) | ((uint32_t)byc << 12) | ((uint32_t)lgc << 18);
+              const uint32_t avc = block_availability(c, 1, bxc, byc, lgc);
+              pc = (tu_chroma_mode(wl) << 14) | ((wl & TU_CBF_CB) ? kWCbfA : 0u) | ((wl & TU_CBF_CR) ? kWCbfB : 0u);
+              if (lgc == 2) pc |= kW4 | ((avc & 15u) | (avc >> 4)) << 20 | (uint32_t)(byc * c.stride[1] + bxc + kApron - 1);
+              else pc |= (uint32_t)(bxc >> 2) | ((uint32_t)(byc >> 2) << 4) | ((uint32_t)lgc << 8), pb |= avc << 16;
             }
           }
           uint32_t todo = __ballot_sync(0xffffffffu, (wl & TU_ORIGIN) != 0);
           while (todo) {  // warp-uniform
             const int src = __ffs(todo) - 1;
             todo &= todo - 1;
-            const uint32_t a = __shfl_sync(0xffffffffu, pa, src), b = __shfl_sync(0xffffffffu, pb, src);
-            const uint32_t cc = __shfl_sync(0xffffffffu, pc, src);
+            const uint32_t wc = __shfl_sync(0xffffffffu, pc, src);  // non-zero iff the unit carries the chroma pair
+            uint32_t w = __shfl_sync(0xffffffffu, pa, src);
             const int idx = base + src;
-            // luma, then (when this unit carries them) Cb and Cr as a pair: ONE call site keeps the kernel's code small
-            const int n_calls = (int)((a >> 22) & 1u) + 1;
+            // luma, then (when this unit carries them) Cb and Cr as a pair: ONE call site per body keeps the kernel small
 #pragma unroll 1
-            for (int k = 0; k < n_calls; k++) {
+            for (int k = 0;; k++) {
               const bool pr = k != 0;
-              const uint32_t geo = pr ? cc >> 6 : a;        // bx | by << 6 | log2 << 12
-              const uint32_t av = pr ? b >> 16 : b;         // lo | hi << 8
-              predict_block(c, pr, pr ? c.buf[1] : c.buf[0], pr ? buf_delta : 0, pr ? c.stride[1] : c.stride[0], (int)(geo & 63u),
-                            (int)((geo >> 6) & 63u), (int)((geo >> 12) & 7u), (int)((pr ? cc : a >> 15) & 63u), ((a >> (pr ? 23 : 21)) & 1u) != 0,
-                            pr && ((a >> 24) & 1u), pr ? c.res[1] + (idx >> 2) * 16 : c.res[0] + idx * 16, pr ? res_delta : 0,
-                            (int)(av & 0xffu), (int)((av >> 8) & 0xffu));
+              uint8_t* buf = pr ? c.buf[1] : c.buf[0];
+              const int stride = pr ? c.stride[1] : c.stride[0];
+              const int16_t* resid = pr ? c.res[1] + (idx >> 2) * 16 : c.res[0] + idx * 16;
+              const int mode = (int)((w >> 14) & 63u);
+              if (w & kW4) {
+                predict4(lane, pr, buf, buf_delta, stride, w, mode, resid, res_delta);
+              } else {
+                const uint32_t av = __shfl_sync(0xffffffffu, pb, src) >> (pr ? 16 : 0);  // lo | hi << 8
+                predict_block(c, pr, buf, buf_delta, stride, (int)(w & 15u) << 2, (int)((w >> 4) & 15u) << 2, (int)((w >> 8) & 7u),
+                              mode, (w & kWCbfA) != 0, (w & kWCbfB) != 0, resid, res_delta, (int)(av & 0xffu), (int)((av >> 8) & 0xffu));
+              }
+              if (pr || !wc) break;
+              w = wc;
             }
           }
         }
