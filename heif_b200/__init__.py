@@ -265,6 +265,19 @@ def _transform_array(transforms, n: int):
     return arr
 
 
+def _output_options(images, apply_transforms, transforms, reduce, resize, resample):
+    """The per-image output options as the _resized entry points take them.  None when every option is at its default (the
+    whole canvas, turned by irot when apply_transforms is set; factor 1; no resize): the calls without arrays build those
+    on the C side.  Otherwise (the transforms as a list, their ctypes array, the factors' array, the resizes' array)."""
+    n = len(images)
+    ks, rs = _reduce_list(reduce, n), _resize_list(resize, n)
+    resized = any(r is not None for r in rs)
+    if transforms is None and not resized and all(k == 1 for k in ks):
+        return None
+    xf = _transform_array(transforms if transforms is not None else [canvas_transform(im, apply_transforms) for im in images], n)
+    return list(xf), xf, _reduce_array(ks), _resize_array(rs, _resample_list(resample, n) if resized else [0] * n)
+
+
 def _desc_array(images):
     arr = (K.ImageDesc * len(images))()
     for i, im in enumerate(images):
@@ -291,26 +304,13 @@ class Batch:
         self.resize = _resize_list(resize, len(self.images))
         self._arr = _desc_array(self.images)
         self._h = C.c_void_p()
-        if any(r is not None for r in self.resize):
-            xf = transforms if transforms is not None else [canvas_transform(im, self.apply_transforms) for im in self.images]
-            self._xf = _transform_array(xf, len(self.images))
-            self.transforms = list(self._xf)
-            rs = _resize_array(self.resize, _resample_list(resample, len(self.images)))
-            K.check(self._lib.heic_b200_batch_create_resized(dec._h, self._arr, self._xf, _reduce_array(self.reduce), rs,
-                                                             len(self.images), C.byref(self._h)))
-        elif any(k != 1 for k in self.reduce):
-            xf = transforms if transforms is not None else [canvas_transform(im, self.apply_transforms) for im in self.images]
-            self._xf = _transform_array(xf, len(self.images))
-            self.transforms = list(self._xf)
-            K.check(self._lib.heic_b200_batch_create_reduced(dec._h, self._arr, self._xf, _reduce_array(self.reduce), len(self.images),
-                                                             C.byref(self._h)))
-        elif transforms is None:
+        opts = _output_options(self.images, self.apply_transforms, transforms, self.reduce, self.resize, resample)
+        if opts is None:
             self.transforms = [canvas_transform(im, self.apply_transforms) for im in self.images]
             K.check(self._lib.heic_b200_batch_create_ex(dec._h, self._arr, len(self.images), int(self.apply_transforms), C.byref(self._h)))
         else:
-            self._xf = _transform_array(transforms, len(self.images))
-            self.transforms = list(self._xf)
-            K.check(self._lib.heic_b200_batch_create_transformed(dec._h, self._arr, self._xf, len(self.images), C.byref(self._h)))
+            self.transforms = opts[0]
+            K.check(self._lib.heic_b200_batch_create_resized(dec._h, self._arr, *opts[1:], len(self.images), C.byref(self._h)))
 
     def close(self):
         if self._h:
@@ -457,7 +457,8 @@ class HeicDecoder:
         (see Batch)."""
         images = list(images)
         arr = _desc_array(images)
-        xf = [None] * len(images) if transforms is None else list(transforms)
+        transforms = None if transforms is None else list(transforms)
+        xf = [None] * len(images) if transforms is None else transforms
         ks = _reduce_list(reduce, len(images))
         rs = _resize_list(resize, len(images))
         sizes = [_canvas(im, apply_transforms, t, k, r) for im, t, k, r in zip(images, xf, ks, rs)]
@@ -468,21 +469,13 @@ class HeicDecoder:
             out = np.empty((len(images), h, w, 3), np.uint8)
         n_tiles = sum(im.n_tiles for im in images)
         st = (K.TileStatus * n_tiles)()
-        if any(r is not None for r in rs):
-            xf = [canvas_transform(im, apply_transforms) if t is None else t for im, t in zip(images, xf)]
-            rc = self._lib.heic_b200_decode_grids_resized(self._h, arr, _transform_array(xf, len(images)), _reduce_array(ks),
-                                                          _resize_array(rs, _resample_list(resample, len(images))), len(images),
-                                                          out.ctypes.data, out.strides[1], out.strides[0], st)
-        elif any(k != 1 for k in ks):
-            xf = [canvas_transform(im, apply_transforms) if t is None else t for im, t in zip(images, xf)]
-            rc = self._lib.heic_b200_decode_grids_reduced(self._h, arr, _transform_array(xf, len(images)), _reduce_array(ks), len(images),
-                                                          out.ctypes.data, out.strides[1], out.strides[0], st)
-        elif transforms is None:
+        opts = _output_options(images, apply_transforms, transforms, ks, rs, resample)
+        if opts is None:
             rc = self._lib.heic_b200_decode_grids(self._h, arr, len(images), out.ctypes.data, out.strides[1], out.strides[0],
                                                   1 if apply_transforms else 0, st)
         else:
-            rc = self._lib.heic_b200_decode_grids_transformed(self._h, arr, _transform_array(xf, len(images)), len(images),
-                                                              out.ctypes.data, out.strides[1], out.strides[0], st)
+            rc = self._lib.heic_b200_decode_grids_resized(self._h, arr, *opts[1:], len(images), out.ctypes.data, out.strides[1],
+                                                          out.strides[0], st)
         if return_status:
             return out, rc, st
         K.check(rc)
@@ -496,26 +489,13 @@ class HeicDecoder:
         n_tiles = sum(im.n_tiles for im in images)
         st = (K.TileStatus * n_tiles)()
         job = C.c_void_p()
-        ks = _reduce_list(reduce, len(images))
-        rs = _resize_list(resize, len(images))
-        if any(r is not None for r in rs):
-            xf = transforms if transforms is not None else [canvas_transform(im, apply_transforms) for im in images]
-            K.check(self._lib.heic_b200_decode_grids_submit_resized(self._h, arr, _transform_array(xf, len(images)), _reduce_array(ks),
-                                                                    _resize_array(rs, _resample_list(resample, len(images))),
-                                                                    len(images), out.ctypes.data, out.strides[1], out.strides[0], st,
-                                                                    C.byref(job)))
-        elif any(k != 1 for k in ks):
-            xf = transforms if transforms is not None else [canvas_transform(im, apply_transforms) for im in images]
-            K.check(self._lib.heic_b200_decode_grids_submit_reduced(self._h, arr, _transform_array(xf, len(images)), _reduce_array(ks),
-                                                                    len(images), out.ctypes.data, out.strides[1], out.strides[0], st,
-                                                                    C.byref(job)))
-        elif transforms is None:
+        opts = _output_options(images, apply_transforms, transforms, reduce, resize, resample)
+        if opts is None:
             K.check(self._lib.heic_b200_decode_grids_submit(self._h, arr, len(images), out.ctypes.data, out.strides[1], out.strides[0],
                                                             1 if apply_transforms else 0, st, C.byref(job)))
         else:
-            K.check(self._lib.heic_b200_decode_grids_submit_transformed(self._h, arr, _transform_array(transforms, len(images)),
-                                                                        len(images), out.ctypes.data, out.strides[1],
-                                                                        out.strides[0], st, C.byref(job)))
+            K.check(self._lib.heic_b200_decode_grids_submit_resized(self._h, arr, *opts[1:], len(images), out.ctypes.data,
+                                                                    out.strides[1], out.strides[0], st, C.byref(job)))
         return (job, st, out)
 
     def unescape(self, nal_payload: bytes, data_offset: int = 0, substream_offsets=()):

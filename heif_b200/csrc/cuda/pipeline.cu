@@ -10,7 +10,6 @@
 #include <cstdlib>
 
 #include <algorithm>
-#include <cstdlib>
 #include <cstring>
 #include <map>
 #include <memory>
@@ -111,12 +110,8 @@ struct heic_b200_ctx {
   int cabac_tiles_per_cta = 32;  // 32: thread per substream, 1: warp per substream
   int cabac_slots = 0;           // 0: derive from the picture geometry
   int low_latency_tiles = 384;   // loads of at most this many tiles use the warp-per-substream CABAC mapping
-  int cabac_group_factor = 1;    // CABAC CTAs per 32 tiles; > 1 splits heavy groups (measured slower: a CTA costs its
-                                 // critical-path lane, not the sum of its lanes, so full warps are the cheapest)
   int intra_slots = 0;           // 0: automatic (wavefront for small batches, one warp per picture for large)
   int intra_single_warp_tiles = 2048;
-  int cabac_group_cap_pct = 0;   // > 0: a group's slice bytes are capped at this per cent of (batch slice bytes / resident CTAs), so the
-                                 // heaviest groups -- the kernel's critical path -- carry fewer than 32 lanes
   int cabac_plain_sort = 0;      // measurement knob: plain size sort, copies of a slice may share a warp (bench.py's upper bound)
   int cabac_resident = 0;        // persistent CABAC CTAs to launch; 0: as many as are resident at once (tests use 2)
   int cabac_persistent = 1;      // large batches: CABAC CTAs take group after group, warp by warp (no ramp-up / drain per group)
@@ -137,16 +132,31 @@ struct heic_b200_ctx {
   ~heic_b200_ctx();
 };
 
+// One image of a batch.  Everything but first_tile, pic and src_slot is planned before the batch is loaded (plan_image).
 struct ImageInfo {
   uint32_t first_tile, n_tiles, pic;
-  uint32_t grid_rows, grid_cols, out_w, out_h, rot_w, rot_h;  // rot_w x rot_h: the RGB output (oriented, reduced, resized)
+  uint32_t grid_rows, grid_cols, canvas_w, canvas_h;        // canvas: output_width x output_height of the descriptor
   uint32_t tile_w, tile_h, win_x, win_y;                    // conformance window of every tile (luma samples)
   uint32_t crop_x, crop_y, crop_w, crop_h, orientation;     // heic_image_transform
   uint32_t reduce;                                          // box reduction factor (1: none)
-  uint32_t src_w, src_h;                                    // size of the colour stage's output (oriented, reduced)
-  uint32_t filter;                                          // resize filter (HEIC_RESAMPLE_*); 0: rot_w x rot_h = src_w x src_h
+  uint32_t color_w, color_h;                                // size of the colour stage's output (oriented, reduced)
+  uint32_t rgb_w, rgb_h;                                    // the RGB output (oriented, reduced, resized)
+  uint32_t filter;                                          // resize filter (HEIC_RESAMPLE_*); 0: rgb_w x rgb_h = color_w x color_h
   uint32_t src_slot;                                        // resized images: index in the batch's source arena
   uint32_t full_range, matrix_coeffs;
+};
+
+// What one image's RGB output is: the crop and turn of its canvas, then the box reduction, then the resize.
+struct OutputSpec {
+  heic_image_transform xf;
+  uint32_t reduce;
+  heic_resize resize;
+};
+
+// An image planned and validated before anything is queued: its ImageInfo and the parameters of its decoded pictures.
+struct ImagePlan {
+  ImageInfo info;
+  PicParams pp;
 };
 
 namespace {
@@ -158,7 +168,7 @@ struct TileWindow {
 
 // Decoded picture, conformance window and output canvas of an image descriptor; throws for a window or a canvas that
 // the tiles do not cover.
-void image_geometry(const heic_image_desc& im, PicParams& pp, TileWindow& tw, uint32_t& out_w, uint32_t& out_h) {
+void image_geometry(const heic_image_desc& im, PicParams& pp, TileWindow& tw, uint32_t& canvas_w, uint32_t& canvas_h) {
   if (!im.tiles || im.n_tiles == 0 || im.n_tiles != im.grid_rows * im.grid_cols)
     bail(HEIC_E_INVALID_ARG, "image descriptor: n_tiles must equal grid_rows * grid_cols");
   make_pic_params(im.sps, im.pps, pp);
@@ -173,12 +183,12 @@ void image_geometry(const heic_image_desc& im, PicParams& pp, TileWindow& tw, ui
   const uint64_t mosaic_w = (uint64_t)im.grid_cols * tw.w, mosaic_h = (uint64_t)im.grid_rows * tw.h;
   const uint64_t ow = im.output_width ? im.output_width : mosaic_w, oh = im.output_height ? im.output_height : mosaic_h;
   if (ow > mosaic_w || oh > mosaic_h) bail(HEIC_E_BITSTREAM, "grid canvas is larger than the tile mosaic");
-  out_w = (uint32_t)ow;
-  out_h = (uint32_t)oh;
+  canvas_w = (uint32_t)ow;
+  canvas_h = (uint32_t)oh;
 }
 
-void check_transform(const heic_image_transform& x, uint32_t out_w, uint32_t out_h) {
-  if (x.orientation > 7 || !x.crop_w || !x.crop_h || (uint64_t)x.crop_x + x.crop_w > out_w || (uint64_t)x.crop_y + x.crop_h > out_h)
+void check_transform(const heic_image_transform& x, uint32_t canvas_w, uint32_t canvas_h) {
+  if (x.orientation > 7 || !x.crop_w || !x.crop_h || (uint64_t)x.crop_x + x.crop_w > canvas_w || (uint64_t)x.crop_y + x.crop_h > canvas_h)
     bail(HEIC_E_INVALID_ARG, "image transform: crop rectangle not inside the canvas, or orientation above 7");
 }
 
@@ -186,50 +196,77 @@ void check_reduce(uint32_t k) {
   if (k < 1 || k > 16) bail(HEIC_E_INVALID_ARG, "reduction factor outside 1..16");
 }
 
-// Size of the RGB output of a transform and a reduction factor: the crop, turned for odd quarter turns, then
-// ceil(w / k) x ceil(h / k).
-void output_size(const heic_image_transform& x, uint32_t k, uint32_t& w, uint32_t& h) {
-  const uint32_t ow = (x.orientation & 1u) ? x.crop_h : x.crop_w, oh = (x.orientation & 1u) ? x.crop_w : x.crop_h;
-  w = (ow + k - 1) / k;
-  h = (oh + k - 1) / k;
-}
-
-// What the calls without reduction factors apply: 1 for every image.
-std::vector<uint32_t> no_reduction(uint32_t n_imgs) { return std::vector<uint32_t>(std::max(n_imgs, 1u), 1u); }
-
 void check_resize(const heic_resize& r) {
   if ((r.width == 0) != (r.height == 0) || r.width > kResampleMaxSide || r.height > kResampleMaxSide ||
       (r.width && (r.filter < HEIC_RESAMPLE_LANCZOS || r.filter > HEIC_RESAMPLE_HAMMING)))
     bail(HEIC_E_INVALID_ARG, "resize: exactly one side 0, a side above 32768, or a filter outside 1..5");
 }
 
-// Size of the RGB output after the resize: the resize's size, or the colour stage's w x h when there is none.
-void resized_size(const heic_resize& r, uint32_t& w, uint32_t& h) {
-  if (r.width) w = r.width, h = r.height;
-}
-
-// What the calls without resizes apply: none.
-std::vector<heic_resize> no_resize(uint32_t n_imgs) {
-  return std::vector<heic_resize>(std::max(n_imgs, 1u), heic_resize{0, 0, 0});
-}
-
-// What the calls without transforms apply: the whole canvas, turned by irot when apply_transforms is set.
-std::vector<heic_image_transform> canvas_transforms(const heic_image_desc* imgs, uint32_t n_imgs, int32_t apply_transforms) {
+// One OutputSpec per image from the caller's arrays of n_imgs entries.  A null array is the default: the whole canvas,
+// turned by irot when apply_transforms is set; factor 1; no resize.  (A public call that takes an array rejects a null one
+// before it gets here.)
+std::vector<OutputSpec> output_specs(const heic_image_desc* imgs, uint32_t n_imgs, const heic_image_transform* xforms,
+                                     const uint32_t* reduce, const heic_resize* resize, int32_t apply_transforms) {
   if (!imgs) bail(HEIC_E_INVALID_ARG, "null argument");
-  std::vector<heic_image_transform> x(n_imgs);
+  std::vector<OutputSpec> specs(n_imgs);
   for (uint32_t i = 0; i < n_imgs; i++) {
-    PicParams pp;
-    TileWindow tw;
-    uint32_t ow, oh;
-    image_geometry(imgs[i], pp, tw, ow, oh);
-    x[i] = {0, 0, ow, oh, apply_transforms ? (imgs[i].rotation_ccw_quarter_turns & 3u) : 0u};
+    OutputSpec& s = specs[i];
+    if (xforms) {
+      s.xf = xforms[i];
+    } else {
+      PicParams pp;
+      TileWindow tw;
+      uint32_t cw, ch;
+      image_geometry(imgs[i], pp, tw, cw, ch);
+      s.xf = {0, 0, cw, ch, apply_transforms ? (imgs[i].rotation_ccw_quarter_turns & 3u) : 0u};
+    }
+    s.reduce = reduce ? reduce[i] : 1u;
+    s.resize = resize ? resize[i] : heic_resize{0, 0, 0};
   }
-  return x;
+  return specs;
+}
+
+// Plans one image: throws for an invalid descriptor or spec, checking in this order the descriptor and its canvas, the
+// transform, the factor, the resize and every tile's slice header.  Without RGB output (with_rgb = false) no resize runs.
+ImagePlan plan_image(const heic_image_desc& im, const OutputSpec& s, bool with_rgb) {
+  ImagePlan p;
+  ImageInfo& info = p.info;
+  TileWindow win;
+  image_geometry(im, p.pp, win, info.canvas_w, info.canvas_h);
+  check_transform(s.xf, info.canvas_w, info.canvas_h);
+  check_reduce(s.reduce);
+  check_resize(s.resize);
+  TileParams tp;
+  for (uint32_t t = 0; t < im.n_tiles; t++) make_tile_params(p.pp, im.pps, im.tiles[t], tp);
+  info.first_tile = info.pic = info.src_slot = 0;  // set by load()
+  info.n_tiles = im.n_tiles;
+  info.grid_rows = im.grid_rows;
+  info.grid_cols = im.grid_cols;
+  info.tile_w = win.w;
+  info.tile_h = win.h;
+  info.win_x = win.x;
+  info.win_y = win.y;
+  info.crop_x = s.xf.crop_x;
+  info.crop_y = s.xf.crop_y;
+  info.crop_w = s.xf.crop_w;
+  info.crop_h = s.xf.crop_h;
+  info.orientation = s.xf.orientation;
+  info.reduce = s.reduce;
+  // the crop, turned for odd quarter turns, then ceil(w / k) x ceil(h / k)
+  const bool turned = s.xf.orientation & 1u;
+  info.color_w = ((turned ? s.xf.crop_h : s.xf.crop_w) + s.reduce - 1) / s.reduce;
+  info.color_h = ((turned ? s.xf.crop_w : s.xf.crop_h) + s.reduce - 1) / s.reduce;
+  info.rgb_w = with_rgb && s.resize.width ? s.resize.width : info.color_w;
+  info.rgb_h = with_rgb && s.resize.width ? s.resize.height : info.color_h;
+  // a resize to the size it already has is Pillow's copy(): the colour stage writes the output
+  info.filter = info.rgb_w != info.color_w || info.rgb_h != info.color_h ? s.resize.filter : 0u;
+  info.full_range = im.sps.vui_parameters_present_flag ? im.sps.video_full_range_flag : 0u;
+  info.matrix_coeffs = im.sps.vui_parameters_present_flag ? im.sps.matrix_coeffs : 2u;
+  return p;
 }
 
 }  // namespace
 
-// Images in a row of a batch with equal (source size, target size, filter): one launch per resampling pass.
 // One distinct coefficient table of a load: its device layout sits in heic_b200_batch::rs_tables at these int32 offsets.
 struct ResampleTableRef {
   ResampleAxis ax;              // the pointers are filled in by run()
@@ -237,6 +274,7 @@ struct ResampleTableRef {
   uint32_t row0, row_end;       // as a vertical table: the first and one past the last source row it reads
 };
 
+// Images in a row of a batch with equal (source size, target size, filter): one launch per resampling pass.
 struct ResampleRun {
   uint32_t first, count;      // images
   int h_table, v_table;       // index into heic_b200_batch::rs_axes; -1: that pass does not run
@@ -279,7 +317,6 @@ struct heic_b200_batch {
   // d_rgb's allocation also holds, after the RGB output, the source arena (the colour stage's output of the resized
   // images; the output then holds the resized ones) and the uint8 rows of the horizontal pass of the two-pass images: one
   // allocation, so a context that alternates resized and unresized calls keeps the larger of the two layouts, not both.
-  // pass's uint8 rows of the images that take both passes
   DevBuf d_bitstream, d_params, d_tu, d_coeff, d_recon, d_final, d_ipm, d_ctd,
       d_qp, d_sao, d_wpp, d_status, d_rgb, d_list, d_list_count, d_raw, d_counters;
   PinnedBuf h_raw;
@@ -309,9 +346,11 @@ struct heic_b200_batch {
     for (int k = 0; k < LIST_CLASSES; k++) a.list_off[k] = list_off[k];
     return a;
   }
-  void load(const heic_image_desc* imgs, const heic_image_transform* xforms, const uint32_t* reduce, const heic_resize* resize,
-            uint32_t n_imgs, bool with_rgb);
+  void load(const heic_image_desc* imgs, const ImagePlan* plans, uint32_t n_imgs, bool with_rgb);
+  void layout_tiles(const heic_image_desc* imgs, const ImagePlan* plans, uint32_t n_imgs);
   void plan_resample();
+  void plan_cabac(const heic_image_desc* imgs, uint32_t n_imgs);
+  void upload(const heic_image_desc* imgs, uint32_t n_imgs, bool with_rgb);
   void run(uint32_t mask);
 };
 
@@ -330,16 +369,22 @@ heic_b200_ctx::~heic_b200_ctx() {
 }
 
 // ---- batch construction --------------------------------------------------------------------------------
-void heic_b200_batch::load(const heic_image_desc* imgs, const heic_image_transform* xforms, const uint32_t* reduce,
-                           const heic_resize* resize, uint32_t n_imgs, bool with_rgb) {
+// Loads planned images: arena layout, resampling, CABAC launch classes, then the uploads on the batch's stream.
+void heic_b200_batch::load(const heic_image_desc* imgs, const ImagePlan* plans, uint32_t n_imgs, bool with_rgb) {
+  layout_tiles(imgs, plans, n_imgs);
+  plan_resample();
+  if (tiles.size() >= (1u << 24)) bail(HEIC_E_UNSUPPORTED, "more than 2^24 tiles in one batch (the transform lists keep the tile index in 24 bits)");
+  plan_cabac(imgs, n_imgs);
+  upload(imgs, n_imgs, with_rgb);
+}
+
+// Per-tile parameters and the offsets of every tile's slice of the per-batch arenas; the RGB output's layout.
+void heic_b200_batch::layout_tiles(const heic_image_desc* imgs, const ImagePlan* plans, uint32_t n_imgs) {
   pics.clear();
   scaling.clear();
   tiles.clear();
   images.clear();
   substreams.clear();
-  order.clear();
-  heavy_first.clear();
-  classes.clear();
   raw_bytes = 0;
   any_plain = false;
   bs_bytes = tu_words = coeff_elems = plane_bytes = map4_bytes = map8_bytes = sao_words = wpp_bytes = 0;
@@ -349,20 +394,10 @@ void heic_b200_batch::load(const heic_image_desc* imgs, const heic_image_transfo
   intra_slots = 1;
   max_hctb = 1;
   stages_run = 0;
-  size_t max_rgb_rows = 0, max_rgb_pitch = 0, n_tiles_hint = 0;
-  for (uint32_t i = 0; i < n_imgs; i++) n_tiles_hint += imgs[i].n_tiles;
+  size_t max_rgb_rows = 0, max_rgb_pitch = 0;
   for (uint32_t i = 0; i < n_imgs; i++) {
     const heic_image_desc& im = imgs[i];
-    if (!im.tiles || im.n_tiles == 0 || im.n_tiles != im.grid_rows * im.grid_cols)
-      bail(HEIC_E_INVALID_ARG, "image descriptor: n_tiles must equal grid_rows * grid_cols");
-    PicParams pp;
-    TileWindow win;
-    uint32_t out_w, out_h;
-    image_geometry(im, pp, win, out_w, out_h);
-    const heic_image_transform& xf = xforms[i];
-    check_transform(xf, out_w, out_h);
-    check_reduce(reduce[i]);
-    check_resize(resize[i]);
+    PicParams pp = plans[i].pp;
     ScalingSet ss;
     build_scaling_set(im.sps, im.pps, ss);
     size_t s = 0;
@@ -373,39 +408,12 @@ void heic_b200_batch::load(const heic_image_desc* imgs, const heic_image_transfo
     // consecutive images with identical parameters share one PicParams entry
     if (pics.empty() || std::memcmp(&pics.back(), &pp, sizeof pp)) pics.push_back(pp);
     const uint32_t pic = (uint32_t)pics.size() - 1;
-    ImageInfo info;
+    ImageInfo info = plans[i].info;
     info.first_tile = (uint32_t)tiles.size();
-    info.n_tiles = im.n_tiles;
     info.pic = pic;
-    info.grid_rows = im.grid_rows;
-    info.grid_cols = im.grid_cols;
-    info.out_w = out_w;
-    info.out_h = out_h;
-    info.tile_w = win.w;
-    info.tile_h = win.h;
-    info.win_x = win.x;
-    info.win_y = win.y;
-    info.crop_x = xf.crop_x;
-    info.crop_y = xf.crop_y;
-    info.crop_w = xf.crop_w;
-    info.crop_h = xf.crop_h;
-    info.orientation = xf.orientation;
-    info.reduce = reduce[i];
-    output_size(xf, reduce[i], info.src_w, info.src_h);
-    info.rot_w = info.src_w;
-    info.rot_h = info.src_h;
-    resized_size(resize[i], info.rot_w, info.rot_h);
-    // a resize to the size it already has is Pillow's copy(): the colour stage writes the output
-    info.filter = (info.rot_w != info.src_w || info.rot_h != info.src_h) && with_rgb ? resize[i].filter : 0u;
-    if (!with_rgb) info.rot_w = info.src_w, info.rot_h = info.src_h;
-    info.src_slot = 0;
-    info.full_range = im.sps.vui_parameters_present_flag ? im.sps.video_full_range_flag : 0u;
-    info.matrix_coeffs = im.sps.vui_parameters_present_flag ? im.sps.matrix_coeffs : 2u;
     images.push_back(info);
-    const size_t pitch = up((size_t)info.rot_w * 3, 16);
-    max_rgb_pitch = std::max(max_rgb_pitch, pitch);
-    max_rgb_rows = std::max(max_rgb_rows, (size_t)info.rot_h);
-    const int ctb4 = 1 << (pp.log2_ctb - 2);
+    max_rgb_pitch = std::max(max_rgb_pitch, up((size_t)info.rgb_w * 3, 16));
+    max_rgb_rows = std::max(max_rgb_rows, (size_t)info.rgb_h);
     for (uint32_t t = 0; t < im.n_tiles; t++) {
       TileParams tp;
       std::memset(&tp, 0, sizeof tp);
@@ -446,7 +454,6 @@ void heic_b200_batch::load(const heic_image_desc* imgs, const heic_image_transfo
       tp.wpp_off = wpp_bytes;
       wpp_bytes += (size_t)pp.hctb * NUM_CTX_PAD;
       tiles.push_back(tp);
-      (void)ctb4;
     }
     max_tu = std::max(max_tu, (uint32_t)pp.n_tu);
     max_w = std::max(max_w, (uint32_t)pp.w);
@@ -460,13 +467,17 @@ void heic_b200_batch::load(const heic_image_desc* imgs, const heic_image_transfo
   rgb_pitch = max_rgb_pitch;
   // every image is written at the widest pitch: the stride holds the tallest image at that pitch
   rgb_image_stride = up(max_rgb_pitch * max_rgb_rows, 256);
-  plan_resample();
-  if (tiles.size() >= (1u << 24)) bail(HEIC_E_UNSUPPORTED, "more than 2^24 tiles in one batch (the transform lists keep the tile index in 24 bits)");
+}
 
-  // ---- CABAC launch classes: tiles with the same wavefront shape, heaviest first, TILES per CTA ----------
+// CABAC launch classes: tiles with the same wavefront shape, heaviest first, tiles_per_cta per CTA; and the intra
+// kernel's launch order.
+void heic_b200_batch::plan_cabac(const heic_image_desc* imgs, uint32_t n_imgs) {
+  order.clear();
+  heavy_first.clear();
+  classes.clear();
   // few tiles: a warp per substream finishes a 12 MP image in about half the time of the 32-tiles-per-CTA mapping
   // (the GPU is mostly empty either way); many tiles: thread per substream is 11x the throughput
-  tiles_per_cta = (ctx->cabac_tiles_per_cta == 32 && n_tiles_hint > (size_t)ctx->low_latency_tiles) ? 32 : 1;
+  tiles_per_cta = (ctx->cabac_tiles_per_cta == 32 && tiles.size() > (size_t)ctx->low_latency_tiles) ? 32 : 1;
   const int tpc = tiles_per_cta;
   // content fingerprint of every slice (four 8-byte samples): equal length + equal fingerprint = "the same picture again"
   std::vector<uint64_t> fingerprint(tiles.size(), 0);
@@ -506,73 +517,41 @@ void heic_b200_batch::load(const heic_image_desc* imgs, const heic_image_transfo
     c.order_off = (uint32_t)order.size();
     // Tiles stay sorted by slice size so that the lanes of a warp carry similar statistics: measured on a B200,
     // dealing heavy and light tiles round-robin into the same warp is 3.5x slower (the light lanes idle while one
-    // heavy lane runs at single-thread latency).  With group_factor > 1 the sorted list is additionally cut into
-    // groups of about equal slice bytes (heavy groups get fewer lanes); that measured slower too, see DESIGN.md.
+    // heavy lane runs at single-thread latency).  Groups of about equal slice bytes and a byte cap on the heaviest
+    // groups (fewer lanes for them) measured slower too, see DESIGN.md.
     c.n_groups = 0;
     if (tpc == 1) {
       for (uint32_t t : v) order.push_back(t);
       c.n_groups = (uint32_t)v.size();
     } else {
-      if (ctx->cabac_group_factor == 1) {
-        // Groups of 32 tiles of neighbouring slice size, NO TWO OF THEM BYTE-IDENTICAL.  The sorted list is seen as runs of
-        // identical slices (same length and same content fingerprint; a batch of distinct pictures has runs of one, and the
-        // groups are then simply consecutive blocks of the sorted list).  A group takes one tile from each of the first 32
-        // runs that still have one, so copies of a picture -- which would run converged in one warp and flatter the
-        // throughput, as a benchmark batch built from few distinct tiles does -- always land in different warps, while the
-        // lanes of a warp stay as similar in size as the input allows.
-        struct Run {
-          size_t first, left;
-        };
-        std::vector<Run> runs;
-        for (size_t i = 0; i < v.size();) {
-          size_t j = i + 1;
-          while (!ctx->cabac_plain_sort && j < v.size() && tiles[v[j]].bs_len == tiles[v[i]].bs_len && fingerprint[v[j]] == fingerprint[v[i]]) j++;
-          runs.push_back({i, j - i});
-          i = j;
+      // Groups of 32 tiles of neighbouring slice size, NO TWO OF THEM BYTE-IDENTICAL.  The sorted list is seen as runs of
+      // identical slices (same length and same content fingerprint; a batch of distinct pictures has runs of one, and the
+      // groups are then simply consecutive blocks of the sorted list).  A group takes one tile from each of the first 32
+      // runs that still have one, so copies of a picture -- which would run converged in one warp and flatter the
+      // throughput, as a benchmark batch built from few distinct tiles does -- always land in different warps, while the
+      // lanes of a warp stay as similar in size as the input allows.
+      struct Run {
+        size_t first, left;
+      };
+      std::vector<Run> runs;
+      for (size_t i = 0; i < v.size();) {
+        size_t j = i + 1;
+        while (!ctx->cabac_plain_sort && j < v.size() && tiles[v[j]].bs_len == tiles[v[i]].bs_len && fingerprint[v[j]] == fingerprint[v[i]]) j++;
+        runs.push_back({i, j - i});
+        i = j;
+      }
+      size_t head = 0;  // runs before `head` are exhausted
+      while (head < runs.size()) {
+        int n = 0;
+        for (size_t r = head; r < runs.size() && n < tpc; r++) {
+          if (!runs[r].left) continue;
+          order.push_back(v[runs[r].first++]);
+          runs[r].left--;
+          n++;
         }
-        uint64_t cap = ~0ull;
-        if (ctx->cabac_group_cap_pct > 0) {
-          uint64_t total = 0;
-          for (uint32_t t : v) total += tiles[t].bs_len;
-          cap = total / (uint64_t)(ctx->n_sm * 3) * (uint64_t)ctx->cabac_group_cap_pct / 100u;
-        }
-        size_t head = 0;  // runs before `head` are exhausted
-        while (head < runs.size()) {
-          int n = 0;
-          uint64_t wsum = 0;
-          for (size_t r = head; r < runs.size() && n < tpc; r++) {
-            if (!runs[r].left) continue;
-            if (n > 0 && wsum + tiles[v[runs[r].first]].bs_len > cap) break;  // sorted: the later runs are no lighter than allowed either
-            wsum += tiles[v[runs[r].first]].bs_len;
-            order.push_back(v[runs[r].first++]);
-            runs[r].left--;
-            n++;
-          }
-          while (head < runs.size() && !runs[head].left) head++;
-          if (!n) break;
-          for (; n < tpc; n++) order.push_back(0xffffffffu);
-          c.n_groups++;
-        }
-      } else {
-        // group_factor > 1: the sorted list cut into groups of about equal slice bytes (heavy groups get fewer lanes; measured
-        // slower: a CTA costs its critical-path lane, not the sum of its lanes)
-        uint64_t total = 0;
-        for (uint32_t t : v) total += tiles[t].bs_len;
-        const uint64_t target_groups = std::max<uint64_t>(1, (uint64_t)ctx->cabac_group_factor * ((v.size() + tpc - 1) / tpc));
-        const uint64_t w_target = std::max<uint64_t>(1, total / target_groups);
-        size_t i = 0;
-        while (i < v.size()) {
-          uint64_t wsum = 0;
-          int n = 0;
-          while (i < v.size() && n < tpc && (n == 0 || wsum + tiles[v[i]].bs_len <= w_target)) {
-            wsum += tiles[v[i]].bs_len;
-            order.push_back(v[i]);
-            i++;
-            n++;
-          }
-          for (; n < tpc; n++) order.push_back(0xffffffffu);
-          c.n_groups++;
-        }
+        while (head < runs.size() && !runs[head].left) head++;
+        for (; n < tpc; n++) order.push_back(0xffffffffu);
+        c.n_groups++;
       }
     }
     c.hctb = hctb;
@@ -585,8 +564,10 @@ void heic_b200_batch::load(const heic_image_desc* imgs, const heic_image_transfo
   heavy_first.resize(tiles.size());
   for (uint32_t t = 0; t < tiles.size(); t++) heavy_first[t] = t;
   std::stable_sort(heavy_first.begin(), heavy_first.end(), [&](uint32_t a, uint32_t b) { return tiles[a].bs_len > tiles[b].bs_len; });
+}
 
-  // ---- device memory + uploads: one pinned blob for all parameter tables, one for the slice data ------------------
+// Device memory and uploads: one pinned blob for all parameter tables, one for the slice data.
+void heic_b200_batch::upload(const heic_image_desc* imgs, uint32_t n_imgs, bool with_rgb) {
   cudaStream_t st = stream;
   if (any_plain) h_bitstream.ensure(bs_bytes + 16);
   if (raw_bytes) h_raw.ensure(raw_bytes + 16);
@@ -667,8 +648,8 @@ void heic_b200_batch::plan_resample() {
   for (ImageInfo& im : images) {
     if (!im.filter) continue;
     im.src_slot = (uint32_t)n_src++;
-    src_pitch = std::max(src_pitch, up((size_t)im.src_w * 3, 16));
-    max_rows = std::max(max_rows, (size_t)im.src_h);
+    src_pitch = std::max(src_pitch, up((size_t)im.color_w * 3, 16));
+    max_rows = std::max(max_rows, (size_t)im.color_h);
   }
   if (!n_src) return;
   src_image_stride = up(src_pitch * max_rows, 256);
@@ -726,19 +707,19 @@ void heic_b200_batch::plan_resample() {
     }
     const ImageInfo& im = images[i];
     size_t j = i + 1;
-    while (j < images.size() && images[j].filter == im.filter && images[j].src_w == im.src_w && images[j].src_h == im.src_h &&
-           images[j].rot_w == im.rot_w && images[j].rot_h == im.rot_h)
+    while (j < images.size() && images[j].filter == im.filter && images[j].color_w == im.color_w &&
+           images[j].color_h == im.color_h && images[j].rgb_w == im.rgb_w && images[j].rgb_h == im.rgb_h)
       j++;
     ResampleRun r;
     r.first = (uint32_t)i;
     r.count = (uint32_t)(j - i);
-    r.h_table = im.rot_w != im.src_w ? table(im.src_w, im.rot_w, im.filter) : -1;
-    r.v_table = im.rot_h != im.src_h ? table(im.src_h, im.rot_h, im.filter) : -1;
+    r.h_table = im.rgb_w != im.color_w ? table(im.color_w, im.rgb_w, im.filter) : -1;
+    r.v_table = im.rgb_h != im.color_h ? table(im.color_h, im.rgb_h, im.filter) : -1;
     r.row0 = 0;
-    r.rows = im.src_h;
+    r.rows = im.color_h;
     if (r.v_table >= 0) r.row0 = rs_axes[r.v_table].row0, r.rows = rs_axes[r.v_table].row_end - r.row0;
     r.tmp_off = tmp_bytes;
-    r.tmp_pitch = up((size_t)im.rot_w * 3, 16);
+    r.tmp_pitch = up((size_t)im.rgb_w * 3, 16);
     r.tmp_stride = up(r.tmp_pitch * r.rows, 256);
     if (r.h_table >= 0 && r.v_table >= 0) tmp_bytes += r.tmp_stride * r.count;
     rs_runs.push_back(r);
@@ -809,8 +790,8 @@ void heic_b200_batch::run(uint32_t mask) {
     while (i < images.size()) {
       size_t j = i + 1;
       auto same = [&](const ImageInfo& a, const ImageInfo& b) {
-        return a.pic == b.pic && a.n_tiles == b.n_tiles && a.grid_cols == b.grid_cols && a.out_w == b.out_w &&
-               a.out_h == b.out_h && a.tile_w == b.tile_w && a.tile_h == b.tile_h && a.win_x == b.win_x && a.win_y == b.win_y &&
+        return a.pic == b.pic && a.n_tiles == b.n_tiles && a.grid_cols == b.grid_cols && a.canvas_w == b.canvas_w &&
+               a.canvas_h == b.canvas_h && a.tile_w == b.tile_w && a.tile_h == b.tile_h && a.win_x == b.win_x && a.win_y == b.win_y &&
                a.crop_x == b.crop_x && a.crop_y == b.crop_y && a.crop_w == b.crop_w && a.crop_h == b.crop_h &&
                a.orientation == b.orientation && a.full_range == b.full_range && a.matrix_coeffs == b.matrix_coeffs &&
                a.reduce == b.reduce && (a.filter != 0) == (b.filter != 0);
@@ -838,8 +819,8 @@ void heic_b200_batch::run(uint32_t mask) {
       job.tile_h = im.tile_h;
       job.grid_cols = im.grid_cols;
       job.grid_rows = im.grid_rows;
-      job.out_w = im.out_w;
-      job.out_h = im.out_h;
+      job.out_w = im.canvas_w;
+      job.out_h = im.canvas_h;
       job.n_images = (uint32_t)(j - i);
       job.chroma = (uint32_t)pp.chroma;
       job.full_range = im.full_range;
@@ -875,7 +856,7 @@ void heic_b200_batch::run(uint32_t mask) {
       rj.src_pitch = src_pitch;
       rj.src_image_stride = src_image_stride;
       rj.n_images = r.count;
-      rj.out_w = im.rot_w;
+      rj.out_w = im.rgb_w;
       uint8_t* out = (uint8_t*)d_rgb.p + (size_t)r.first * rgb_image_stride;
       const bool two = r.h_table >= 0 && r.v_table >= 0;
       if (r.h_table >= 0) {
@@ -896,7 +877,7 @@ void heic_b200_batch::run(uint32_t mask) {
         rj.dst = out;
         rj.dst_pitch = rgb_pitch;
         rj.dst_image_stride = rgb_image_stride;
-        rj.rows = im.rot_h;
+        rj.rows = im.rgb_h;
         rj.row0 = two ? r.row0 : 0;
         CU(launch_resample_v(rj, axis(r.v_table), st));
         ctx->launches++;
@@ -909,17 +890,46 @@ void heic_b200_batch::run(uint32_t mask) {
 // ---- C ABI ---------------------------------------------------------------------------------------------
 namespace {
 
+// The host copy of the device status of n tiles in the C ABI's form.
+void convert_status(const TileStatusDev* s, size_t n, heic_tile_status* out) {
+  for (size_t i = 0; i < n; i++) {
+    out[i].code = s[i].code;
+    out[i].bins_decoded = s[i].bins;
+    out[i].ctus_decoded = s[i].ctus;
+    out[i].reserved = 0;
+  }
+}
+
 void collect_status(heic_b200_batch* b, heic_tile_status* status) {
   cudaStream_t st = b->stream;
   const size_t n = b->tiles.size();
   CU(cudaMemcpyAsync(b->h_status.p, b->d_status.p, n * sizeof(TileStatusDev), cudaMemcpyDeviceToHost, st));
   CU(cudaStreamSynchronize(st));
-  const TileStatusDev* s = (const TileStatusDev*)b->h_status.p;
-  for (size_t i = 0; i < n; i++) {
-    status[i].code = s[i].code;
-    status[i].bins_decoded = s[i].bins;
-    status[i].ctus_decoded = s[i].ctus;
-    status[i].reserved = 0;
+  convert_status((const TileStatusDev*)b->h_status.p, n, status);
+}
+
+// The caller's RGB layout for one of n_imgs images: rows of at least rgb_w * 3 bytes and, with more than one image, an
+// image stride that holds its rows.
+void check_rgb_layout(const ImageInfo& im, size_t pitch, size_t image_stride, size_t n_imgs) {
+  if (pitch < (size_t)im.rgb_w * 3) bail(HEIC_E_INVALID_ARG, "output pitch smaller than a row of RGB");
+  if (n_imgs > 1 && (size_t)im.rgb_h * pitch > image_stride) bail(HEIC_E_INVALID_ARG, "image_stride smaller than one image (rows x pitch)");
+}
+
+// Queues on the batch's stream the device->host copy of the RGB of images [first, first + n) to dst, image i at
+// dst + (i - first) * image_stride.  When the caller's layout is the batch's and leaves no padding, that is one copy.
+void queue_rgb_download(const heic_b200_batch* b, size_t first, size_t n, uint8_t* dst, size_t pitch, size_t image_stride) {
+  const uint8_t* src = (const uint8_t*)b->d_rgb.p + first * b->rgb_image_stride;
+  bool one_copy = image_stride == b->rgb_image_stride && pitch == b->rgb_pitch;
+  for (size_t i = first; i < first + n && one_copy; i++)
+    one_copy = (size_t)b->images[i].rgb_w * 3 == pitch && (size_t)b->images[i].rgb_h * pitch == image_stride;
+  if (one_copy) {
+    CU(cudaMemcpyAsync(dst, src, n * image_stride, cudaMemcpyDeviceToHost, b->stream));
+    return;
+  }
+  for (size_t i = first; i < first + n; i++) {
+    const ImageInfo& im = b->images[i];
+    CU(cudaMemcpy2DAsync(dst + (i - first) * image_stride, pitch, src + (i - first) * b->rgb_image_stride, b->rgb_pitch,
+                         (size_t)im.rgb_w * 3, im.rgb_h, cudaMemcpyDeviceToHost, b->stream));
   }
 }
 
@@ -952,14 +962,12 @@ int32_t heic_b200_create(int32_t device, heic_b200_ctx** out_ctx) {
     c->cabac_tiles_per_cta = env_int("HEIC_B200_CABAC_TILES_PER_CTA", 32) == 1 ? 1 : 32;
     c->cabac_slots = env_int("HEIC_B200_CABAC_SLOTS", 0);
     c->intra_slots = std::min(8, env_int("HEIC_B200_INTRA_SLOTS", 0));
-    c->cabac_group_factor = std::max(1, env_int("HEIC_B200_CABAC_GROUP_FACTOR", 1));
     c->pipe_chunk = std::max(0, env_int("HEIC_B200_PIPE_CHUNK", 0));
     c->low_latency_tiles = env_int("HEIC_B200_LOW_LATENCY_TILES", 384);
     c->fuse_sao = env_int("HEIC_B200_FUSE_SAO", 1) != 0;
     c->cabac_persistent = env_int("HEIC_B200_CABAC_PERSISTENT", 1) != 0;
     c->cabac_resident = std::max(0, env_int("HEIC_B200_CABAC_RESIDENT", 0));
     c->cabac_plain_sort = env_int("HEIC_B200_CABAC_PLAIN_SORT", 0) != 0;
-    c->cabac_group_cap_pct = std::max(0, env_int("HEIC_B200_CABAC_GROUP_CAP", 0));
     c->pipe_slots = std::min((int)heic_b200_ctx::kPipe, std::max(0, env_int("HEIC_B200_PIPE_SLOTS", 0)));
     c->pipe_order = env_int("HEIC_B200_PIPE_ORDER", 1) != 0;
     *out_ctx = c.release();
@@ -980,15 +988,17 @@ int32_t heic_b200_batch_create(heic_b200_ctx* ctx, const heic_image_desc* imgs, 
   return heic_b200_batch_create_ex(ctx, imgs, n_imgs, 0, out);
 }
 
-static int64_t batch_create(heic_b200_ctx* ctx, const heic_image_desc* imgs, const heic_image_transform* xforms, const uint32_t* reduce,
-                            const heic_resize* resize, uint32_t n_imgs, heic_b200_batch** out) {
-  if (!ctx || !imgs || !xforms || !reduce || !resize || !out || !n_imgs) bail(HEIC_E_INVALID_ARG, "null argument");
+static int64_t batch_create(heic_b200_ctx* ctx, const heic_image_desc* imgs, const OutputSpec* specs, uint32_t n_imgs,
+                            heic_b200_batch** out) {
+  if (!ctx || !imgs || !out || !n_imgs) bail(HEIC_E_INVALID_ARG, "null argument");
   *out = nullptr;
   CU(cudaSetDevice(ctx->device));
+  std::vector<ImagePlan> plans(n_imgs);
+  for (uint32_t i = 0; i < n_imgs; i++) plans[i] = plan_image(imgs[i], specs[i], true);
   auto b = std::make_unique<heic_b200_batch>();
   b->ctx = ctx;
   b->stream = ctx->stream;
-  b->load(imgs, xforms, reduce, resize, n_imgs, true);
+  b->load(imgs, plans.data(), n_imgs, true);
   CU(cudaStreamSynchronize(ctx->stream));
   *out = b.release();
   return 0;
@@ -999,28 +1009,32 @@ int32_t heic_b200_batch_create_ex(heic_b200_ctx* ctx, const heic_image_desc* img
   return static_cast<int32_t>(guard([&]() -> int64_t {
     if (!ctx || !imgs || !out || !n_imgs) bail(HEIC_E_INVALID_ARG, "null argument");
     *out = nullptr;
-    return batch_create(ctx, imgs, canvas_transforms(imgs, n_imgs, apply_transforms).data(), no_reduction(n_imgs).data(),
-                        no_resize(n_imgs).data(), n_imgs, out);
+    return batch_create(ctx, imgs, output_specs(imgs, n_imgs, nullptr, nullptr, nullptr, apply_transforms).data(), n_imgs, out);
   }));
 }
 
 int32_t heic_b200_batch_create_transformed(heic_b200_ctx* ctx, const heic_image_desc* imgs, const heic_image_transform* xforms,
                                            uint32_t n_imgs, heic_b200_batch** out) {
   return static_cast<int32_t>(guard([&]() -> int64_t {
-    return batch_create(ctx, imgs, xforms, no_reduction(n_imgs).data(), no_resize(n_imgs).data(), n_imgs, out);
+    if (!xforms) bail(HEIC_E_INVALID_ARG, "null argument");
+    return batch_create(ctx, imgs, output_specs(imgs, n_imgs, xforms, nullptr, nullptr, 0).data(), n_imgs, out);
   }));
 }
 
 int32_t heic_b200_batch_create_reduced(heic_b200_ctx* ctx, const heic_image_desc* imgs, const heic_image_transform* xforms,
                                        const uint32_t* reduce, uint32_t n_imgs, heic_b200_batch** out) {
   return static_cast<int32_t>(guard([&]() -> int64_t {
-    return batch_create(ctx, imgs, xforms, reduce, no_resize(n_imgs).data(), n_imgs, out);
+    if (!xforms || !reduce) bail(HEIC_E_INVALID_ARG, "null argument");
+    return batch_create(ctx, imgs, output_specs(imgs, n_imgs, xforms, reduce, nullptr, 0).data(), n_imgs, out);
   }));
 }
 
 int32_t heic_b200_batch_create_resized(heic_b200_ctx* ctx, const heic_image_desc* imgs, const heic_image_transform* xforms,
                                        const uint32_t* reduce, const heic_resize* resize, uint32_t n_imgs, heic_b200_batch** out) {
-  return static_cast<int32_t>(guard([&]() -> int64_t { return batch_create(ctx, imgs, xforms, reduce, resize, n_imgs, out); }));
+  return static_cast<int32_t>(guard([&]() -> int64_t {
+    if (!xforms || !reduce || !resize) bail(HEIC_E_INVALID_ARG, "null argument");
+    return batch_create(ctx, imgs, output_specs(imgs, n_imgs, xforms, reduce, resize, 0).data(), n_imgs, out);
+  }));
 }
 
 void heic_b200_batch_destroy(heic_b200_batch* b) {
@@ -1066,19 +1080,10 @@ int32_t heic_b200_batch_download_rgb(heic_b200_batch* b, uint8_t* rgb_out, size_
   return static_cast<int32_t>(guard([&]() -> int64_t {
     if (!b || !rgb_out) bail(HEIC_E_INVALID_ARG, "null argument");
     CU(cudaSetDevice(b->ctx->device));
-    cudaStream_t st = b->stream;
-    for (size_t i = 0; i < b->images.size(); i++) {  // validate the whole layout before the first copy is queued
-      const ImageInfo& im = b->images[i];
-      if (pitch < (size_t)im.rot_w * 3) bail(HEIC_E_INVALID_ARG, "output pitch smaller than a row of RGB");
-      if (b->images.size() > 1 && (size_t)im.rot_h * pitch > image_stride)
-        bail(HEIC_E_INVALID_ARG, "image_stride smaller than one image (rows x pitch)");
-    }
-    for (size_t i = 0; i < b->images.size(); i++) {
-      const ImageInfo& im = b->images[i];
-      CU(cudaMemcpy2DAsync(rgb_out + i * image_stride, pitch, (const uint8_t*)b->d_rgb.p + i * b->rgb_image_stride,
-                           b->rgb_pitch, (size_t)im.rot_w * 3, im.rot_h, cudaMemcpyDeviceToHost, st));
-    }
-    CU(cudaStreamSynchronize(st));
+    // validate the whole layout before the first copy is queued
+    for (const ImageInfo& im : b->images) check_rgb_layout(im, pitch, image_stride, b->images.size());
+    queue_rgb_download(b, 0, b->images.size(), rgb_out, pitch, image_stride);
+    CU(cudaStreamSynchronize(b->stream));
     return 0;
   }));
 }
@@ -1089,10 +1094,8 @@ int32_t heic_b200_batch_download_image(heic_b200_batch* b, uint32_t image_index,
     if (!b || !rgb_out || image_index >= b->images.size()) bail(HEIC_E_INVALID_ARG, "invalid argument");
     if (!b->d_rgb.p) bail(HEIC_E_INVALID_ARG, "the batch has no RGB output");
     CU(cudaSetDevice(b->ctx->device));
-    const ImageInfo& im = b->images[image_index];
-    if (pitch < (size_t)im.rot_w * 3) bail(HEIC_E_INVALID_ARG, "output pitch smaller than a row of RGB");
-    CU(cudaMemcpy2DAsync(rgb_out, pitch, (const uint8_t*)b->d_rgb.p + (size_t)image_index * b->rgb_image_stride, b->rgb_pitch,
-                         (size_t)im.rot_w * 3, im.rot_h, cudaMemcpyDeviceToHost, b->stream));
+    check_rgb_layout(b->images[image_index], pitch, 0, 1);
+    queue_rgb_download(b, image_index, 1, rgb_out, pitch, 0);
     CU(cudaStreamSynchronize(b->stream));
     return 0;
   }));
@@ -1180,47 +1183,28 @@ static void harvest_slot(heic_b200_ctx* ctx, int slot) {
     std::fprintf(stderr, "[heic_b200] chunk slot %2d tiles %6zu: queued %8.1f  h2d %8.1f  cabac %8.1f  kernels %8.1f  d2h %8.1f ms\n", slot,
                  pd.n_tiles, t[0], t[1], t[2], t[3], t[4]);
   }
-  const TileStatusDev* s = (const TileStatusDev*)b->h_status.p;
-  heic_tile_status* out = pd.job->status + pd.tile0;
-  for (size_t i = 0; i < pd.n_tiles; i++) {
-    out[i].code = s[i].code;
-    out[i].bins_decoded = s[i].bins;
-    out[i].ctus_decoded = s[i].ctus;
-    out[i].reserved = 0;
-  }
+  convert_status((const TileStatusDev*)b->h_status.p, pd.n_tiles, pd.job->status + pd.tile0);
   pd.job = nullptr;
 }
 
-// xforms: one output geometry per image (RGB output; ignored for the planar output, which applies none)
-static heic_b200_job* submit_grids(heic_b200_ctx* ctx, const heic_image_desc* imgs, const heic_image_transform* xforms,
-                                   const uint32_t* reduce, const heic_resize* resize, uint32_t n_imgs, uint8_t* rgb_out, size_t pitch,
-                                   size_t image_stride, uint8_t* y_out, uint8_t* cb_out, uint8_t* cr_out, heic_tile_status* status) {
-  if (!ctx || !imgs || !xforms || !reduce || !resize || !n_imgs) bail(HEIC_E_INVALID_ARG, "null argument");
+// specs: one output per image (RGB output; the planar output applies no transform)
+static heic_b200_job* submit_grids(heic_b200_ctx* ctx, const heic_image_desc* imgs, const OutputSpec* specs, uint32_t n_imgs,
+                                   uint8_t* rgb_out, size_t pitch, size_t image_stride, uint8_t* y_out, uint8_t* cb_out,
+                                   uint8_t* cr_out, heic_tile_status* status) {
+  if (!ctx || !imgs || !n_imgs) bail(HEIC_E_INVALID_ARG, "null argument");
   CU(cudaSetDevice(ctx->device));
-  // validate every descriptor before any work is queued, so a bad image rejects the call as a whole
+  // plan every image, and check the caller's buffer layout for it, before any work is queued, so a bad image rejects the
+  // call as a whole
+  std::vector<ImagePlan> plans(n_imgs);
   std::vector<size_t> first_tile(n_imgs + 1, 0), y_off(n_imgs + 1, 0), c_off(n_imgs + 1, 0);
   for (uint32_t i = 0; i < n_imgs; i++) {
-    const heic_image_desc& im = imgs[i];
-    PicParams pp;
-    TileWindow win;
-    uint32_t out_w, out_h;
-    image_geometry(im, pp, win, out_w, out_h);
-    check_transform(xforms[i], out_w, out_h);
-    check_reduce(reduce[i]);
-    check_resize(resize[i]);
-    TileParams tp;
-    for (uint32_t t = 0; t < im.n_tiles; t++) make_tile_params(pp, im.pps, im.tiles[t], tp);
-    const size_t ow = out_w, oh = out_h;
-    if (rgb_out) {  // the caller's buffer layout, checked for every image before anything is queued
-      uint32_t rw, rh;
-      output_size(xforms[i], reduce[i], rw, rh);
-      resized_size(resize[i], rw, rh);
-      if (pitch < (size_t)rw * 3) bail(HEIC_E_INVALID_ARG, "output pitch smaller than a row of RGB");
-      if (n_imgs > 1 && (size_t)rh * pitch > image_stride) bail(HEIC_E_INVALID_ARG, "image_stride smaller than one image (rows x pitch)");
-    }
+    plans[i] = plan_image(imgs[i], specs[i], rgb_out != nullptr);
+    const ImageInfo& im = plans[i].info;
+    if (rgb_out) check_rgb_layout(im, pitch, image_stride, n_imgs);
+    const size_t cw = im.canvas_w, ch = im.canvas_h;
     first_tile[i + 1] = first_tile[i] + im.n_tiles;
-    y_off[i + 1] = y_off[i] + ow * oh;
-    c_off[i + 1] = c_off[i] + ((ow + 1) / 2) * ((oh + 1) / 2);
+    y_off[i + 1] = y_off[i] + cw * ch;
+    c_off[i + 1] = c_off[i] + ((cw + 1) / 2) * ((ch + 1) / 2);
   }
   static const bool trace = std::getenv("HEIC_B200_TRACE") != nullptr;  // host-side phase times of a submit, to stderr
   static const bool trace2 = trace && std::atoi(std::getenv("HEIC_B200_TRACE")) >= 2;  // + the device timeline of every chunk
@@ -1271,7 +1255,7 @@ static heic_b200_job* submit_grids(heic_b200_ctx* ctx, const heic_image_desc* im
     heic_b200_batch* b = ctx->pipe_batch[slot].get();
     cudaStream_t st = b->stream;
     t0 = clk::now();
-    b->load(imgs + i0, xforms + i0, reduce + i0, resize + i0, cnt, rgb_out != nullptr);
+    b->load(imgs + i0, plans.data() + i0, cnt, rgb_out != nullptr);
     t_load += ms_since(t0);
     t0 = clk::now();
     PipePending& pend = ctx->pipe_pending[slot];
@@ -1308,33 +1292,21 @@ static heic_b200_job* submit_grids(heic_b200_ctx* ctx, const heic_image_desc* im
     if (ctx->pipe_order && ctx->d2h_recorded) CU(cudaStreamWaitEvent(st, ctx->ev_d2h, 0));
     t_run += ms_since(t0);
     if (rgb_out) {
-      bool one_copy = image_stride == b->rgb_image_stride && pitch == b->rgb_pitch;
-      for (size_t i = 0; i < b->images.size() && one_copy; i++)
-        one_copy = (size_t)b->images[i].rot_w * 3 == pitch && (size_t)b->images[i].rot_h * pitch == image_stride;
-      if (one_copy) {
-        CU(cudaMemcpyAsync(rgb_out + (size_t)i0 * image_stride, b->d_rgb.p, (size_t)cnt * image_stride, cudaMemcpyDeviceToHost, st));
-      } else {
-        for (size_t i = 0; i < b->images.size(); i++) {
-          const ImageInfo& im = b->images[i];
-          if (pitch < (size_t)im.rot_w * 3) bail(HEIC_E_INVALID_ARG, "output pitch smaller than a row of RGB");
-          CU(cudaMemcpy2DAsync(rgb_out + (i0 + i) * image_stride, pitch, (const uint8_t*)b->d_rgb.p + i * b->rgb_image_stride,
-                               b->rgb_pitch, (size_t)im.rot_w * 3, im.rot_h, cudaMemcpyDeviceToHost, st));
-        }
-      }
+      queue_rgb_download(b, 0, cnt, rgb_out + (size_t)i0 * image_stride, pitch, image_stride);
     } else {
       // planar output: tile mosaic (each tile's conformance window) cropped to the canvas, images back to back
       for (size_t i = 0; i < b->images.size(); i++) {
         const ImageInfo& im = b->images[i];
         const PicParams& pp = b->pics[im.pic];
         const size_t yo = y_off[i0 + i], co = c_off[i0 + i];
-        const size_t cw = (im.out_w + 1) / 2, chh = (im.out_h + 1) / 2;
+        const size_t cw = (im.canvas_w + 1) / 2, chh = (im.canvas_h + 1) / 2;
         const uint8_t* fin = (const uint8_t*)b->d_final.p;
         for (uint32_t t = 0; t < im.n_tiles; t++) {
           const TileParams& tp = b->tiles[im.first_tile + t];
           const size_t tx = (size_t)(t % im.grid_cols) * im.tile_w, ty = (size_t)(t / im.grid_cols) * im.tile_h;
-          if (tx >= im.out_w || ty >= im.out_h) continue;
-          const size_t w = std::min<size_t>(im.tile_w, im.out_w - tx), h = std::min<size_t>(im.tile_h, im.out_h - ty);
-          CU(cudaMemcpy2DAsync(y_out + yo + ty * im.out_w + tx, im.out_w,
+          if (tx >= im.canvas_w || ty >= im.canvas_h) continue;
+          const size_t w = std::min<size_t>(im.tile_w, im.canvas_w - tx), h = std::min<size_t>(im.tile_h, im.canvas_h - ty);
+          CU(cudaMemcpy2DAsync(y_out + yo + ty * im.canvas_w + tx, im.canvas_w,
                                fin + tp.plane_off[0] + (size_t)im.win_y * pp.pitch_y + im.win_x, pp.pitch_y, w, h,
                                cudaMemcpyDeviceToHost, st));
           if (pp.chroma && cb_out && cr_out) {  // 4:2:0: the window's offsets and sizes are even
@@ -1391,18 +1363,18 @@ static int64_t job_wait(heic_b200_job* job) {
   return 0;
 }
 
-static int64_t decode_grids_impl(heic_b200_ctx* ctx, const heic_image_desc* imgs, const heic_image_transform* xforms,
-                                 const uint32_t* reduce, const heic_resize* resize, uint32_t n_imgs, uint8_t* rgb_out, size_t pitch,
-                                 size_t image_stride, uint8_t* y_out, uint8_t* cb_out, uint8_t* cr_out, heic_tile_status* status) {
-  return job_wait(submit_grids(ctx, imgs, xforms, reduce, resize, n_imgs, rgb_out, pitch, image_stride, y_out, cb_out, cr_out, status));
+static int64_t decode_grids_impl(heic_b200_ctx* ctx, const heic_image_desc* imgs, const OutputSpec* specs, uint32_t n_imgs,
+                                 uint8_t* rgb_out, size_t pitch, size_t image_stride, uint8_t* y_out, uint8_t* cb_out,
+                                 uint8_t* cr_out, heic_tile_status* status) {
+  return job_wait(submit_grids(ctx, imgs, specs, n_imgs, rgb_out, pitch, image_stride, y_out, cb_out, cr_out, status));
 }
 
 int32_t heic_b200_decode_grids(heic_b200_ctx* ctx, const heic_image_desc* imgs, uint32_t n_imgs, uint8_t* rgb_out,
                                size_t pitch, size_t image_stride, int32_t apply_transforms, heic_tile_status* status) {
   return static_cast<int32_t>(guard([&]() -> int64_t {
     if (!ctx || !rgb_out) bail(HEIC_E_INVALID_ARG, "null argument");
-    return decode_grids_impl(ctx, imgs, canvas_transforms(imgs, n_imgs, apply_transforms).data(), no_reduction(n_imgs).data(),
-                             no_resize(n_imgs).data(), n_imgs, rgb_out, pitch, image_stride, nullptr, nullptr, nullptr, status);
+    return decode_grids_impl(ctx, imgs, output_specs(imgs, n_imgs, nullptr, nullptr, nullptr, apply_transforms).data(), n_imgs,
+                             rgb_out, pitch, image_stride, nullptr, nullptr, nullptr, status);
   }));
 }
 
@@ -1411,7 +1383,8 @@ int32_t heic_b200_decode_grids_transformed(heic_b200_ctx* ctx, const heic_image_
                                            heic_tile_status* status) {
   return static_cast<int32_t>(guard([&]() -> int64_t {
     if (!rgb_out) bail(HEIC_E_INVALID_ARG, "null output buffer");
-    return decode_grids_impl(ctx, imgs, xforms, no_reduction(n_imgs).data(), no_resize(n_imgs).data(), n_imgs, rgb_out, pitch,
+    if (!xforms) bail(HEIC_E_INVALID_ARG, "null argument");
+    return decode_grids_impl(ctx, imgs, output_specs(imgs, n_imgs, xforms, nullptr, nullptr, 0).data(), n_imgs, rgb_out, pitch,
                              image_stride, nullptr, nullptr, nullptr, status);
   }));
 }
@@ -1421,8 +1394,9 @@ int32_t heic_b200_decode_grids_reduced(heic_b200_ctx* ctx, const heic_image_desc
                                        heic_tile_status* status) {
   return static_cast<int32_t>(guard([&]() -> int64_t {
     if (!rgb_out) bail(HEIC_E_INVALID_ARG, "null output buffer");
-    return decode_grids_impl(ctx, imgs, xforms, reduce, no_resize(n_imgs).data(), n_imgs, rgb_out, pitch, image_stride, nullptr,
-                             nullptr, nullptr, status);
+    if (!xforms || !reduce) bail(HEIC_E_INVALID_ARG, "null argument");
+    return decode_grids_impl(ctx, imgs, output_specs(imgs, n_imgs, xforms, reduce, nullptr, 0).data(), n_imgs, rgb_out, pitch,
+                             image_stride, nullptr, nullptr, nullptr, status);
   }));
 }
 
@@ -1431,8 +1405,9 @@ int32_t heic_b200_decode_grids_resized(heic_b200_ctx* ctx, const heic_image_desc
                                        size_t pitch, size_t image_stride, heic_tile_status* status) {
   return static_cast<int32_t>(guard([&]() -> int64_t {
     if (!rgb_out) bail(HEIC_E_INVALID_ARG, "null output buffer");
-    return decode_grids_impl(ctx, imgs, xforms, reduce, resize, n_imgs, rgb_out, pitch, image_stride, nullptr, nullptr, nullptr,
-                             status);
+    if (!xforms || !reduce || !resize) bail(HEIC_E_INVALID_ARG, "null argument");
+    return decode_grids_impl(ctx, imgs, output_specs(imgs, n_imgs, xforms, reduce, resize, 0).data(), n_imgs, rgb_out, pitch,
+                             image_stride, nullptr, nullptr, nullptr, status);
   }));
 }
 
@@ -1441,8 +1416,8 @@ int32_t heic_b200_decode_grids_submit(heic_b200_ctx* ctx, const heic_image_desc*
                                       heic_b200_job** out_job) {
   return static_cast<int32_t>(guard([&]() -> int64_t {
     if (!ctx || !rgb_out || !out_job) bail(HEIC_E_INVALID_ARG, "null argument");
-    *out_job = submit_grids(ctx, imgs, canvas_transforms(imgs, n_imgs, apply_transforms).data(), no_reduction(n_imgs).data(),
-                            no_resize(n_imgs).data(), n_imgs, rgb_out, pitch, image_stride, nullptr, nullptr, nullptr, status);
+    *out_job = submit_grids(ctx, imgs, output_specs(imgs, n_imgs, nullptr, nullptr, nullptr, apply_transforms).data(), n_imgs,
+                            rgb_out, pitch, image_stride, nullptr, nullptr, nullptr, status);
     return 0;
   }));
 }
@@ -1452,8 +1427,8 @@ int32_t heic_b200_decode_grids_submit_transformed(heic_b200_ctx* ctx, const heic
                                                   size_t pitch, size_t image_stride, heic_tile_status* status,
                                                   heic_b200_job** out_job) {
   return static_cast<int32_t>(guard([&]() -> int64_t {
-    if (!rgb_out || !out_job) bail(HEIC_E_INVALID_ARG, "null argument");
-    *out_job = submit_grids(ctx, imgs, xforms, no_reduction(n_imgs).data(), no_resize(n_imgs).data(), n_imgs, rgb_out, pitch,
+    if (!rgb_out || !out_job || !xforms) bail(HEIC_E_INVALID_ARG, "null argument");
+    *out_job = submit_grids(ctx, imgs, output_specs(imgs, n_imgs, xforms, nullptr, nullptr, 0).data(), n_imgs, rgb_out, pitch,
                             image_stride, nullptr, nullptr, nullptr, status);
     return 0;
   }));
@@ -1463,9 +1438,9 @@ int32_t heic_b200_decode_grids_submit_reduced(heic_b200_ctx* ctx, const heic_ima
                                               const uint32_t* reduce, uint32_t n_imgs, uint8_t* rgb_out, size_t pitch,
                                               size_t image_stride, heic_tile_status* status, heic_b200_job** out_job) {
   return static_cast<int32_t>(guard([&]() -> int64_t {
-    if (!rgb_out || !out_job) bail(HEIC_E_INVALID_ARG, "null argument");
-    *out_job = submit_grids(ctx, imgs, xforms, reduce, no_resize(n_imgs).data(), n_imgs, rgb_out, pitch, image_stride, nullptr,
-                            nullptr, nullptr, status);
+    if (!rgb_out || !out_job || !xforms || !reduce) bail(HEIC_E_INVALID_ARG, "null argument");
+    *out_job = submit_grids(ctx, imgs, output_specs(imgs, n_imgs, xforms, reduce, nullptr, 0).data(), n_imgs, rgb_out, pitch,
+                            image_stride, nullptr, nullptr, nullptr, status);
     return 0;
   }));
 }
@@ -1474,8 +1449,9 @@ int32_t heic_b200_decode_grids_submit_resized(heic_b200_ctx* ctx, const heic_ima
                                               const uint32_t* reduce, const heic_resize* resize, uint32_t n_imgs, uint8_t* rgb_out,
                                               size_t pitch, size_t image_stride, heic_tile_status* status, heic_b200_job** out_job) {
   return static_cast<int32_t>(guard([&]() -> int64_t {
-    if (!rgb_out || !out_job) bail(HEIC_E_INVALID_ARG, "null argument");
-    *out_job = submit_grids(ctx, imgs, xforms, reduce, resize, n_imgs, rgb_out, pitch, image_stride, nullptr, nullptr, nullptr, status);
+    if (!rgb_out || !out_job || !xforms || !reduce || !resize) bail(HEIC_E_INVALID_ARG, "null argument");
+    *out_job = submit_grids(ctx, imgs, output_specs(imgs, n_imgs, xforms, reduce, resize, 0).data(), n_imgs, rgb_out, pitch,
+                            image_stride, nullptr, nullptr, nullptr, status);
     return 0;
   }));
 }
@@ -1491,8 +1467,8 @@ int32_t heic_b200_decode_grids_yuv(heic_b200_ctx* ctx, const heic_image_desc* im
                                    uint8_t* cb_out, uint8_t* cr_out, heic_tile_status* status) {
   return static_cast<int32_t>(guard([&]() -> int64_t {
     if (!ctx || !y_out) bail(HEIC_E_INVALID_ARG, "null argument");
-    return decode_grids_impl(ctx, imgs, canvas_transforms(imgs, n_imgs, 0).data(), no_reduction(n_imgs).data(),
-                             no_resize(n_imgs).data(), n_imgs, nullptr, 0, 0, y_out, cb_out, cr_out, status);
+    return decode_grids_impl(ctx, imgs, output_specs(imgs, n_imgs, nullptr, nullptr, nullptr, 0).data(), n_imgs, nullptr, 0, 0,
+                             y_out, cb_out, cr_out, status);
   }));
 }
 
@@ -1501,10 +1477,9 @@ int32_t heic_b200_decode_file(heic_b200_ctx* ctx, const uint8_t* data, size_t le
   return static_cast<int32_t>(guard([&]() -> int64_t {
     if (!ctx || !data || !rgb_out) bail(HEIC_E_INVALID_ARG, "null argument");
     std::unique_ptr<HeicFile> f = HeicDecoder::open(data, len);
-    const heic_image_transform xf = apply_transforms ? f->primary.transform : canvas_transforms(&f->primary.desc, 1, 0)[0];
-    const uint32_t k = 1;
-    const heic_resize none = {0, 0, 0};
-    return decode_grids_impl(ctx, &f->primary.desc, &xf, &k, &none, 1, rgb_out, pitch, 0, nullptr, nullptr, nullptr, nullptr);
+    const heic_image_transform* xf = apply_transforms ? &f->primary.transform : nullptr;
+    return decode_grids_impl(ctx, &f->primary.desc, output_specs(&f->primary.desc, 1, xf, nullptr, nullptr, 0).data(), 1, rgb_out,
+                             pitch, 0, nullptr, nullptr, nullptr, nullptr);
   }));
 }
 

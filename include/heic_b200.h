@@ -415,7 +415,8 @@ void*   heic_b200_batch_stream(heic_b200_batch* b);
 /* Device pointer + layout of the RGB output (image i at base + i*image_stride). */
 int32_t heic_b200_batch_rgb(heic_b200_batch* b, void** dev_ptr, size_t* pitch, size_t* image_stride);
 int32_t heic_b200_batch_download_rgb(heic_b200_batch* b, uint8_t* rgb_out, size_t pitch, size_t image_stride);
-/* RGB of one image of the batch (rows of rot_w*3 bytes, `pitch` apart) to host memory; synchronises the batch's stream. */
+/* RGB of one image of the batch (rows of 3 bytes per output pixel, `pitch` apart) to host memory; synchronises the batch's
+ * stream. */
 int32_t heic_b200_batch_download_image(heic_b200_batch* b, uint32_t image_index, uint8_t* rgb_out, size_t pitch);
 int32_t heic_b200_batch_status(heic_b200_batch* b, heic_tile_status* status /* n_total_tiles */);
 uint32_t heic_b200_batch_tile_count(const heic_b200_batch* b);

@@ -49,7 +49,7 @@ def test_fixture_orientations_and_crops(decoder, heic_file, fixture_rgb, crop):
     img = heic_file.primary
     xfs = [_xf(CROPS[crop], o) for o in range(8)]
     exp = [apply_transform(fixture_rgb, t) for t in xfs]
-    # decode_grids_transformed: one call per output shape
+    # decode_grids with transforms: one call per output shape
     for parity in (0, 1):
         sel = [o for o in range(8) if (o & 1) == parity]
         got = decoder.decode_grids([img] * len(sel), transforms=[xfs[o] for o in sel])

@@ -5,7 +5,7 @@ geometry (tiles drawn from the fixture and the synthetic pool as bench.py does).
    orientations {0, 1, 6} (k = 1 is color_stitch_kernel / color_geom_kernel, k > 1 color_reduce_kernel).  Reports us per
    image and GB/s on the algorithmic traffic of 1.5 B in + 3 / k^2 B out per canvas pixel.  The rounds alternate the cases,
    and the median round is reported.
-2. Serving loop: calls of --call-images images through heic_b200_decode_grids_submit_reduced / _job_wait with 3 calls in
+2. Serving loop: calls of --call-images images through HeicDecoder.submit_grids / wait_job with 3 calls in
    flight (pinned host RGB, as bench.py's e2e), and the synchronous call one at a time, for k in {1, 2, 4, 8}: canvas MP/s
    (12.19 MP per image, whatever k) and the device->host bytes per call.  The rounds alternate the factors.
 
